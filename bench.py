@@ -336,6 +336,8 @@ def run_gpu(args):
         st_dyn[k].copy_(o["STATUS_DYN"]); it_dyn[k].copy_(o["ITER_DYN"]); st_ss[k].copy_(o["STATUS_SS"])
     barrier()
     windows.append((t_w0, time.time()))
+    # what the caller of the timed path received from its last step (the buffers behind `o` are reused by the runs below)
+    last = {key: val.clone() for key, val in o.items() if isinstance(val, torch.Tensor)} if args.dump_outputs else None
     elapsed_ms = ev[0].elapsed_time(ev[K])
     launches = ctl.h.launches - launches0
     step_ms = np.array([ev[k].elapsed_time(ev[k + 1]) for k in range(K)])
@@ -479,6 +481,8 @@ def run_gpu(args):
         "roofline": roofline, "roofline_others": roofline_others, "cpu_baseline": cpu_baseline, "cpu_baseline_numpy": cpu_numpy, "clocks": clocks,
         "solver_stats": stats,
     }
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     emit(out)
     if world > 1:
         dist.destroy_process_group()
@@ -490,6 +494,14 @@ def cp_ws_bytes(cp):
     nz = d.nx + d.nu
     rec = nz * d.nx + d.nx + nz * nz + 7 * nz + d.ng * (nz + 10) + 10
     return 8 * (d.N * (rec + 20 + 4 * d.nx + 6 * d.ng) + 5 * d.nw + d.npar)
+
+
+def dump_outputs(path, outputs):
+    """``<path>/<name>.npy`` for every output of one fused step (rank 0's instances; [B, ...] float64, integer status
+    and iteration counts included as float64): 0.7 MB at B = 4096, so nothing is sampled."""
+    os.makedirs(path, exist_ok=True)
+    for key, val in outputs.items():
+        np.save(os.path.join(path, key + ".npy"), val.detach().cpu().numpy().astype(np.float64))
 
 
 _JSON_FD = None
@@ -510,7 +522,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the arrays the last timed step returned as DIR/<name>.npy, to compare two builds "
+                         "output for output on the same seeded workload")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     # stdout carries exactly ONE line, the JSON record: everything else that libraries write to file descriptor 1 (NCCL
     # prints its version banner there) is sent to stderr, and the record goes to the saved descriptor at the end
     global _JSON_FD

@@ -9,6 +9,7 @@ import hashlib
 import os
 import shutil
 import subprocess
+import tempfile
 
 from .devicegen import generate_header
 
@@ -26,6 +27,19 @@ def _nvcc() -> str:
     if not os.path.exists(exe):
         raise RuntimeError("nvcc not found: the CUDA library cannot be built (there is no CPU fallback)")
     return exe
+
+
+def build_dir_for(path: str, artefact: str) -> str:
+    """Where to keep ``artefact``: ``path`` (in the tree) when it is already there or ``path`` can be written, else a
+    per-user directory under the system temporary directory, so that a read-only tree compiles what it lacks there."""
+    if os.path.exists(os.path.join(path, artefact)):
+        return path
+    probe = path
+    while not os.path.exists(probe):
+        probe = os.path.dirname(probe)
+    if os.access(probe, os.W_OK):
+        return path
+    return os.path.join(tempfile.gettempdir(), "mpc_code_b200_%d" % os.getuid(), os.path.basename(os.path.dirname(path)))
 
 
 def source_digest(header_text: str) -> str:
@@ -47,8 +61,9 @@ def build_library(name: str, prob, ss_spec, ocp_spec, verbose: bool = False, ext
     extra_flags = tuple(extra_flags) + tuple(os.environ.get("MPCB_EXTRA_FLAGS", "").split())
     gen = generate_header(prob, ss_spec, ocp_spec)
     digest = source_digest(gen["text"] + " ".join(extra_flags))
-    work = os.path.join(BUILD_DIR, "%s_%s" % (name, digest))
-    so_path = os.path.join(BUILD_DIR, "libmpcb_%s_%s.so" % (name, digest))
+    base = build_dir_for(BUILD_DIR, "libmpcb_%s_%s.so" % (name, digest))
+    work = os.path.join(base, "%s_%s" % (name, digest))
+    so_path = os.path.join(base, "libmpcb_%s_%s.so" % (name, digest))
     header = os.path.join(work, "mpcb_model.h")
     os.makedirs(work, exist_ok=True)
     if not os.path.exists(header):          # published atomically: several ranks may start on a cold _build at once

@@ -280,6 +280,8 @@ class CModule:
         src = emit_header("MPCB_GEN_%s_H" % name.upper(), {}, functions,
                           preamble="#undef MPCB_FN\n#define MPCB_FN __attribute__((visibility(\"default\")))\n#undef MPCB_FN_BIG\n#define MPCB_FN_BIG MPCB_FN\n")
         digest = hashlib.sha256((src + " ".join(cflags)).encode()).hexdigest()[:16]
+        from .build import build_dir_for
+        build_dir = build_dir_for(build_dir, "%s_%s.so" % (name, digest))
         os.makedirs(build_dir, exist_ok=True)
         c_path = os.path.join(build_dir, "%s_%s.c" % (name, digest))
         so_path = os.path.join(build_dir, "%s_%s.so" % (name, digest))

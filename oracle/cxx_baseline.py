@@ -22,6 +22,7 @@ VP = ctypes.c_void_p
 
 def build(name, prob, ss, ocp):
     """Compile the loop for one problem; returns the path of the shared object (cached by content hash)."""
+    from mpc_code_b200.build import build_dir_for
     from mpc_code_b200.devicegen import generate_header
     text = generate_header(prob, ss, ocp)["text"]
     hsh = hashlib.sha256(text.encode())
@@ -32,8 +33,9 @@ def build(name, prob, ss, ocp):
         hsh.update(fh.read())
     hsh.update(_cpu_flags().encode())        # -march=native: a library built on another host CPU must not be reused
     digest = hsh.hexdigest()[:16]
-    work = os.path.join(BUILD, "cxx_%s_%s" % (name, digest))
-    so = os.path.join(BUILD, "cxx_%s_%s.so" % (name, digest))
+    base = build_dir_for(BUILD, "cxx_%s_%s.so" % (name, digest))
+    work = os.path.join(base, "cxx_%s_%s" % (name, digest))
+    so = os.path.join(base, "cxx_%s_%s.so" % (name, digest))
     if not os.path.exists(so):
         os.makedirs(work, exist_ok=True)
         hdr = os.path.join(work, "mpcb_model.h")

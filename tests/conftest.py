@@ -12,7 +12,7 @@ if ROOT not in sys.path:
 import mpc_code_b200  # noqa: E402,F401
 import __graft_entry__ as entry  # noqa: E402
 
-REFERENCE = "/root/reference"
+REFERENCE = os.environ.get("MPC_CODE_REFERENCE", "")     # an unmodified CPCLAB-UNIPI/MPC-code checkout, if any
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 

@@ -1,13 +1,16 @@
-"""Regenerate the committed fixtures (run in the build container, where /root/reference exists):
+"""Regenerate the committed fixtures from an unmodified CPCLAB-UNIPI/MPC-code checkout:
 
-    python tests/golden/make_golden.py
+    MPC_CODE_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 * ``kat.json``  - known-answer facts read from the reference's own example files (SURVEY.md section 4):
   KAT1 steady state of Ex_NMPC.py, KAT2 the printed linearisation in Ex_LMPC_nlplant.py:85-91,
   KAT3 closed-form targets derived from Ex_NMPC.py:129-148,217-219,241-242.
 * ``ref_examples_oracle.npz`` - oracle closed loops of the unmodified Ex_NMPC_dis.py and Ex_LMPCxp_nlplant.py.
-* ``nmpc_oracle.npz`` - outputs of the CPU oracle on the UNMODIFIED /root/reference/Ex_NMPC.py
+* ``nmpc_oracle.npz`` - outputs of the CPU oracle on the UNMODIFIED Ex_NMPC.py of the checkout
   (loaded through the casadi stand-in): OCP and target solutions, EKF updates, a short closed loop.
+* ``problem_records.json`` - what defines each problem (tests/problem_record.py) of the unmodified files that
+  examples/ restates (``--only-problem-records``).  ``--only-problem-records --from-examples`` records the
+  restatements instead, for use where no checkout exists; the file names its source.
 """
 import json
 import os
@@ -26,7 +29,7 @@ from oracle.closed_loop import OracleLoop  # noqa: E402
 from oracle.ipm import IpmOptions  # noqa: E402
 from oracle.nlp import OcpNlp, TargetNlp  # noqa: E402
 
-REF = "/root/reference"
+REF = os.environ.get("MPC_CODE_REFERENCE", "")
 
 
 def make_synthetic(names):
@@ -73,7 +76,30 @@ def make_reference_examples():
     np.savez_compressed(os.path.join(HERE, "ref_examples_oracle.npz"), **out)
 
 
+def make_problem_records(from_examples):
+    """``problem_records.json``: the records of the reference files examples/ restates, or of the restatements."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    import __graft_entry__ as entry
+    from problem_record import PAIRS, RECORDS, TIMES, plain, record
+    out = dict(source="examples/ restatements" if from_examples else "unmodified reference files", times=plain(TIMES),
+               problems={})
+    for name, fname, edits in PAIRS:
+        if from_examples:
+            prob, ss, ocp = entry._problem(name)
+        else:
+            prob = build_problem(load_example(os.path.join(REF, fname), source_edits=edits))
+            ss, ocp = make_specs(prob)
+        out["problems"][name] = record(prob, ss, ocp)
+    with open(RECORDS, "w") as fh:
+        json.dump(out, fh)
+
+
 def main():
+    if "--only-problem-records" in sys.argv:                      # python make_golden.py --only-problem-records
+        make_problem_records("--from-examples" in sys.argv)
+        return
+    if not os.path.isdir(REF) and "--only-synthetic" not in " ".join(sys.argv):
+        raise SystemExit("set MPC_CODE_REFERENCE to an unmodified CPCLAB-UNIPI/MPC-code checkout")
     if "--only-examples" in sys.argv:                             # python make_golden.py --only-examples
         make_reference_examples()
         return
@@ -176,6 +202,7 @@ def main():
     if syn_args:
         make_synthetic(tuple(syn_args[0].split("=", 1)[1].split(",")) if "=" in syn_args[0] else ("syn_8_3_50",))
     make_reference_examples()
+    make_problem_records(False)
     print("wrote fixtures")
 
 

@@ -1,24 +1,16 @@
-"""The problem files under examples/ are condensed restatements of the reference's Ex_*.py.  Where the reference
-checkout exists (the build container), every one of them must define the SAME problem as the unmodified reference
-file: dimensions, flags, model / plant / output maps and costs evaluated at random points, set-points, parameters,
-bounds, parameter offsets, estimator data and initial state.  This is what lets the GPU tests (which cannot read
-/root/reference) use the oracle fixtures generated from the unmodified files (tests/golden/make_golden.py)."""
-import os
-
+"""The problem files under examples/ are condensed restatements of the reference's Ex_*.py.  Every one of them must
+define the SAME problem as the unmodified reference file: dimensions, flags, model / plant / output maps and costs
+evaluated at random points, set-points, parameters, bounds, parameter offsets, estimator data and initial state.
+The reference side is stored in tests/golden/problem_records.json (see tests/problem_record.py); its `source` field
+says whether it was recorded from the unmodified files or from restatements that this test had checked against them.
+This is what lets the tests use the oracle fixtures generated from the unmodified files (tests/golden/make_golden.py)."""
 import numpy as np
 import pytest
 
 import __graft_entry__ as entry
-from conftest import REFERENCE
-from mpc_code_b200.loader import load_example
-from mpc_code_b200.problem import build_problem, make_specs
+from problem_record import PAIRS, load_records, evaluate, plain, record
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")
-
-PAIRS = [("nmpc_cstr", "Ex_NMPC.py", ()), ("lmpc_cstr", "Ex_LMPC_CSTR.py", ()), ("lmpc_wb", "Ex_LMPC_WB.py", ()),
-         ("lmpc_nlplant", "Ex_LMPC_nlplant.py", ()), ("nmpc_dis", "Ex_NMPC_dis.py", ()),
-         ("lmpcxp_nlplant", "Ex_LMPCxp_nlplant.py", ()),
-         ("enmpc_reactor", "Ex_ENMPC.py", (("mhe_mod = 'on'", "mhe_mod = 'off'"),))]
+REF = load_records()
 
 
 def _same(a, b):
@@ -28,51 +20,37 @@ def _same(a, b):
 
 @pytest.mark.parametrize("name,fname,edits", PAIRS)
 def test_example_restates_the_reference_file(name, fname, edits):
-    ref = build_problem(load_example(os.path.join(REFERENCE, fname), source_edits=edits))
+    ref = REF["problems"][name]
     mine, ss_b, ocp_b = entry._problem(name)
+    rec = record(mine, ss_b, ocp_b)
     for attr in ("nx", "nxp", "nu", "ny", "nd", "N", "h", "npx", "npy", "npxp", "npyp", "nxi"):
-        assert getattr(ref, attr) == getattr(mine, attr), attr
-    assert ref.flags == mine.flags
+        assert ref[attr] == rec[attr], attr
+    assert ref["flags"] == rec["flags"]
     for attr in ("x0_p", "x0_m", "u0", "dhat0"):
-        assert _same(getattr(ref, attr), getattr(mine, attr)), attr
-    rng = np.random.default_rng(0)
-    nx, nxp, nu, ny, nd = mine.nx, mine.nxp, mine.nu, mine.ny, mine.nd
-    for _ in range(4):
-        x = mine.x0_m * (1 + 0.02 * rng.standard_normal(nx)) + 1e-3 * rng.standard_normal(nx)
-        xp = mine.x0_p * (1 + 0.02 * rng.standard_normal(nxp)) + 1e-3 * rng.standard_normal(nxp)
-        u = mine.u0 * (1 + 0.01 * rng.standard_normal(nu)) + 1e-3 * rng.standard_normal(nu)
-        d = 0.1 * rng.standard_normal(nd); t = float(rng.uniform(0, 30))
-        px, py = 1e-3 * rng.standard_normal(mine.npx), 1e-3 * rng.standard_normal(mine.npy)
-        pxp, pyp = 1e-3 * rng.standard_normal(mine.npxp), 1e-3 * rng.standard_normal(mine.npyp)
-        if mine.flags["offree"] == "nl":
-            d = np.abs(d) + 0.05                      # a physical feed rate for the CSTR models
-        assert _same(ref.Fx_model(x, u, mine.h, d, t, px), mine.Fx_model(x, u, mine.h, d, t, px))
-        assert _same(ref.Fy_model(x, u, d, t, py), mine.Fy_model(x, u, d, t, py))
-        assert _same(ref.Fx_p(xp, u, pxp, t, mine.h, pxp), mine.Fx_p(xp, u, pxp, t, mine.h, pxp))
-        assert _same(ref.Fy_p(xp, u, pyp, t, pyp), mine.Fy_p(xp, u, pyp, t, pyp))
-        y = rng.standard_normal(ny); xs = rng.standard_normal(nx); us = rng.standard_normal(nu); ys = rng.standard_normal(ny)
-        assert _same(ref.F_obj(x, u, y, xs, us, ys), mine.F_obj(x, u, y, xs, us, ys))
-        assert _same(ref.Fss_obj(x, u, y, xs, us, ys), mine.Fss_obj(x, u, y, xs, us, ys))
-        assert _same(ref.Vfin(x, xs), mine.Vfin(x, xs))
-    for t in (0.0, 4.9, 19.9, 20.0, 25.0, 50.0, 55.0, 1500.0, 2250.0, 2251.0, 4500.0, 6000.0):
-        if mine.defSP is not None:
-            for a, b in zip(ref.defSP(t), mine.defSP(t)):
-                assert _same(a, b), ("defSP", t)
-        for fn in ("def_px", "def_py", "def_pxp", "def_pyp", "def_pxmp", "def_pymp"):
-            assert (fn in ref.ns) == (fn in mine.ns), fn
-            if fn in mine.ns:
-                assert _same(ref.ns[fn](t)[0], mine.ns[fn](t)[0]), (fn, t)
-    ss_a, ocp_a = make_specs(ref)
-    for k in ("w_lb", "w_ub", "g_lb", "g_ub"):
-        assert np.array_equal(getattr(ocp_a, k), getattr(ocp_b, k)), k
-        assert np.array_equal(getattr(ss_a, k), getattr(ss_b, k)), k
-    assert ocp_a.off == ocp_b.off and ss_a.off == ss_b.off and ocp_a.flags == ocp_b.flags
-    assert ocp_a.yFree == ocp_b.yFree and ocp_a.DuFree == ocp_b.DuFree and ocp_a.uses_uprev == ocp_b.uses_uprev
-    ea, eb = ref.estimator, mine.estimator
+        assert _same(ref[attr], rec[attr]), attr
+    for pt, ev_ref in zip(ref["points"], ref["evals"]):        # the maps of both problems at the same points
+        ev = evaluate(mine, pt)
+        for fn, val in ev_ref.items():
+            assert _same(val, ev[fn]), fn
+    assert (ref["defSP"] is None) == (rec["defSP"] is None)
+    if rec["defSP"] is not None:
+        for t, a, b in zip(REF["times"], ref["defSP"], rec["defSP"]):
+            assert len(a) == len(b) and all(_same(u, v) for u, v in zip(a, b)), ("defSP", t)
+    assert sorted(ref["params"]) == sorted(rec["params"])
+    for fn in rec["params"]:
+        for t, a, b in zip(REF["times"], ref["params"][fn], rec["params"][fn]):
+            assert _same(a, b), (fn, t)
+    for tag in ("ocp", "ss"):
+        for k in ("w_lb", "w_ub", "g_lb", "g_ub"):
+            assert np.array_equal(ref[tag][k], rec[tag][k]), (tag, k)
+        assert ref[tag]["off"] == rec[tag]["off"], tag
+    for k in ("flags", "yFree", "DuFree", "uses_uprev"):
+        assert ref["ocp"][k] == rec["ocp"][k], k
+    ea, eb = ref["estimator"], rec["estimator"]
     assert ea["type"] == eb["type"]
     for k in ("Q", "R", "K", "P0", "dmin", "dmax"):
-        assert (ea.get(k) is None) == (eb.get(k) is None), k
-        if eb.get(k) is not None:
+        assert (ea[k] is None) == (eb[k] is None), k
+        if eb[k] is not None:
             assert _same(ea[k], eb[k]), k
-    assert ref.sol_optss == mine.sol_optss and ref.sol_optdyn == mine.sol_optdyn
-    assert (ref.R_wn is None) == (mine.R_wn is None) and (mine.R_wn is None or _same(ref.R_wn, mine.R_wn))
+    assert ref["sol_optss"] == plain(mine.sol_optss) and ref["sol_optdyn"] == plain(mine.sol_optdyn)
+    assert (ref["R_wn"] is None) == (rec["R_wn"] is None) and (rec["R_wn"] is None or _same(ref["R_wn"], rec["R_wn"]))

@@ -53,27 +53,24 @@ def test_kat3_target_solutions_of_the_oracle(nmpc):
             assert abs(r.x[1] - exp_["xs1"]) < 2e-6 and abs(r.x[3] - exp_["us0"]) < 2e-6
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")
 def test_unmodified_reference_example_defines_the_same_problem(nmpc):
-    ref = build_problem(load_example(os.path.join(REFERENCE, "Ex_NMPC.py")))
+    """Bit-exact against the stored record of the Ex_NMPC.py problem (tests/golden/problem_records.json)."""
+    from problem_record import evaluate, load_records, record
+    ref = load_records()["problems"]["nmpc_cstr"]
     mine = nmpc.prob
+    rec = record(mine, nmpc.ss, nmpc.ocp)
     for name in ("nx", "nu", "ny", "nd", "N", "h", "Nsim", "npx", "npy"):
-        assert getattr(ref, name) == getattr(mine, name)
-    assert ref.flags == mine.flags
-    rng = np.random.default_rng(0)
-    for _ in range(3):
-        x = mine.x0_m * (1 + 0.02 * rng.standard_normal(3)); u = mine.u0 * (1 + 0.01 * rng.standard_normal(2))
-        d = np.array([0.1 * rng.standard_normal(), 0.1 + 0.02 * rng.standard_normal()]); t = float(rng.uniform(0, 30))
-        a = np.asarray(ref.Fx_model(x, u, 0.2, d, t, np.zeros(3))); b = np.asarray(mine.Fx_model(x, u, 0.2, d, t, np.zeros(3)))
-        assert np.array_equal(a, b)
-        a = np.asarray(ref.Fx_p(x, u, np.zeros(3), t, 0.2, np.zeros(3))); b = np.asarray(mine.Fx_p(x, u, np.zeros(3), t, 0.2, np.zeros(3)))
-        assert np.array_equal(a, b)
-    sa, oa = make_specs(ref); sb, ob = nmpc.ss, nmpc.ocp
-    assert np.array_equal(oa.w_lb, ob.w_lb) and np.array_equal(oa.w_ub, ob.w_ub) and np.array_equal(oa.g_lb, ob.g_lb)
-    assert np.array_equal(oa.g_ub, ob.g_ub) and oa.off == ob.off and sa.off == sb.off
-    assert np.array_equal(sa.w_lb, sb.w_lb) and np.array_equal(sa.w_ub, sb.w_ub)
+        assert ref[name] == rec[name]
+    assert ref["flags"] == rec["flags"]
+    for pt, ev_ref in zip(ref["points"], ref["evals"]):
+        ev = evaluate(mine, pt)
+        assert np.array_equal(ev_ref["Fx_model"], ev["Fx_model"]) and np.array_equal(ev_ref["Fx_p"], ev["Fx_p"])
+    oa, ob = ref["ocp"], rec["ocp"]
+    assert np.array_equal(oa["w_lb"], ob["w_lb"]) and np.array_equal(oa["w_ub"], ob["w_ub"]) and np.array_equal(oa["g_lb"], ob["g_lb"])
+    assert np.array_equal(oa["g_ub"], ob["g_ub"]) and oa["off"] == ob["off"] and ref["ss"]["off"] == rec["ss"]["off"]
+    assert np.array_equal(ref["ss"]["w_lb"], rec["ss"]["w_lb"]) and np.array_equal(ref["ss"]["w_ub"], rec["ss"]["w_ub"])
     for k in ("Q", "R", "P0"):
-        assert np.array_equal(ref.estimator[k], mine.estimator[k])
+        assert np.array_equal(ref["estimator"][k], rec["estimator"][k])
 
 
 @pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")

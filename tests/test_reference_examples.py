@@ -1,19 +1,16 @@
-"""Every example file the reference ships, loaded UNMODIFIED from /root/reference (skipped where that checkout
-does not exist, e.g. on the GPU box): the device code (run on the CPU through the harness) must reproduce the oracle's
-closed loop - same IPOPT statuses and iteration counts, trajectories to 1e-6.
+"""Every example file the reference ships, through its restatement under examples/ (test_examples_equivalence.py pins
+each restatement to the unmodified file): the device code (run on the CPU through the harness) must reproduce the
+oracle's closed loop - same IPOPT statuses and iteration counts, trajectories to 1e-6.
 
 Covers what the four BASELINE configurations do not: a discrete-time model with `if_else` clamps, Delta-u bounds and
 a user terminal cost (Ex_NMPC_dis.py), nx != nxp (Ex_LMPCxp_nlplant.py), linear model on a nonlinear plant."""
-import os
-
 import numpy as np
 import pytest
 
-import __graft_entry__ as entry
-from conftest import REFERENCE, _bundle
+from conftest import _bundle
+from problem_record import PAIRS
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present")
-
+RESTATED = {fname: name for name, fname, _ in PAIRS}
 CASES = [("Ex_NMPC_dis.py", 6, ()), ("Ex_LMPC_nlplant.py", 8, ()), ("Ex_LMPCxp_nlplant.py", 8, ()),
          ("Ex_LMPC_CSTR.py", 6, ()), ("Ex_LMPC_WB.py", 6, ()), ("Ex_NMPC.py", 4, ())]
 
@@ -22,9 +19,7 @@ CASES = [("Ex_NMPC_dis.py", 6, ()), ("Ex_LMPC_nlplant.py", 8, ()), ("Ex_LMPCxp_n
 def test_reference_file_closed_loop(fname, nsteps, edits):
     from harness_loop import HarnessLoop
     from oracle.closed_loop import OracleLoop
-    name = "ref_" + fname[3:-3].lower()
-    entry.EXAMPLES[name] = os.path.join(REFERENCE, fname)
-    b = _bundle(name)
+    b = _bundle(RESTATED[fname])
     p = b.prob
     ref = OracleLoop(p, b.ss, b.ocp, b.oracle).run(Nsim=nsteps)
     rec = HarnessLoop(b, 1).run(nsteps)

@@ -1,4 +1,4 @@
-import sys, time; sys.path.insert(0, '/root/repo')
+import os, sys, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import __graft_entry__ as entry
 from mpc_code_b200.mpc_loop import CompiledProblem

@@ -1,6 +1,6 @@
 import os, sys, time
 import numpy as np, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from mpc_code_b200.mpc_loop import CompiledProblem
 prob, ss, ocp = bench._problem()
