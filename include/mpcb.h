@@ -97,6 +97,30 @@ int  mpcb_target(mpcb_handle_t h, const double* par_ss, double* wss, double* fss
  * par [B,npar]; w [B,nw] initial guess in, solution out; f [B]; status, iters [B]. */
 int  mpcb_ocp(mpcb_handle_t h, const double* par, double* w, double* f, int* status, int* iters, void* stream);
 
+/* Sensitivities of the OCP solution with respect to theta = [x_hat (nx) | x_s (nx) | u_s (nu) | u_{k-1} (nu)]
+ * (par[0 : 2nx+nu] and par[2nx+nu+nd : 2nx+2nu+nd]; ntheta = 2 (nx+nu)).  At the returned iterate of an instance the
+ * primal-dual barrier system F(v; theta) = 0 that the solver iterates on is differentiated (implicit function
+ * theorem, as sIPOPT does): bound multipliers and range-row slacks are condensed as in the Newton step (Sigma = Z/D,
+ * no regularisation) and x_0 is eliminated, so dw[0:nx] = dx_hat exactly.  Strongly active bounds therefore give
+ * derivatives of the order of the final barrier parameter, inactive ones the unconstrained derivative.  The
+ * parameters d, t, lambda, px, py are held constant.
+ *   mpcb_ocp_sens_size:   doubles per instance of the capture buffer `fac`.
+ *   mpcb_ocp_sens_factor: after mpcb_ocp on the same handle and with that call's par; factors the solution's KKT
+ *                         matrix (one Riccati sweep with delta_w = 0) and writes everything the sweeps need into
+ *                         fac [B, size].  status [B]: 0 computed; 1 the solve's status was not 0 or 1; 2 wrong inertia
+ *                         (some R~_k not positive definite, or a singular terminal-equality Gramian).  Any status
+ *                         other than 0 makes that instance's outputs of the sweeps NaN.  The solver's workspace is
+ *                         only read.
+ *   mpcb_ocp_jvp:         dw [B, ndir, nw] = J dtheta for dtheta [B, ndir, ntheta], J = d(w opt)/d(theta), in the
+ *                         caller's w layout.
+ *   mpcb_ocp_vjp:         gtheta [B, ntheta] = J' gw for gw [B, nw].
+ * The sweeps read only fac: their results do not depend on what the handle did after the factor call.  A problem
+ * whose ContForm cost integrand depends on theta cannot provide these derivatives: jvp / vjp return < 0. */
+long mpcb_ocp_sens_size(void);
+int  mpcb_ocp_sens_factor(mpcb_handle_t h, const double* par, double* fac, int* status, void* stream);
+int  mpcb_ocp_jvp(mpcb_handle_t h, const double* fac, int ndir, const double* dtheta, double* dw, void* stream);
+int  mpcb_ocp_vjp(mpcb_handle_t h, const double* fac, const double* gw, double* gtheta, void* stream);
+
 /* Plant measurement  y = Fy_p(x,u,pyp,t,pymp) + noise   (MPC_code.py:531-541); noise may be NULL. */
 int  mpcb_plant_meas(mpcb_handle_t h, const double* x, const double* u, const double* t, const double* pyp,
                      const double* pymp, const double* noise, double* y, void* stream);

@@ -19,7 +19,7 @@ INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 BUILD_DIR = os.path.join(PKG_DIR, "_build")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
-_SOURCES = ("mpcb_api.cu", "mpcb_device.cuh", "mpcb_ocp.cuh", "mpcb_target.cuh")
+_SOURCES = ("mpcb_api.cu", "mpcb_device.cuh", "mpcb_ocp.cuh", "mpcb_target.cuh", "mpcb_sens.cuh")
 
 
 def _nvcc() -> str:

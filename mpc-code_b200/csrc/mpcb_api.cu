@@ -11,6 +11,9 @@
 #include <vector>
 #include "mpcb.h"
 #include "mpcb_target.cuh"
+#if MPCB_HAS_OCP
+#include "mpcb_sens.cuh"
+#endif
 
 #define MPCB_NKERNELS 8
 enum { KC_OCP_INIT = 0, KC_OCP_EVAL = 1, KC_OCP_KKT = 2, KC_OCP_TRIAL = 3, KC_OCP_ACCEPT = 4, KC_TARGET = 5, KC_ESTIMATE = 6, KC_OTHER = 7 };
@@ -211,6 +214,44 @@ __global__ void EVAL_BOUNDS k_stage_derivs(int B, const double* par, const doubl
     for (int i = 0; i < NX * NU; ++i) Bm[s * NX * NU + i] = Bl[i];
     for (int i = 0; i < NX; ++i) c[s * NX + i] = xn[i] - wi[(k + 1) * NZ + i];
     for (int i = 0; i < NZP; ++i) H[s * NZP + i] = Hp[i];
+}
+
+// ---- sensitivities of the last OCP solve (mpcb_ocp_sens_factor / mpcb_ocp_jvp / mpcb_ocp_vjp) ----------------------
+// factor: the mapping of k_ocp_kkt (ocp_riccati runs on the same lanes and the same shared-memory scratch)
+__device__ __forceinline__ void sens_factor_inst(const double* ws, const double* par, InstState* st, double* fac, int* status,
+                                                 int inst, double* sm) {
+    OcpInst I = ocp_inst(const_cast<double*>(ws) + (size_t)inst * OcpLayout::total, nullptr, par + (size_t)inst * NPAR, st + inst);
+    const int r = ocp_sens_factor(I, fac + (size_t)inst * SensLayout::total, sm);
+    if ((threadIdx.x & (MPCB_KKT_LANES - 1)) == 0) status[inst] = r;
+}
+#if MPCB_KKT_LANES > 1
+__global__ void KKT_BOUNDS k_ocp_sens_factor(int B, const double* ws, const double* par, InstState* st, double* fac, int* status) {
+    constexpr int GROUPS = 32 * KKT_WARPS / MPCB_KKT_LANES;
+    __shared__ __align__(16) double scratch[GROUPS][KktScratch::total];
+    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) / MPCB_KKT_LANES;
+    if (inst >= B) return;
+    sens_factor_inst(ws, par, st, fac, status, inst, scratch[threadIdx.x / MPCB_KKT_LANES]);
+}
+#else
+__global__ void __launch_bounds__(32) k_ocp_sens_factor(int B, const double* ws, const double* par, InstState* st, double* fac, int* status) {
+    const int inst = blockIdx.x * blockDim.x + threadIdx.x;
+    if (inst >= B) return;
+    double scratch[KktScratch::total];
+    sens_factor_inst(ws, par, st, fac, status, inst, scratch);
+}
+#endif
+// JVP: one thread per (instance, direction); the directions of an instance sit on consecutive lanes, so their reads of
+// the instance's capture are broadcasts.  VJP: one thread per instance.
+__global__ void __launch_bounds__(128) k_ocp_jvp(int B, int ndir, const double* fac, const double* dth, double* dw) {
+    const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tid >= (long)B * ndir) return;
+    const long inst = tid / ndir;
+    sens_jvp_dir(fac + inst * SensLayout::total, dth + tid * NTH, dw + tid * NW);
+}
+__global__ void __launch_bounds__(128) k_ocp_vjp(int B, const double* fac, const double* gw, double* gth) {
+    const long inst = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (inst >= B) return;
+    sens_vjp_inst(fac + inst * SensLayout::total, gw + inst * NW, gth + inst * NTH);
 }
 #endif
 
@@ -844,6 +885,65 @@ int mpcb_ocp(mpcb_handle_t h, const double* par, double* w, double* f, int* stat
     }
     h->host_launches += 2;                       // init + output; the ticks are counted on the device (4-5 launches each)
     h->last_launches = -1; h->last_ticks = -1;   // known once the stream has run: see mpcb_last_ticks
+    return 0;
+#else
+    h->err = "library built without the OCP"; return -3;
+#endif
+}
+
+long mpcb_ocp_sens_size(void) {
+#if MPCB_HAS_OCP
+    return SensLayout::total;
+#else
+    return 0;
+#endif
+}
+
+// Reads the workspace of the handle's last mpcb_ocp (records, iterate, multipliers, per-instance status) and writes
+// only `fac` and `status`: the next solve starts from k_ocp_init exactly as without this call.
+int mpcb_ocp_sens_factor(mpcb_handle_t h, const double* par, double* fac, int* status, void* stream) {
+#if MPCB_HAS_OCP
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_ocp_sens_factor<<<KKT_GRID(h->B), 0, s>>>(h->B, h->ws, par, h->st, fac, status); }
+    CK(cudaGetLastError());
+    return 0;
+#else
+    h->err = "library built without the OCP"; return -3;
+#endif
+}
+
+#if MPCB_HAS_OCP
+static int sens_refuse(mpcb_ctx* h) {
+    if (!MPCB_SENS_CONT_DEP) return 0;
+    h->err = "OCP sensitivities: the ContForm cost integrand depends on the targets / initial state, whose mixed "
+             "derivatives through the integrator are not generated";
+    return -4;
+}
+#endif
+
+int mpcb_ocp_jvp(mpcb_handle_t h, const double* fac, int ndir, const double* dtheta, double* dw, void* stream) {
+#if MPCB_HAS_OCP
+    if (int rc = sens_refuse(h)) return rc;
+    if (ndir < 0) { h->err = "mpcb_ocp_jvp: ndir must be >= 0"; return -2; }
+    if (ndir == 0) return 0;
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_ocp_jvp<<<nblk((long)h->B * ndir, 128), 128, 0, s>>>(h->B, ndir, fac, dtheta, dw); }
+    CK(cudaGetLastError());
+    return 0;
+#else
+    h->err = "library built without the OCP"; return -3;
+#endif
+}
+
+int mpcb_ocp_vjp(mpcb_handle_t h, const double* fac, const double* gw, double* gtheta, void* stream) {
+#if MPCB_HAS_OCP
+    if (int rc = sens_refuse(h)) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_ocp_vjp<<<nblk(h->B, 128), 128, 0, s>>>(h->B, fac, gw, gtheta); }
+    CK(cudaGetLastError());
     return 0;
 #else
     h->err = "library built without the OCP"; return -3;

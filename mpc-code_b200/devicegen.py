@@ -140,6 +140,27 @@ def _discrete_functions(prefix: str, Fx_model: Function, nx, nu, nd, npx, nxi) -
     return fns
 
 
+def _sens_functions(o, D, ins_c, zz, stage_cost, rows) -> List[CFunction]:
+    """Mixed second derivatives for the OCP sensitivities (csrc/mpcb_sens.cuh): derivatives of the stage gradients, the
+    range rows and the terminal maps with respect to theta = [x0 | xs | us | um1] (the parameters fed in by the estimator,
+    the target problem and the previous input).  ContForm: the integrated cost has no generated mixed derivatives; when
+    it depends on theta the flag MPCB_SENS_CONT_DEP makes the sensitivity entry points refuse."""
+    par, off, n, m = o.par, o.off, o.n, o.m
+    th = vertcat(par[off["x0"]:off["us"] + m], par[off["um1"]:off["um1"] + m])
+    D["MPCB_NTH"] = 2 * (n + m)
+    D["MPCB_SENS_CONT_DEP"] = int(o.flags["ContForm"] is True and _depends_on(SX(o.quad_cost), th))
+    gc = gradient(stage_cost, zz)
+    fns = [CFunction("ocp_cost_dth", ins_c, [("Lt", jacobian(gc, th))]),
+           CFunction("ocp_term_dth", [("XN", o.XN), ("par", par)], [("Tt", jacobian(gradient(o.term_cost, o.XN), th))])]
+    if o.term_eq is not None:
+        fns.append(CFunction("ocp_termc_dth", [("XN", o.XN), ("par", par)], [("Rt", jacobian(o.term_eq, th))]))
+    if rows is not None:
+        R, mult = rows
+        fns.append(CFunction("ocp_out_dth", ins_c + [("mult", mult)],
+                             [("Yt", jacobian(R, th)), ("HYt", jacobian(gradient(mtimes(mult.T, R), zz), th))]))
+    return fns
+
+
 def generate_header(prob, ss_spec, ocp_spec, opts: Optional[Dict] = None) -> Dict[str, object]:
     """Return ``{"text": header_source, "defines": {...}, "flops": {...}}`` for one problem."""
     nx, nu, ny, nd, npx, npy, N = prob.nx, prob.nu, prob.ny, prob.nd, prob.npx, prob.npy, prob.N
@@ -276,6 +297,7 @@ def generate_header(prob, ss_spec, ocp_spec, opts: Optional[Dict] = None) -> Dic
             fns.append(CFunction("ocp_out_d", ins_y + [("mult", mult)],
                                  [("Y", R), ("JY", jacobian(R, zz)), ("HY", tril_pack(Hy))]))
             D["MPCB_OUT_LINEAR"] = int(all(e is S.ZERO for e in Hy.elements()))
+        fns += _sens_functions(o, D, ins_c, zz, stage_cost, rows=(R, mult) if n_rows else None)
     else:
         D["MPCB_HAS_OCP"] = 0
 

@@ -262,6 +262,15 @@ class BatchedMpc:
         self.ksim += 1
         return out
 
+    def feedback_gain(self):
+        """Local feedback law of the controller at the last `step()`: dU_0/dx_hat [B, nu, nx] of that step's OCP solve
+        (with Delta-u terms also dU_0/du_{k-1}, see `OcpSensitivity.feedback_gain`).  Not available after
+        `step_fused`, whose OCP parameters stay on the device."""
+        if self._fused:
+            raise RuntimeError("feedback_gain() after step_fused(): the fused step keeps its OCP parameters on the device; "
+                               "use step()")
+        return self.solver.sensitivity().feedback_gain()
+
     # -- the same step through the fused C entry point (mpcb_step): no host glue between the solves ----------
     def fused_reset(self):
         """Hand the current loop state to the device-resident loop of `mpcb_step`.  Only at the start of a run: the

@@ -1,0 +1,122 @@
+"""Sensitivities of the batched OCP solution with respect to theta = [x_hat | x_s | u_s | u_{k-1}].
+
+theta is the part of the OCP parameter vector that the closed loop feeds in from the estimator, the target problem and
+the previous input: ``par[0 : 2nx+nu]`` and ``par[2nx+nu+nd : 2nx+2nu+nd]`` (``ntheta = 2 (nx + nu)``).  The
+derivative is the implicit-function derivative of the barrier KKT system at the returned iterate (as sIPOPT computes
+it, see ``include/mpcb.h``): strongly active bounds give derivatives of the order of the final barrier parameter.
+
+* `OcpSensitivity` (from ``BatchedNlpSolver.sensitivity()``): JVP, VJP and the feedback gain dU_0/dx_hat.
+* `OcpLayer`: the solve as a differentiable function of theta for ``torch.autograd``.
+"""
+from __future__ import annotations
+
+
+def _torch():
+    import torch
+    return torch
+
+
+def theta_slices(nx: int, nu: int, nd: int):
+    """The two slices of ``par`` that make up theta."""
+    return slice(0, 2 * nx + nu), slice(2 * nx + nu + nd, 2 * nx + 2 * nu + nd)
+
+
+def theta_of(par, nx: int, nu: int, nd: int):
+    """theta [B, 2(nx+nu)] of OCP parameter vectors ``par`` [B, npar]."""
+    a, b = theta_slices(nx, nu, nd)
+    return _torch().cat([par[:, a], par[:, b]], dim=1)
+
+
+def with_theta(par, theta, nx: int, nu: int, nd: int):
+    """``par`` with its theta part replaced by ``theta`` (differentiable in both)."""
+    a, b = theta_slices(nx, nu, nd)
+    return _torch().cat([theta[:, :a.stop], par[:, a.stop:b.start], theta[:, a.stop:], par[:, b.stop:]], dim=1)
+
+
+class OcpSensitivity:
+    """Captured sensitivities of one batched OCP solve.  ``status`` [B] (int32, device): 0 computed, 1 the solve ended
+    with a status other than 0 / 1, 2 wrong inertia of the KKT matrix; every output of an instance with status != 0 is
+    NaN.  The capture ``fac`` belongs to this object, so results do not change when the handle solves again."""
+
+    def __init__(self, handle, fac, status, uses_uprev: bool):
+        self.handle, self.fac, self.status, self.uses_uprev = handle, fac, status, uses_uprev
+        d = handle.lib.dims
+        self.nx, self.nu, self.nd, self.ntheta = d.nx, d.nu, d.nd, handle.ntheta
+
+    def jvp(self, dtheta):
+        """dw [B, ndir, nw] for dtheta [B, ndir, ntheta]; a [B, ntheta] input gives [B, nw]."""
+        dw = self.handle.ocp_jvp(self.fac, dtheta)
+        return dw[:, 0] if getattr(dtheta, "ndim", 3) == 2 else dw
+
+    def vjp(self, gw):
+        """gtheta [B, ntheta] = (dw/dtheta)' gw for gw [B, nw]."""
+        return self.handle.ocp_vjp(self.fac, gw)
+
+    def feedback_gain(self):
+        """dU_0/dx_hat [B, nu, nx], the local feedback law of the controller; with Delta-u terms (u_{k-1} carried as
+        state) also dU_0/du_{k-1} [B, nu, nu], returned as a second tensor."""
+        torch = _torch()
+        nx, nu, B = self.nx, self.nu, self.handle.batch
+        cols = list(range(nx)) + (list(range(2 * nx + nu, 2 * nx + 2 * nu)) if self.uses_uprev else [])
+        E = torch.zeros(len(cols), self.ntheta, dtype=torch.float64, device=self.handle.device)
+        E[torch.arange(len(cols)), torch.tensor(cols)] = 1.0
+        dw = self.handle.ocp_jvp(self.fac, E.expand(B, -1, -1))
+        du0 = dw[:, :, nx:nx + nu].transpose(1, 2).contiguous()          # [B, nu, ndir]
+        return (du0[:, :, :nx].contiguous(), du0[:, :, nx:].contiguous()) if self.uses_uprev else du0
+
+
+class OcpLayer:
+    """``w = OcpLayer(solver)(theta, par, w0)``: the batched OCP solve as a function of theta, differentiable through
+    ``torch.autograd`` (backward = one VJP sweep on the captured factorisation).  theta is the only differentiable
+    input: ``par`` supplies the other parameters (its theta part is replaced) and ``w0`` is the initial guess; neither
+    may require grad.  Once differentiable (the backward pass is not itself differentiable)."""
+
+    def __init__(self, solver, lbx=None, ubx=None, lbg=None, ubg=None):
+        if solver.kind != "ocp":
+            raise NotImplementedError("OcpLayer wraps the dynamic OCP solver")
+        self.solver, self.bounds = solver, dict(lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg)
+        self.last = None                # OcpSensitivity of the last forward pass
+
+    def __call__(self, theta, par, w0):
+        for name, t in (("par", par), ("w0", w0)):
+            if getattr(t, "requires_grad", False):
+                raise ValueError("OcpLayer differentiates with respect to theta only: %s must not require grad "
+                                 "(sensitivities with respect to d, t, lambda, px, py are not available)" % name)
+        return _ocp_function().apply(theta, par, w0, self)
+
+
+def _make_function():
+    torch = _torch()
+    from torch.autograd.function import once_differentiable
+
+    class OcpFunction(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, theta, par, w0, layer):
+            h = layer.solver.handle
+            d = h.lib.dims
+            p = with_theta(h.tensor(par, d.npar), theta.detach().to(h.device, torch.float64), d.nx, d.nu, d.nd)
+            sol = layer.solver(x0=w0, p=p, **layer.bounds)
+            sens = layer.solver.sensitivity()
+            layer.last = sens
+            ctx.sens = sens
+            ctx.dtype, ctx.device = theta.dtype, theta.device
+            return sol["x"]
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, gw):
+            g = ctx.sens.vjp(gw.contiguous())
+            return g.to(device=ctx.device, dtype=ctx.dtype), None, None, None
+
+    return OcpFunction
+
+
+_FUNCTION = None
+
+
+def _ocp_function():
+    """The autograd Function, defined on first use (the package imports torch lazily)."""
+    global _FUNCTION
+    if _FUNCTION is None:
+        _FUNCTION = _make_function()
+    return _FUNCTION

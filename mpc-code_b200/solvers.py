@@ -35,7 +35,8 @@ C_SYMBOLS = ("mpcb_abi_version", "mpcb_default_opts", "mpcb_get_dims", "mpcb_mod
              "mpcb_destroy", "mpcb_last_error", "mpcb_set_const", "mpcb_estimate", "mpcb_target", "mpcb_ocp",
              "mpcb_plant_meas", "mpcb_plant_step", "mpcb_model_output", "mpcb_model_step", "mpcb_stage_derivs",
              "mpcb_last_launches", "mpcb_last_ticks", "mpcb_total_launches", "mpcb_set_groups", "mpcb_set_policy", "mpcb_set_profiling", "mpcb_get_profile", "mpcb_dfma_peak",
-             "mpcb_loop_reset", "mpcb_step", "mpcb_loop_get")
+             "mpcb_loop_reset", "mpcb_step", "mpcb_loop_get",
+             "mpcb_ocp_sens_size", "mpcb_ocp_sens_factor", "mpcb_ocp_jvp", "mpcb_ocp_vjp")
 
 
 class MpcbLibrary:
@@ -75,6 +76,10 @@ class MpcbLibrary:
         L.mpcb_loop_reset.argtypes = [vp] * 5
         L.mpcb_step.argtypes = [vp, ci] + [vp] * 15
         L.mpcb_loop_get.argtypes = [vp] * 5
+        L.mpcb_ocp_sens_size.restype = ctypes.c_long
+        L.mpcb_ocp_sens_factor.argtypes = [vp] * 5
+        L.mpcb_ocp_jvp.argtypes = [vp, vp, ci, vp, vp, vp]
+        L.mpcb_ocp_vjp.argtypes = [vp] * 5
         self.dims = MpcbDims()
         L.mpcb_get_dims(ctypes.byref(self.dims))
 
@@ -110,6 +115,7 @@ class MpcbHandle:
                 setattr(tgt, k, v)
         self.opts_ss, self.opts_dyn = oss, ody
         self._h = ctypes.c_void_p()
+        self.ocp_solves = 0             # OCP solves made through the handle (mpcb_ocp and the fused step): they reuse one workspace
         with torch.cuda.device(self.device):
             rc = self.L.mpcb_create(self.batch, ctypes.byref(oss), ctypes.byref(ody), ctypes.byref(self._h))
         self._check(rc)
@@ -163,7 +169,43 @@ class MpcbHandle:
         par = self.tensor(par, d.npar); w = self.tensor(w, d.nw).clone()
         f = self.empty(self.batch); st = self.empty(self.batch, dtype=torch.int32); it = self.empty(self.batch, dtype=torch.int32)
         self._check(self.L.mpcb_ocp(self._h, par.data_ptr(), w.data_ptr(), f.data_ptr(), st.data_ptr(), it.data_ptr(), self._stream()))
+        self.ocp_solves += 1
         return w, f, st, it
+
+    # -- sensitivities of the last OCP solve (include/mpcb.h, mpcb_ocp_sens_factor) -------------------------------
+    @property
+    def ntheta(self) -> int:
+        d = self.lib.dims
+        return 2 * (d.nx + d.nu)
+
+    def ocp_sens_factor(self, par):
+        """Capture of the sensitivities of the last `ocp` solve (``par`` must be that call's): ``(fac [B, size], status [B])``."""
+        torch = _torch()
+        par = self.tensor(par, self.lib.dims.npar)
+        fac = self.empty(self.batch, int(self.L.mpcb_ocp_sens_size()))
+        st = self.empty(self.batch, dtype=torch.int32)
+        self._check(self.L.mpcb_ocp_sens_factor(self._h, par.data_ptr(), fac.data_ptr(), st.data_ptr(), self._stream()))
+        return fac, st
+
+    def ocp_jvp(self, fac, dtheta):
+        """dw [B, ndir, nw] = J dtheta for dtheta [B, ndir, ntheta] (or [B, ntheta]: one direction)."""
+        d = self.lib.dims
+        dt = self.tensor(dtheta)
+        if dt.ndim == 2:
+            dt = dt.unsqueeze(1)
+        if dt.ndim != 3 or dt.shape[0] != self.batch or dt.shape[2] != self.ntheta:
+            raise ValueError("dtheta must be [B, ndir, %d], got %s" % (self.ntheta, tuple(dt.shape)))
+        dt = dt.contiguous()
+        dw = self.empty(self.batch, dt.shape[1], d.nw)
+        self._check(self.L.mpcb_ocp_jvp(self._h, fac.data_ptr(), int(dt.shape[1]), dt.data_ptr(), dw.data_ptr(), self._stream()))
+        return dw
+
+    def ocp_vjp(self, fac, gw):
+        """gtheta [B, ntheta] = J' gw for gw [B, nw]."""
+        gw = self.tensor(gw, self.lib.dims.nw)
+        g = self.empty(self.batch, self.ntheta)
+        self._check(self.L.mpcb_ocp_vjp(self._h, fac.data_ptr(), gw.data_ptr(), g.data_ptr(), self._stream()))
+        return g
 
     def target(self, par_ss, wss):
         torch = _torch()
@@ -248,6 +290,7 @@ class MpcbHandle:
         px = self.tensor(px, d.npx * d.N) if px is not None else None
         py = self.tensor(py, d.npy * d.N) if py is not None else None
         o = self._step_out
+        self.ocp_solves += 1
         self._check(self.L.mpcb_step(self._h, int(est_type), y.data_ptr(), t.data_ptr(), sp.data_ptr(),
                                      px.data_ptr() if px is not None else None, py.data_ptr() if py is not None else None,
                                      o["u"].data_ptr(), o["xhat"].data_ptr(), o["dhat"].data_ptr(), o["xs"].data_ptr(),
@@ -310,6 +353,7 @@ class BatchedNlpSolver:
         self.kind, self.spec = kind, spec
         self.handle: Optional[MpcbHandle] = None
         self._last = None
+        self._last_ocp = None           # (par, handle solve count) of the last OCP call, for sensitivity()
         self._bounds_key = None
 
     def attach(self, handle: MpcbHandle):
@@ -366,11 +410,29 @@ class BatchedNlpSolver:
         self._require()
         self._push_bounds(lbx, ubx, lbg, ubg)
         if self.kind == "ocp":
-            x, f, st, it = self.handle.ocp(p, x0)
+            par = self.handle.tensor(p, self.handle.lib.dims.npar)
+            x, f, st, it = self.handle.ocp(par, x0)
+            self._last_ocp = (par, self.handle.ocp_solves)
         else:
             x, f, st, it = self.handle.target(p, x0)
         self._last = (st, it)
         return {"x": x, "f": f}
+
+    def sensitivity(self):
+        """Sensitivities of the last solve with respect to theta = [x_hat | x_s | u_s | u_{k-1}] (see
+        `mpc_code_b200.sensitivity`): an `OcpSensitivity` that owns its capture and stays valid after later solves.
+        Must be called before the handle solves another OCP, with the solve's ``p`` not modified in place since."""
+        if self.kind != "ocp":
+            raise NotImplementedError("sensitivities are available for the dynamic OCP only, not the target problem")
+        self._require()
+        if self._last_ocp is None:
+            raise RuntimeError("sensitivity() before the first solve")
+        par, solves = self._last_ocp
+        if solves != self.handle.ocp_solves:
+            raise RuntimeError("the handle has solved another OCP since this solver's last call: its workspace is gone")
+        from .sensitivity import OcpSensitivity
+        fac, st = self.handle.ocp_sens_factor(par)
+        return OcpSensitivity(self.handle, fac, st, uses_uprev=bool(self.spec.uses_uprev))
 
     def stats(self):
         if self._last is None:

@@ -1,0 +1,70 @@
+"""Cost of the OCP sensitivities on the GPU, against the solve they belong to (Ex_NMPC, B = 4096 by default).
+
+CUDA events around, after warm-up: the batched mpcb_ocp solve, mpcb_ocp_sens_factor, the full theta-Jacobian (one JVP
+of all ntheta unit directions) and one VJP; the median of --reps repetitions each.  Prints the card name and power
+limit read in the same run.  Usage: python tools/sens_timing.py [--batch 4096] [--reps 20]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--batch", type=int, default=4096)
+    ap.add_argument("--reps", type=int, default=20)
+    a = ap.parse_args()
+    import torch
+    import __graft_entry__ as entry
+    from mpc_code_b200.mpc_loop import CompiledProblem
+    from mpc_code_b200.solvers import BatchedNlpSolver, MpcbHandle
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
+                          capture_output=True, text=True).stdout.strip().splitlines()
+    prob, ss, ocp = entry._problem("nmpc_cstr")
+    cp = CompiledProblem(prob, "nmpc_cstr")
+    G = np.load(os.path.join(ROOT, "tests", "golden", "nmpc_oracle.npz"))
+    B = a.batch
+    rng = np.random.default_rng(0)
+    par = G["ocp_par"][np.arange(B) % G["ocp_par"].shape[0]].copy()
+    par[:, :2 * prob.nx] *= 1 + 0.002 * rng.uniform(-1, 1, (B, 2 * prob.nx))
+    h = MpcbHandle(cp.library, B)
+    solver = BatchedNlpSolver("ocp", cp.ocp_spec).attach(h)
+    par_t = h.tensor(par, prob.npar)
+    w0 = h.tensor(G["ocp_w0"], prob.nw)
+    nth = h.ntheta
+    eye = torch.eye(nth, dtype=torch.float64, device=h.device).expand(B, -1, -1).contiguous()
+    gw = torch.as_tensor(rng.standard_normal((B, prob.nw)), device=h.device)
+
+    def timed(fn):
+        out = []
+        for _ in range(a.reps):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(); fn(); e1.record(); torch.cuda.synchronize()
+            out.append(e0.elapsed_time(e1))
+        return float(np.median(out))
+
+    solver(x0=w0, p=par_t)                                   # warm-up: graph build, module load
+    sens = solver.sensitivity(); sens.jvp(eye); sens.vjp(gw); torch.cuda.synchronize()
+    t_solve = timed(lambda: solver(x0=w0, p=par_t))
+    solver(x0=w0, p=par_t)
+    t_factor = timed(lambda: h.ocp_sens_factor(par_t))
+    fac, st = h.ocp_sens_factor(par_t)
+    t_jac = timed(lambda: h.ocp_jvp(fac, eye))
+    t_vjp = timed(lambda: h.ocp_vjp(fac, gw))
+    res = dict(card=card, problem="nmpc_cstr (Ex_NMPC)", batch=B, ntheta=nth, reps=a.reps,
+               sens_status_counts={int(k): int(v) for k, v in zip(*np.unique(st.cpu().numpy(), return_counts=True))},
+               solve_ms=t_solve, factor_ms=t_factor, jacobian_ms=t_jac, vjp_ms=t_vjp,
+               factor_plus_jacobian_over_solve=(t_factor + t_jac) / t_solve, vjp_over_solve=t_vjp / t_solve,
+               factor_plus_vjp_over_solve=(t_factor + t_vjp) / t_solve)
+    print(json.dumps(res, indent=1))
+
+
+if __name__ == "__main__":
+    main()
