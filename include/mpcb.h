@@ -121,6 +121,27 @@ int  mpcb_ocp_sens_factor(mpcb_handle_t h, const double* par, double* fac, int* 
 int  mpcb_ocp_jvp(mpcb_handle_t h, const double* fac, int ndir, const double* dtheta, double* dw, void* stream);
 int  mpcb_ocp_vjp(mpcb_handle_t h, const double* fac, const double* gw, double* gtheta, void* stream);
 
+/* Sensitivities of the OCP solution with respect to the parameters that enter the dynamics,
+ *   p = [d (nd) | px_0 .. px_{N-1} (npx N) | py_0 .. py_{N-1} (npy N)] = par[2nx+nu : 2nx+nu+nd] ++ par[off_px : npar]
+ * (n_p = nd + (npx+npy) N; off_px = 2nx+2nu+nd+1+ny*nu).  The same derivative as above (theta held constant, t and
+ * lambda too); p enters the model's state map, so the sweeps carry the defects (dF_k/dp_k) dp_k of the dynamics rows.
+ *   mpcb_ocp_sens_size_p:   doubles per instance of the capture of mpcb_ocp_sens_factor_p.
+ *   mpcb_ocp_sens_factor_p: as mpcb_ocp_sens_factor (same status), into fac [B * size_p]: the first B * size doubles
+ *                           are exactly what mpcb_ocp_sens_factor writes, so the theta entry points accept this
+ *                           capture; the derivative blocks of p follow.  Element 1 of an instance's theta capture
+ *                           is set to 1 to mark that its p-blocks are present.
+ *   mpcb_ocp_jvp_p:         dw [B, ndir, nw] = J_p dp for dp [B, ndir, n_p].
+ *   mpcb_ocp_vjp_p:         gp [B, n_p] = J_p' gw for gw [B, nw].
+ * The p sweeps write NaN for an instance whose status is not 0 and for one whose capture has no p-blocks (element 1
+ * of its theta capture is not 1, e.g. a zero-filled buffer of size_p that only mpcb_ocp_sens_factor wrote).
+ * mpcb_ocp_sens_factor does not clear that mark: refresh a p capture with mpcb_ocp_sens_factor_p.  A ContForm problem,
+ * a large model on the dense derivative path (MPCB_DENSE_SH) or a stage map that reads another stage's px / py through
+ * par cannot provide the p-blocks (decided at code generation): the three p entry points return < 0. */
+long mpcb_ocp_sens_size_p(void);
+int  mpcb_ocp_sens_factor_p(mpcb_handle_t h, const double* par, double* fac, int* status, void* stream);
+int  mpcb_ocp_jvp_p(mpcb_handle_t h, const double* fac, int ndir, const double* dp, double* dw, void* stream);
+int  mpcb_ocp_vjp_p(mpcb_handle_t h, const double* fac, const double* gw, double* gp, void* stream);
+
 /* Plant measurement  y = Fy_p(x,u,pyp,t,pymp) + noise   (MPC_code.py:531-541); noise may be NULL. */
 int  mpcb_plant_meas(mpcb_handle_t h, const double* x, const double* u, const double* t, const double* pyp,
                      const double* pymp, const double* noise, double* y, void* stream);

@@ -253,6 +253,31 @@ __global__ void __launch_bounds__(128) k_ocp_vjp(int B, const double* fac, const
     if (inst >= B) return;
     sens_vjp_inst(fac + inst * SensLayout::total, gw + inst * NW, gth + inst * NTH);
 }
+#if MPCB_SENS_P
+// p-blocks: one thread per (instance, stage k = 0..NH), the mapping of k_ocp_eval (k = NH: the terminal blocks).  The
+// generated derivative code runs on independent threads, not on the lanes of a per-instance warp.
+__global__ void __launch_bounds__(128) k_ocp_sens_pblocks(int B, const double* ws, const double* par, InstState* st, double* fac) {
+    const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tid >= (long)B * (NH + 1)) return;
+    const long inst = tid / (NH + 1);
+    const int k = (int)(tid % (NH + 1));
+    OcpInst I = ocp_inst(const_cast<double*>(ws) + inst * OcpLayout::total, nullptr, par + inst * NPAR, st + inst);
+    ocp_sens_pblocks(I, k, fac + inst * SensLayout::total, fac + (long)B * SensLayout::total + inst * SensPLayout::total);
+}
+__global__ void __launch_bounds__(128) k_ocp_jvp_p(int B, int ndir, const double* fac, const double* dp, double* dw) {
+    const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tid >= (long)B * ndir) return;
+    const long inst = tid / ndir;
+    sens_jvp_p_dir(fac + inst * SensLayout::total, fac + (long)B * SensLayout::total + inst * SensPLayout::total,
+                   dp + tid * NPP, dw + tid * NW);
+}
+__global__ void __launch_bounds__(128) k_ocp_vjp_p(int B, const double* fac, const double* gw, double* gp) {
+    const long inst = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (inst >= B) return;
+    sens_vjp_p_inst(fac + inst * SensLayout::total, fac + (long)B * SensLayout::total + inst * SensPLayout::total,
+                    gw + inst * NW, gp + inst * NPP);
+}
+#endif
 #endif
 
 #if MPCB_HAS_TARGET
@@ -944,6 +969,71 @@ int mpcb_ocp_vjp(mpcb_handle_t h, const double* fac, const double* gw, double* g
     h->host_launches += 1;
     { Prof p(h, s, KC_OTHER); k_ocp_vjp<<<nblk(h->B, 128), 128, 0, s>>>(h->B, fac, gw, gtheta); }
     CK(cudaGetLastError());
+    return 0;
+#else
+    h->err = "library built without the OCP"; return -3;
+#endif
+}
+
+long mpcb_ocp_sens_size_p(void) {
+#if MPCB_HAS_OCP
+    return SensLayout::total + SensPLayout::total;
+#else
+    return 0;
+#endif
+}
+
+#if MPCB_HAS_OCP
+static int sens_p_refuse(mpcb_ctx* h) {
+    if (MPCB_SENS_P) return 0;
+    h->err = "OCP sensitivities with respect to d / px / py are not generated for this problem (ContForm, or a large "
+             "model on the dense derivative path, or a stage map that reads another stage's px / py)";
+    return -4;
+}
+#endif
+
+int mpcb_ocp_sens_factor_p(mpcb_handle_t h, const double* par, double* fac, int* status, void* stream) {
+#if MPCB_HAS_OCP
+    if (int rc = sens_p_refuse(h)) return rc;
+#if MPCB_SENS_P
+    if (int rc = mpcb_ocp_sens_factor(h, par, fac, status, stream)) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_ocp_sens_pblocks<<<nblk((long)h->B * (NH + 1), 128), 128, 0, s>>>(h->B, h->ws, par, h->st, fac); }
+    CK(cudaGetLastError());
+#endif
+    return 0;
+#else
+    h->err = "library built without the OCP"; return -3;
+#endif
+}
+
+int mpcb_ocp_jvp_p(mpcb_handle_t h, const double* fac, int ndir, const double* dp, double* dw, void* stream) {
+#if MPCB_HAS_OCP
+    if (int rc = sens_p_refuse(h)) return rc;
+    if (ndir < 0) { h->err = "mpcb_ocp_jvp_p: ndir must be >= 0"; return -2; }
+    if (ndir == 0) return 0;
+#if MPCB_SENS_P
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_ocp_jvp_p<<<nblk((long)h->B * ndir, 128), 128, 0, s>>>(h->B, ndir, fac, dp, dw); }
+    CK(cudaGetLastError());
+#endif
+    return 0;
+#else
+    h->err = "library built without the OCP"; return -3;
+#endif
+}
+
+int mpcb_ocp_vjp_p(mpcb_handle_t h, const double* fac, const double* gw, double* gp, void* stream) {
+#if MPCB_HAS_OCP
+    if (int rc = sens_p_refuse(h)) return rc;
+#if MPCB_SENS_P
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_ocp_vjp_p<<<nblk(h->B, 128), 128, 0, s>>>(h->B, fac, gw, gp); }
+    CK(cudaGetLastError());
+#endif
     return 0;
 #else
     h->err = "library built without the OCP"; return -3;

@@ -188,7 +188,14 @@ MPCB_HD int ocp_sens_factor(const OcpInst& I, double* fac, double* sm) {
 // Solves the condensed KKT system for one right-hand side given by `src`:
 //   src.q(k, q)   stage gradient (NZA),  src.pN(p)  terminal gradient (NXA),  src.rT(r)  terminal-equality residual,
 //   src.z0(z)     fixed dz_0,            src.y(k, dz, du) / src.yN(dz)  receive the solution,  src.p0(p0)  costate of z_0
+// Sources with SensDefects<Src>::value (the p sweeps) also give the defect of the dynamics row of stage k and see the
+// multiplier of that row:
+//   src.c(k, c)   defect c_k (NXA):  dz_{k+1} = A_k dz_k + B_k du_k + c_k,
+//   src.keep(k, p)  the backward costate p_k (k = 1..NH),  src.lam(k, dz_{k+1}, nu)  after dz_{k+1} is known.
+// For the other sources the defect terms are not compiled: the theta sweeps keep their arithmetic.
 // Everything is read from fac; kk holds the feed-forward terms between the two sweeps.
+template <class Src> struct SensDefects { static constexpr bool value = false; };
+
 template <class Src>
 MPCB_HD void sens_sweep(const double* fac, Src& src, double* kk) {
     double p[NXA], q[NZA], nu[NXT + 1];
@@ -202,7 +209,19 @@ MPCB_HD void sens_sweep(const double* fac, Src& src, double* kk) {
         const double* F = fac + SensLayout::frec + k * FREC_SZ;
         const double* C = fac + SensLayout::chol + k * (NU * NU + NU);
         src.q(k, q);
-        for (int j = 0; j < NZA; ++j) { double a = q[j]; for (int l = 0; l < NXA; ++l) a += AB[l + NXA * j] * p[l]; q[j] = a; }
+        if constexpr (SensDefects<Src>::value) {
+            // V_{k+1}(A dz + B du + c) contributes [A|B]'(P_{k+1} c + p_{k+1}); c reaches dz_N like B kf does
+            double c[NXA], pc[NXA];
+            src.keep(k + 1, p);
+            src.c(k, c);
+            for (int i = 0; i < NXA; ++i) { double a = p[i]; for (int m = 0; m < NXA; ++m) a += F[FREC_P + i + NXA * m] * c[m]; pc[i] = a; }
+            for (int j = 0; j < NZA; ++j) { double a = q[j]; for (int l = 0; l < NXA; ++l) a += AB[l + NXA * j] * pc[l]; q[j] = a; }
+#if MPCB_TERMCONS
+            for (int j = 0; j < NXT; ++j) { double a = h[j]; for (int l = 0; l < NXA; ++l) a += F[FREC_PI + l + NXA * j] * c[l]; h[j] = a; }
+#endif
+        } else {
+            for (int j = 0; j < NZA; ++j) { double a = q[j]; for (int l = 0; l < NXA; ++l) a += AB[l + NXA * j] * p[l]; q[j] = a; }
+        }
         double* kf = kk + k * NU;
         for (int i = 0; i < NU; ++i) kf[i] = q[NXA + i];
         sens_chol_solve<NU>(C, C + NU * NU, kf);
@@ -258,6 +277,12 @@ MPCB_HD void sens_sweep(const double* fac, Src& src, double* kk) {
             for (int j = 0; j < NXA; ++j) a += AB[i + NXA * j] * dz[j];
             for (int j = 0; j < NU; ++j) a += AB[NXA * NXA + i + NXA * j] * du[j];
             dn[i] = a;
+        }
+        if constexpr (SensDefects<Src>::value) {
+            double c[NXA];
+            src.c(k, c);
+            for (int i = 0; i < NXA; ++i) dn[i] += c[i];
+            src.lam(k, dn, nu);
         }
         for (int i = 0; i < NXA; ++i) dz[i] = dn[i];
     }
@@ -337,3 +362,262 @@ MPCB_HD void sens_vjp_inst(const double* fac, const double* gw, double* gth) {
     SensVjpSrc s{fac, gw, gth};
     sens_sweep(fac, s, kk);
 }
+
+// =====================================================================================================================
+// Sensitivities with respect to the parameters that enter the dynamics:
+//   p = [d (ND) | px_0 .. px_{NH-1} (NPX NH) | py_0 .. py_{NH-1} (NPY NH)] = par[OFF_D : OFF_D+ND] ++ par[OFF_PX : NPAR].
+// Stage k depends on p_k = [d; px_k; py_k] only (NPK columns), the terminal maps on d.  p enters the dynamics rows, so
+// the right-hand sides have defects c_k = Fp_k dp_k.  The capture of mpcb_ocp_sens_factor_p is the theta capture of
+// all B instances, unchanged, followed by the p-blocks of all B instances (SensPLayout each); fac[1] of an instance's
+// theta capture is 1 when its p-blocks were written.
+//   ocp_sens_pblocks  per (instance, stage k = 0..NH), the mapping of ocp_eval_stage: Fp_k, Qp_k, terminal d-blocks
+//   sens_jvp_p_dir    per (instance, direction): dw = J_p dp
+//   sens_vjp_p_inst   per instance: gp = J_p' gw
+// =====================================================================================================================
+#ifndef MPCB_SENS_P
+#define MPCB_SENS_P 0                     // 0: the problem cannot provide the p-blocks (decided by the generator)
+#endif
+#define NPK (ND + NPX + NPY)              // columns of p_k = [d; px_k; py_k]
+#define NPM (ND + NPX)                    // the model's parameters [d; px]: the first NPM columns of p_k
+#define NPP (ND + (NPX + NPY) * NH)       // n_p
+
+struct SensPLayout {                                                 // doubles per instance, after the B theta captures
+    static constexpr int fp = 0;                                     // NH * NXA*NPK  dF_k/dp_k (rows of v_k = u_{k-1}: 0)
+    static constexpr int qp = fp + NH * NXA * NPK;                   // NH * NZA*NPK  d(grad L_k)/dp_k + G'Sigma_s dR_k/dp_k
+    static constexpr int qt = qp + NH * NZA * NPK;                   // NXA*ND  d(grad V_f)/dd
+    static constexpr int rt = qt + NXA * ND;                         // NXT*ND  d(terminal equality)/dd
+    static constexpr int total = (rt + NXT * ND + 1) / 2 * 2;
+};
+
+// local column c of p_k -> index into p
+MPCB_HD int sens_p_index(int k, int c) {
+    return c < ND ? c : (c < NPM ? ND + k * NPX + (c - ND) : ND + NPX * NH + k * NPY + (c - NPM));
+}
+
+#if MPCB_SENS_P
+#if MPCB_DYN_RK4 && MPCB_SENS_NQ > 0
+// The model ODE on the augmented state [x; q], q' = 0: q holds the components MPCB_SENS_QIDX of [d; px] that the
+// right-hand side reads (the generated mdlp_* take them from the state, the rest from the context).  Run with the
+// adjoint seed [lam; 0], the RK4 sweeps of the solve give dx_N/dq in the q columns of S and the mixed Hessian of lam' x_N.
+#ifndef MPCB_MDLP_NC
+#define MPCB_MDLP_NC 0
+#endif
+#ifndef MPCB_MDLP_NR
+#define MPCB_MDLP_NR 0
+#endif
+struct SysModelP {
+    static constexpr int NS = NX + MPCB_SENS_NQ, NM = MX, NC = MPCB_MDLP_NC, NR = MPCB_MDLP_NR;
+    typedef ModelCtx Ctx;
+#if MPCB_MDLP_NC + MPCB_MDLP_NR > 0
+    MPCB_HDM void f_c(const double* x, const Ctx& c, double t, double* o, double* cache) { mdlp_f_c(x, c.u, c.d, &t, c.px, o, cache); }
+    MPCB_HDM void f_rc(const double* x, const Ctx& c, double t, const double* cache, double* o, double* rc) {
+        mdlp_f_rc(x, c.u, c.d, &t, c.px, cache, o, rc);
+    }
+    MPCB_HDM void f_rcp(const double* x, const Ctx& c, double t, const double* cache, double* rc) { mdlp_f_rcp(x, c.u, c.d, &t, c.px, cache, rc); }
+    MPCB_HDM void f_vjp_c(const double* x, const Ctx& c, double t, const double* nu, const double* cache, const double* rc, double* o) {
+        mdlp_f_vjp_c(x, c.u, c.d, &t, c.px, nu, cache, rc, o);
+    }
+    MPCB_HDM void f_sh_c(const double* x, const Ctx& c, double t, const double* S, const double* nu, const double* cache,
+                         const double* rc, double* o, double* K, double* Hc) {
+        mdlp_f_sh_c(x, c.u, c.d, &t, c.px, S, nu, cache, rc, o, K, Hc);
+    }
+#endif
+    MPCB_HDM void f(const double* x, const Ctx& c, double t, double* o) { mdlp_f(x, c.u, c.d, &t, c.px, o); }
+    MPCB_HDM void f_vjp(const double* x, const Ctx& c, double t, const double* nu, double* o) { mdlp_f_vjp(x, c.u, c.d, &t, c.px, nu, o); }
+    MPCB_HDM void f_sh(const double* x, const Ctx& c, double t, const double* S, const double* nu, double* o, double* K, double* Hc) {
+        mdlp_f_sh(x, c.u, c.d, &t, c.px, S, nu, o, K, Hc);
+    }
+};
+#endif
+
+// Fm = dx_{k+1}/d[d; px] (NX x NPM) and Hm = d(grad_{x,u} lam' x_{k+1})/d[d; px] (NZ x NPM), column-major
+MPCB_HD void sens_dyn_dp(const double* x, const double* u, const double* d, const double* px, double t0, const double* lam,
+                         double* Fm, double* Hm) {
+#if MPCB_DYN_RK4
+    for (int e = 0; e < NX * NPM; ++e) Fm[e] = 0.0;
+    for (int e = 0; e < NZ * NPM; ++e) Hm[e] = 0.0;
+#if MPCB_SENS_NQ > 0
+    {
+        constexpr int NQ = MPCB_SENS_NQ, NS = NX + NQ, NZS = NS + NU;
+        constexpr int qi[NQ] = MPCB_SENS_QIDX;
+        ModelCtx c; c.u = u; c.d = d; c.px = px;
+        double xt[NS], lt[NS], xe[NS], S[NS * NZS], Ht[NZS * (NZS + 1) / 2], lbuf[RkSize<SysModelP>::TOTAL];
+        for (int i = 0; i < NX; ++i) { xt[i] = x[i]; lt[i] = lam[i]; }
+        for (int j = 0; j < NQ; ++j) { xt[NX + j] = qi[j] < ND ? d[qi[j]] : px[qi[j] - ND]; lt[NX + j] = 0.0; }
+        for (int e = 0; e < NZS * (NZS + 1) / 2; ++e) Ht[e] = 0.0;
+        rk4_full_t<SysModelP>(xt, c, t0, lt, xe, S, Ht, RkBuf{lbuf, 1});
+        for (int j = 0; j < NQ; ++j) {
+            for (int i = 0; i < NX; ++i) Fm[i + NX * qi[j]] = S[i + NS * (NX + j)];
+            for (int r = 0; r < NZ; ++r) Hm[r + NZ * qi[j]] = Ht[tri(r < NX ? r : r + NQ, NX + j)];
+        }
+    }
+#endif
+    double Jp[NX * NPM + 1];
+    mdl_post_dp(d, px, Jp);
+    for (int e = 0; e < NX * NPM; ++e) Fm[e] += Jp[e];
+#else
+    mdl_F_dp(x, u, d, &t0, px, lam, Fm, Hm);
+#endif
+}
+
+// stage k: Fp (NXA x NPK) and Qp (NZA x NPK) at w*, with the multipliers the stage record was built with
+MPCB_HD void sens_p_stage(const OcpInst& I, int k, double* Fp, double* Qp) {
+    double z[NXA], u[NU], lam[NXA], d[ND + 1], px[NPX + 1], py[NPY + 1], t0;
+    for (int i = 0; i < NXA; ++i) { z[i] = I.w[k * NZA + i]; lam[i] = I.lam[k * NXA + i]; }
+    for (int i = 0; i < NU; ++i) u[i] = I.w[k * NZA + NXA + i];
+    stage_params(I.par, k, d, px, py, &t0);
+    ocp_cost_dp(z, u, I.par, px, py, Qp);
+#if NG > 0
+    {
+        double Yp[NG * NPK], HYp[NZA * NPK];
+        ocp_out_dp(z, u, I.par, px, py, I.ym + k * NG, Yp, HYp);
+        const double* R = I.rec + k * REC_SZ;
+        for (int c = 0; c < NPK; ++c)
+            for (int j = 0; j < NZA; ++j) {
+                double a = HYp[j + NZA * c];
+                for (int r = 0; r < NG; ++r) a += R[R_G + r + NG * j] * R[R_SG + r] * Yp[r + NG * c];
+                Qp[j + NZA * c] += a;
+            }
+    }
+#endif
+    double Fm[NX * NPM + 1], Hm[NZ * NPM + 1];
+    sens_dyn_dp(z, u, d, px, t0, lam, Fm, Hm);
+    for (int e = 0; e < NXA * NPK; ++e) Fp[e] = 0.0;
+    for (int c = 0; c < NPM; ++c) {
+        for (int i = 0; i < NX; ++i) Fp[i + NXA * c] = Fm[i + NX * c];
+        for (int r = 0; r < NZ; ++r) Qp[(r < NX ? r : r + NAUG) + NZA * c] += Hm[r + NZ * c];     // model (x, u) -> (x, v, u)
+    }
+}
+
+// terminal: d(grad V_f)/dd (NXA x ND) and d(r_T)/dd (NXT x ND)
+MPCB_HD void sens_p_term(const OcpInst& I, double* QT, double* RT) {
+    double Tp[NX * ND + 1];
+    ocp_term_dp(I.w + NH * NZA, I.par, Tp);
+    for (int c = 0; c < ND; ++c)
+        for (int i = 0; i < NXA; ++i) QT[i + NXA * c] = i < NX ? Tp[i + NX * c] : 0.0;
+#if MPCB_TERMCONS
+    ocp_termc_dp(I.w + NH * NZA, I.par, RT);
+#else
+    (void)RT;
+#endif
+}
+
+// one (instance, k) of the p-blocks: fac = the instance's theta capture, pb = its p-blocks
+MPCB_HD void ocp_sens_pblocks(const OcpInst& I, int k, double* fac, double* pb) {
+    const int solve_status = I.st->status;
+    if (solve_status == 0 || solve_status == 1) {
+        if (k < NH) sens_p_stage(I, k, pb + SensPLayout::fp + k * NXA * NPK, pb + SensPLayout::qp + k * NZA * NPK);
+        else sens_p_term(I, pb + SensPLayout::qt, pb + SensPLayout::rt);
+    }
+    if (k == 0) fac[1] = 1.0;
+}
+
+// JVP: q_k = Qp_k dp_k, c_k = Fp_k dp_k, p_N = QT dd, r_T = RT dd, dz_0 = 0; writes dw (caller's layout, NW)
+struct SensJvpPSrc {
+    const double* pb; const double* dp; double* dw;
+    SENS_M void loc(int k, double* v) const { for (int c = 0; c < NPK; ++c) v[c] = dp[sens_p_index(k, c)]; }
+    SENS_M void q(int k, double* q) const {
+        const double* Q = pb + SensPLayout::qp + k * NZA * NPK;
+        double v[NPK];
+        loc(k, v);
+        for (int j = 0; j < NZA; ++j) { double a = 0.0; for (int c = 0; c < NPK; ++c) a += Q[j + NZA * c] * v[c]; q[j] = a; }
+    }
+    SENS_M void c(int k, double* cv) const {
+        const double* Fp = pb + SensPLayout::fp + k * NXA * NPK;
+        double v[NPK];
+        loc(k, v);
+        for (int i = 0; i < NXA; ++i) { double a = 0.0; for (int c = 0; c < NPK; ++c) a += Fp[i + NXA * c] * v[c]; cv[i] = a; }
+    }
+    SENS_M void pN(double* p) const {
+        const double* Q = pb + SensPLayout::qt;
+        for (int j = 0; j < NXA; ++j) { double a = 0.0; for (int c = 0; c < ND; ++c) a += Q[j + NXA * c] * dp[c]; p[j] = a; }
+    }
+    SENS_M void rT(double* r) const {
+        const double* Q = pb + SensPLayout::rt;
+        for (int j = 0; j < NXT; ++j) { double a = 0.0; for (int c = 0; c < ND; ++c) a += Q[j + NXT * c] * dp[c]; r[j] = a; }
+    }
+    SENS_M void z0(double* z) const { for (int i = 0; i < NXA; ++i) z[i] = 0.0; }
+    SENS_M void p0(const double*) const {}
+    SENS_M void keep(int, const double*) const {}
+    SENS_M void lam(int, const double*, const double*) const {}
+    SENS_M void y(int k, const double* dz, const double* du) const {
+        for (int i = 0; i < NX; ++i) dw[k * NZ + i] = dz[i];
+        for (int i = 0; i < NU; ++i) dw[k * NZ + NX + i] = du[i];
+    }
+    SENS_M void yN(const double* dz, const double*) const { for (int i = 0; i < NX; ++i) dw[NH * NZ + i] = dz[i]; }
+};
+
+// VJP: the system with the gradient -gw and no defects; with its solution (y, lam^, nu)
+//   gp = -sum_k (Qp_k' y_k + Fp_k' lam^_k) - QT' y_N - RT' nu,   lam^_k = P_{k+1} dz_{k+1} + p_{k+1} + Pi_{k+1} nu,
+// the multiplier of the dynamics row of stage k (p_{k+1} of the backward sweep is kept per stage).
+struct SensVjpPSrc {
+    const double* fac; const double* pb; const double* gw; double* g; double* pk;      // pk: (NH + 1) * NXA
+    SENS_M void q(int k, double* q) const {
+        for (int i = 0; i < NXA; ++i) q[i] = i < NX ? -gw[k * NZ + i] : 0.0;
+        for (int i = 0; i < NU; ++i) q[NXA + i] = -gw[k * NZ + NX + i];
+    }
+    SENS_M void c(int, double* cv) const { for (int i = 0; i < NXA; ++i) cv[i] = 0.0; }
+    SENS_M void pN(double* p) const { for (int i = 0; i < NXA; ++i) p[i] = i < NX ? -gw[NH * NZ + i] : 0.0; }
+    SENS_M void rT(double* r) const { for (int j = 0; j < NXT; ++j) r[j] = 0.0; }
+    SENS_M void z0(double* z) const { for (int i = 0; i < NXA; ++i) z[i] = 0.0; }
+    SENS_M void p0(const double*) const {}
+    SENS_M void keep(int k, const double* p) const { for (int i = 0; i < NXA; ++i) pk[k * NXA + i] = p[i]; }
+    SENS_M void y(int k, const double* dz, const double* du) const {
+        const double* Q = pb + SensPLayout::qp + k * NZA * NPK;
+        for (int c = 0; c < NPK; ++c) {
+            double a = 0.0;
+            for (int j = 0; j < NXA; ++j) a += Q[j + NZA * c] * dz[j];
+            for (int j = 0; j < NU; ++j) a += Q[NXA + j + NZA * c] * du[j];
+            g[sens_p_index(k, c)] -= a;
+        }
+    }
+    SENS_M void lam(int k, const double* dn, const double* nu) const {
+        const double* F = fac + SensLayout::frec + k * FREC_SZ;
+        const double* Fp = pb + SensPLayout::fp + k * NXA * NPK;
+        double l[NXA];
+        for (int i = 0; i < NXA; ++i) {
+            double a = pk[(k + 1) * NXA + i];
+            for (int m = 0; m < NXA; ++m) a += F[FREC_P + i + NXA * m] * dn[m];
+#if MPCB_TERMCONS
+            for (int j = 0; j < NXT; ++j) a += F[FREC_PI + i + NXA * j] * nu[j];
+#else
+            (void)nu;
+#endif
+            l[i] = a;
+        }
+        for (int c = 0; c < NPK; ++c) {
+            double a = 0.0;
+            for (int i = 0; i < NXA; ++i) a += Fp[i + NXA * c] * l[i];
+            g[sens_p_index(k, c)] -= a;
+        }
+    }
+    SENS_M void yN(const double* dz, const double* nu) const {
+        const double* Q = pb + SensPLayout::qt; const double* R = pb + SensPLayout::rt;
+        for (int c = 0; c < ND; ++c) {
+            double a = 0.0;
+            for (int j = 0; j < NXA; ++j) a += Q[j + NXA * c] * dz[j];
+            for (int j = 0; j < NXT; ++j) a += R[j + NXT * c] * nu[j];
+            g[c] -= a;
+        }
+    }
+};
+template <> struct SensDefects<SensJvpPSrc> { static constexpr bool value = true; };
+template <> struct SensDefects<SensVjpPSrc> { static constexpr bool value = true; };
+
+MPCB_HD bool sens_p_valid(const double* fac) { return fac[SensLayout::head] == 0.0 && fac[1] == 1.0; }
+
+MPCB_HD void sens_jvp_p_dir(const double* fac, const double* pb, const double* dp, double* dw) {
+    if (!sens_p_valid(fac)) { for (int i = 0; i < NW; ++i) dw[i] = NAN; return; }
+    double kk[NH * NU];
+    SensJvpPSrc s{pb, dp, dw};
+    sens_sweep(fac, s, kk);
+}
+
+MPCB_HD void sens_vjp_p_inst(const double* fac, const double* pb, const double* gw, double* gp) {
+    if (!sens_p_valid(fac)) { for (int t = 0; t < NPP; ++t) gp[t] = NAN; return; }
+    for (int t = 0; t < NPP; ++t) gp[t] = 0.0;
+    double kk[NH * NU], pk[(NH + 1) * NXA];
+    SensVjpPSrc s{fac, pb, gw, gp, pk};
+    sens_sweep(fac, s, kk);
+}
+#endif  // MPCB_SENS_P

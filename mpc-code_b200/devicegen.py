@@ -161,6 +161,84 @@ def _sens_functions(o, D, ins_c, zz, stage_cost, rows) -> List[CFunction]:
     return fns
 
 
+def _sens_p_refusal(prob, o, stage_exprs) -> Optional[str]:
+    """Why the sensitivities with respect to p = [d | px | py] cannot be generated for this problem, or None."""
+    if o.flags["ContForm"] is True:
+        return "ContForm: the integrand would need its own augmented system"
+    if prob.Fx_model.meta.get("kind") == "rk4" and _use_dense(prob.nx, prob.nu):
+        return "large model (dense derivative products)"
+    par, off = o.par, o.off
+    rest = par[off["px"]:off["end"]] if off["end"] > off["px"] else None
+    if rest is not None and any(_depends_on(SX(e), rest) for e in stage_exprs):
+        return "a stage or terminal map reads px / py of another stage through par"
+    return None
+
+
+def _sens_p_functions(prob, o, D, ins_c, zz, stage_cost, rows) -> List[CFunction]:
+    """Mixed derivatives for the OCP sensitivities with respect to the parameters that enter the dynamics
+    (csrc/mpcb_sens.cuh, mpcb_ocp_sens_factor_p): stage k depends on p_k = [d; px_k; py_k] only, the terminal maps on d.
+
+    * dynamics, RK4: the right-hand side is integrated on the augmented state [x; q] with q' = 0, where q holds the
+      components of (d, px) that the right-hand side reads (MPCB_SENS_QIDX, indices into [d; px]).  The RK4 sweeps of the
+      solve then give dx_N/dq in the q columns of the sensitivity block and the mixed Hessian of lam' x_N in the packed
+      Hessian.  The map applied after the integration (Bd d + px) must be affine; its Jacobian is added.
+    * dynamics, discrete / linear: dF/d[d; px] and d(grad_{x,u} lam' F)/d[d; px] directly.
+    * stage cost, range rows and terminal maps: as ``_sens_functions`` with respect to p_k (terminal: d).
+    MPCB_SENS_P = 0 (the p entry points refuse) when `_sens_p_refusal` names a reason."""
+    nx, nu, nd, npx = prob.nx, prob.nu, prob.nd, prob.npx
+    par, off = o.par, o.off
+    exprs = [stage_cost, o.term_cost] + ([o.term_eq] if o.term_eq is not None else []) + ([rows[0]] if rows else [])
+    why = _sens_p_refusal(prob, o, exprs)
+    D["MPCB_SENS_P"] = int(why is None)
+    if why is not None:
+        return []
+    dpar = par[off["d"]:off["d"] + nd]
+    pk = vertcat(dpar, o.pxk, o.pyk)
+    gc = gradient(stage_cost, zz)
+    fns = [CFunction("ocp_cost_dp", ins_c, [("Lp", jacobian(gc, pk))]),
+           CFunction("ocp_term_dp", [("XN", o.XN), ("par", par)], [("Tp", jacobian(gradient(o.term_cost, o.XN), dpar))])]
+    if o.term_eq is not None:
+        fns.append(CFunction("ocp_termc_dp", [("XN", o.XN), ("par", par)], [("Rp", jacobian(o.term_eq, dpar))]))
+    if rows is not None:
+        R, mult = rows
+        fns.append(CFunction("ocp_out_dp", ins_c + [("mult", mult)],
+                             [("Yp", jacobian(R, pk)), ("HYp", jacobian(gradient(mtimes(mult.T, R), zz), pk))]))
+    x, u, d, t, px = [SX.sym(n, k) for n, k in (("x", nx), ("u", nu), ("d", nd), ("t", 1), ("px", npx))]
+    dpx = vertcat(d, px)
+    base = [("x", x), ("u", u), ("d", d), ("t", t), ("px", px)]
+    if prob.Fx_model.meta.get("kind") == "rk4":
+        rhs = prob.Fx_model.meta["rhs"]
+        f = SX(rhs(x, u, d, t, px))
+        qidx = [i for i, e in enumerate(dpx.elements()) if _depends_on(f, SX([e]))]
+        D["MPCB_SENS_NQ"] = len(qidx)
+        D["MPCB_SENS_QIDX"] = "{%s}" % ", ".join(str(i) for i in (qidx or [0]))
+        post = SX(prob.Fx_model.meta["post"](d, px))
+        Jpost = jacobian(post, dpx)
+        if _depends_on(Jpost, dpx):
+            raise NotImplementedError("the map applied after the RK4 integration must be affine in (d, px)")
+        fns.append(CFunction("mdl_post_dp", [("d", d), ("px", px)], [("Jp", Jpost)]))
+        if qidx:
+            nq = len(qidx)
+
+            def rhs_aug(xt, u_, d_, t_, px_):
+                sub = list(vertcat(d_, px_).elements())
+                for j, i in enumerate(qidx):
+                    sub[i] = xt[nx + j]._as_scalar_expr()
+                dd, pp = SX(sub[:nd]) if nd else d_, SX(sub[nd:]) if npx else px_
+                return vertcat(SX(rhs(xt[0:nx], u_, dd, t_, pp)), SX.zeros(nq, 1))
+
+            aug = _rhs_functions("mdlp_", rhs_aug, nx + nq, nu, nd, npx, nx + nq)
+            fns += [g for g in aug if g.name not in ("mdlp_f_s", "mdlp_f_s_xi")]
+            D["MPCB_MDLP_NC"], D["MPCB_MDLP_NR"] = _rhs_functions.last_cache
+    else:
+        k = SX.sym("k", 1)
+        F = SX(prob.Fx_model(x, u, k, d, t, px))
+        lam = SX.sym("lam", nx)
+        fns.append(CFunction("mdl_F_dp", base + [("lam", lam)],
+                             [("Fp", jacobian(F, dpx)), ("Hp", jacobian(gradient(mtimes(lam.T, F), vertcat(x, u)), dpx))]))
+    return fns
+
+
 def generate_header(prob, ss_spec, ocp_spec, opts: Optional[Dict] = None) -> Dict[str, object]:
     """Return ``{"text": header_source, "defines": {...}, "flops": {...}}`` for one problem."""
     nx, nu, ny, nd, npx, npy, N = prob.nx, prob.nu, prob.ny, prob.nd, prob.npx, prob.npy, prob.N
@@ -298,6 +376,7 @@ def generate_header(prob, ss_spec, ocp_spec, opts: Optional[Dict] = None) -> Dic
                                  [("Y", R), ("JY", jacobian(R, zz)), ("HY", tril_pack(Hy))]))
             D["MPCB_OUT_LINEAR"] = int(all(e is S.ZERO for e in Hy.elements()))
         fns += _sens_functions(o, D, ins_c, zz, stage_cost, rows=(R, mult) if n_rows else None)
+        fns += _sens_p_functions(prob, o, D, ins_c, zz, stage_cost, rows=(R, mult) if n_rows else None)
     else:
         D["MPCB_HAS_OCP"] = 0
 

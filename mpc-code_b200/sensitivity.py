@@ -5,8 +5,13 @@ the previous input: ``par[0 : 2nx+nu]`` and ``par[2nx+nu+nd : 2nx+2nu+nd]`` (``n
 derivative is the implicit-function derivative of the barrier KKT system at the returned iterate (as sIPOPT computes
 it, see ``include/mpcb.h``): strongly active bounds give derivatives of the order of the final barrier parameter.
 
-* `OcpSensitivity` (from ``BatchedNlpSolver.sensitivity()``): JVP, VJP and the feedback gain dU_0/dx_hat.
-* `OcpLayer`: the solve as a differentiable function of theta for ``torch.autograd``.
+The parameters that enter the dynamics, p = [d | px_0 .. px_{N-1} | py_0 .. py_{N-1}] = ``par[off_d : off_d+nd]`` ++
+``par[off_px :]`` (``n_p = nd + (npx+npy) N``), have their own sensitivities (``sensitivity(params=True)``): the
+disturbance estimate d_hat and the per-stage model offsets, whose derivatives are the controller's feed-forward gains.
+
+* `OcpSensitivity` (from ``BatchedNlpSolver.sensitivity()``): JVP, VJP, the feedback gain dU_0/dx_hat and, with
+  ``params=True``, the JVP / VJP in p and the disturbance gain dU_0/dd_hat.
+* `OcpLayer`: the solve as a differentiable function of theta (and of p with ``params=True``) for ``torch.autograd``.
 """
 from __future__ import annotations
 
@@ -33,13 +38,31 @@ def with_theta(par, theta, nx: int, nu: int, nd: int):
     return _torch().cat([theta[:, :a.stop], par[:, a.stop:b.start], theta[:, a.stop:], par[:, b.stop:]], dim=1)
 
 
+def param_slices(nx: int, nu: int, nd: int, ny: int):
+    """The two slices of ``par`` that make up p = [d | px | py]: d, and everything from the offsets of px on."""
+    off_d = 2 * nx + nu
+    return slice(off_d, off_d + nd), slice(2 * nx + 2 * nu + nd + 1 + ny * nu, None)
+
+
+def params_of(par, nx: int, nu: int, nd: int, ny: int):
+    """p [B, n_p] of OCP parameter vectors ``par`` [B, npar]."""
+    a, b = param_slices(nx, nu, nd, ny)
+    return _torch().cat([par[:, a], par[:, b]], dim=1)
+
+
+def with_params(par, p, nx: int, nu: int, nd: int, ny: int):
+    """``par`` with its p part replaced by ``p`` (differentiable in both)."""
+    a, b = param_slices(nx, nu, nd, ny)
+    return _torch().cat([par[:, :a.start], p[:, :nd], par[:, a.stop:b.start], p[:, nd:]], dim=1)
+
+
 class OcpSensitivity:
     """Captured sensitivities of one batched OCP solve.  ``status`` [B] (int32, device): 0 computed, 1 the solve ended
     with a status other than 0 / 1, 2 wrong inertia of the KKT matrix; every output of an instance with status != 0 is
     NaN.  The capture ``fac`` belongs to this object, so results do not change when the handle solves again."""
 
-    def __init__(self, handle, fac, status, uses_uprev: bool):
-        self.handle, self.fac, self.status, self.uses_uprev = handle, fac, status, uses_uprev
+    def __init__(self, handle, fac, status, uses_uprev: bool, params: bool = False):
+        self.handle, self.fac, self.status, self.uses_uprev, self.params = handle, fac, status, uses_uprev, params
         d = handle.lib.dims
         self.nx, self.nu, self.nd, self.ntheta = d.nx, d.nu, d.nd, handle.ntheta
 
@@ -64,25 +87,62 @@ class OcpSensitivity:
         du0 = dw[:, :, nx:nx + nu].transpose(1, 2).contiguous()          # [B, nu, ndir]
         return (du0[:, :, :nx].contiguous(), du0[:, :, nx:].contiguous()) if self.uses_uprev else du0
 
+    def _require_params(self):
+        if not self.params:
+            raise RuntimeError("captured without the p-blocks: use solver.sensitivity(params=True)")
+
+    def jvp_p(self, dp):
+        """dw [B, ndir, nw] for dp [B, ndir, n_p], p = [d | px | py]; a [B, n_p] input gives [B, nw]."""
+        self._require_params()
+        dw = self.handle.ocp_jvp_p(self.fac, dp)
+        return dw[:, 0] if getattr(dp, "ndim", 3) == 2 else dw
+
+    def vjp_p(self, gw):
+        """gp [B, n_p] = (dw/dp)' gw for gw [B, nw]."""
+        self._require_params()
+        return self.handle.ocp_vjp_p(self.fac, gw)
+
+    def disturbance_gain(self):
+        """dU_0/dd_hat [B, nu, nd] with the targets x_s, u_s held fixed: the OCP's response to the disturbance estimate.
+        In the closed loop d_hat also moves x_s and u_s through the target problem; that part of the total derivative is
+        not included (the target problem's sensitivities are not available)."""
+        self._require_params()
+        torch = _torch()
+        nx, nu, nd, B = self.nx, self.nu, self.nd, self.handle.batch
+        E = torch.zeros(nd, self.handle.np_params, dtype=torch.float64, device=self.handle.device)
+        E[torch.arange(nd), torch.arange(nd)] = 1.0
+        dw = self.handle.ocp_jvp_p(self.fac, E.expand(B, -1, -1))
+        return dw[:, :, nx:nx + nu].transpose(1, 2).contiguous()
+
 
 class OcpLayer:
     """``w = OcpLayer(solver)(theta, par, w0)``: the batched OCP solve as a function of theta, differentiable through
     ``torch.autograd`` (backward = one VJP sweep on the captured factorisation).  theta is the only differentiable
     input: ``par`` supplies the other parameters (its theta part is replaced) and ``w0`` is the initial guess; neither
-    may require grad.  Once differentiable (the backward pass is not itself differentiable)."""
+    may require grad.  Once differentiable (the backward pass is not itself differentiable).
 
-    def __init__(self, solver, lbx=None, ubx=None, lbg=None, ubg=None):
+    ``OcpLayer(solver, params=True)(theta, par, w0, p)``: p = [d | px | py] [B, n_p] is a second differentiable input
+    (it replaces the p part of ``par``); the backward pass is still one sweep per input."""
+
+    def __init__(self, solver, lbx=None, ubx=None, lbg=None, ubg=None, params: bool = False):
         if solver.kind != "ocp":
             raise NotImplementedError("OcpLayer wraps the dynamic OCP solver")
-        self.solver, self.bounds = solver, dict(lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg)
+        self.solver, self.bounds, self.params = solver, dict(lbx=lbx, ubx=ubx, lbg=lbg, ubg=ubg), params
         self.last = None                # OcpSensitivity of the last forward pass
 
-    def __call__(self, theta, par, w0):
+    def __call__(self, theta, par, w0, p=None):
         for name, t in (("par", par), ("w0", w0)):
             if getattr(t, "requires_grad", False):
-                raise ValueError("OcpLayer differentiates with respect to theta only: %s must not require grad "
-                                 "(sensitivities with respect to d, t, lambda, px, py are not available)" % name)
-        return _ocp_function().apply(theta, par, w0, self)
+                raise ValueError("OcpLayer differentiates with respect to theta%s only: %s must not require grad "
+                                 "(sensitivities with respect to t and lambda are not available)"
+                                 % (" and p" if self.params else " (and p with params=True)", name))
+        if p is not None and not self.params:
+            raise ValueError("p is a differentiable input only with OcpLayer(..., params=True)")
+        if self.params and p is None:
+            raise ValueError("OcpLayer(..., params=True) takes p [B, n_p] as its fourth input")
+        if not self.params:
+            return _ocp_function().apply(theta, par, w0, self)
+        return _ocp_function_p().apply(theta, p, par, w0, self)
 
 
 def _make_function():
@@ -111,7 +171,38 @@ def _make_function():
     return OcpFunction
 
 
+def _make_function_p():
+    torch = _torch()
+    from torch.autograd.function import once_differentiable
+
+    class OcpFunctionP(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, theta, p, par, w0, layer):
+            h = layer.solver.handle
+            d = h.lib.dims
+            pt = with_theta(h.tensor(par, d.npar), theta.detach().to(h.device, torch.float64), d.nx, d.nu, d.nd)
+            pt = with_params(pt, p.detach().to(h.device, torch.float64), d.nx, d.nu, d.nd, d.ny)
+            sol = layer.solver(x0=w0, p=pt, **layer.bounds)
+            sens = layer.solver.sensitivity(params=True)
+            layer.last = sens
+            ctx.sens = sens
+            ctx.meta = (theta.dtype, theta.device, p.dtype, p.device)
+            return sol["x"]
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, gw):
+            gw = gw.contiguous()
+            tdt, tdev, pdt, pdev = ctx.meta
+            gth = ctx.sens.vjp(gw).to(device=tdev, dtype=tdt) if ctx.needs_input_grad[0] else None
+            gp = ctx.sens.vjp_p(gw).to(device=pdev, dtype=pdt) if ctx.needs_input_grad[1] else None
+            return gth, gp, None, None, None
+
+    return OcpFunctionP
+
+
 _FUNCTION = None
+_FUNCTION_P = None
 
 
 def _ocp_function():
@@ -120,3 +211,10 @@ def _ocp_function():
     if _FUNCTION is None:
         _FUNCTION = _make_function()
     return _FUNCTION
+
+
+def _ocp_function_p():
+    global _FUNCTION_P
+    if _FUNCTION_P is None:
+        _FUNCTION_P = _make_function_p()
+    return _FUNCTION_P

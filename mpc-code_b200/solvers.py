@@ -36,7 +36,8 @@ C_SYMBOLS = ("mpcb_abi_version", "mpcb_default_opts", "mpcb_get_dims", "mpcb_mod
              "mpcb_plant_meas", "mpcb_plant_step", "mpcb_model_output", "mpcb_model_step", "mpcb_stage_derivs",
              "mpcb_last_launches", "mpcb_last_ticks", "mpcb_total_launches", "mpcb_set_groups", "mpcb_set_policy", "mpcb_set_profiling", "mpcb_get_profile", "mpcb_dfma_peak",
              "mpcb_loop_reset", "mpcb_step", "mpcb_loop_get",
-             "mpcb_ocp_sens_size", "mpcb_ocp_sens_factor", "mpcb_ocp_jvp", "mpcb_ocp_vjp")
+             "mpcb_ocp_sens_size", "mpcb_ocp_sens_factor", "mpcb_ocp_jvp", "mpcb_ocp_vjp",
+             "mpcb_ocp_sens_size_p", "mpcb_ocp_sens_factor_p", "mpcb_ocp_jvp_p", "mpcb_ocp_vjp_p")
 
 
 class MpcbLibrary:
@@ -80,6 +81,10 @@ class MpcbLibrary:
         L.mpcb_ocp_sens_factor.argtypes = [vp] * 5
         L.mpcb_ocp_jvp.argtypes = [vp, vp, ci, vp, vp, vp]
         L.mpcb_ocp_vjp.argtypes = [vp] * 5
+        L.mpcb_ocp_sens_size_p.restype = ctypes.c_long
+        L.mpcb_ocp_sens_factor_p.argtypes = [vp] * 5
+        L.mpcb_ocp_jvp_p.argtypes = [vp, vp, ci, vp, vp, vp]
+        L.mpcb_ocp_vjp_p.argtypes = [vp] * 5
         self.dims = MpcbDims()
         L.mpcb_get_dims(ctypes.byref(self.dims))
 
@@ -205,6 +210,48 @@ class MpcbHandle:
         gw = self.tensor(gw, self.lib.dims.nw)
         g = self.empty(self.batch, self.ntheta)
         self._check(self.L.mpcb_ocp_vjp(self._h, fac.data_ptr(), gw.data_ptr(), g.data_ptr(), self._stream()))
+        return g
+
+    # -- sensitivities with respect to p = [d | px | py] (include/mpcb.h, mpcb_ocp_sens_factor_p) --------------------
+    @property
+    def np_params(self) -> int:
+        d = self.lib.dims
+        return d.nd + (d.npx + d.npy) * d.N
+
+    def ocp_sens_factor_p(self, par):
+        """As `ocp_sens_factor`, with the derivative blocks of p: ``(fac [B, size_p], status [B])``.  ``fac`` is one
+        buffer of B * size_p doubles: the B theta captures (which the theta methods accept) followed by the p-blocks."""
+        torch = _torch()
+        par = self.tensor(par, self.lib.dims.npar)
+        fac = self.empty(self.batch, int(self.L.mpcb_ocp_sens_size_p()))
+        st = self.empty(self.batch, dtype=torch.int32)
+        self._check(self.L.mpcb_ocp_sens_factor_p(self._h, par.data_ptr(), fac.data_ptr(), st.data_ptr(), self._stream()))
+        return fac, st
+
+    def _p_capture(self, fac):
+        if fac.numel() != self.batch * int(self.L.mpcb_ocp_sens_size_p()):
+            raise ValueError("the p sweeps need a capture of ocp_sens_factor_p")
+
+    def ocp_jvp_p(self, fac, dp):
+        """dw [B, ndir, nw] = J_p dp for dp [B, ndir, n_p] (or [B, n_p]: one direction)."""
+        self._p_capture(fac)
+        d = self.lib.dims
+        dt = self.tensor(dp)
+        if dt.ndim == 2:
+            dt = dt.unsqueeze(1)
+        if dt.ndim != 3 or dt.shape[0] != self.batch or dt.shape[2] != self.np_params:
+            raise ValueError("dp must be [B, ndir, %d], got %s" % (self.np_params, tuple(dt.shape)))
+        dt = dt.contiguous()
+        dw = self.empty(self.batch, dt.shape[1], d.nw)
+        self._check(self.L.mpcb_ocp_jvp_p(self._h, fac.data_ptr(), int(dt.shape[1]), dt.data_ptr(), dw.data_ptr(), self._stream()))
+        return dw
+
+    def ocp_vjp_p(self, fac, gw):
+        """gp [B, n_p] = J_p' gw for gw [B, nw]."""
+        self._p_capture(fac)
+        gw = self.tensor(gw, self.lib.dims.nw)
+        g = self.empty(self.batch, self.np_params)
+        self._check(self.L.mpcb_ocp_vjp_p(self._h, fac.data_ptr(), gw.data_ptr(), g.data_ptr(), self._stream()))
         return g
 
     def target(self, par_ss, wss):
@@ -418,9 +465,10 @@ class BatchedNlpSolver:
         self._last = (st, it)
         return {"x": x, "f": f}
 
-    def sensitivity(self):
+    def sensitivity(self, params: bool = False):
         """Sensitivities of the last solve with respect to theta = [x_hat | x_s | u_s | u_{k-1}] (see
         `mpc_code_b200.sensitivity`): an `OcpSensitivity` that owns its capture and stays valid after later solves.
+        ``params=True`` also captures the sensitivities with respect to p = [d | px | py] (`OcpSensitivity.jvp_p`).
         Must be called before the handle solves another OCP, with the solve's ``p`` not modified in place since."""
         if self.kind != "ocp":
             raise NotImplementedError("sensitivities are available for the dynamic OCP only, not the target problem")
@@ -431,8 +479,8 @@ class BatchedNlpSolver:
         if solves != self.handle.ocp_solves:
             raise RuntimeError("the handle has solved another OCP since this solver's last call: its workspace is gone")
         from .sensitivity import OcpSensitivity
-        fac, st = self.handle.ocp_sens_factor(par)
-        return OcpSensitivity(self.handle, fac, st, uses_uprev=bool(self.spec.uses_uprev))
+        fac, st = (self.handle.ocp_sens_factor_p if params else self.handle.ocp_sens_factor)(par)
+        return OcpSensitivity(self.handle, fac, st, uses_uprev=bool(self.spec.uses_uprev), params=params)
 
     def stats(self):
         if self._last is None:

@@ -1,7 +1,8 @@
 """Cost of the OCP sensitivities on the GPU, against the solve they belong to (Ex_NMPC, B = 4096 by default).
 
 CUDA events around, after warm-up: the batched mpcb_ocp solve, mpcb_ocp_sens_factor, the full theta-Jacobian (one JVP
-of all ntheta unit directions) and one VJP; the median of --reps repetitions each.  Prints the card name and power
+of all ntheta unit directions) and one VJP; for p = [d | px | py] mpcb_ocp_sens_factor_p, the d-Jacobian (nd unit
+directions), the full p-Jacobian (all n_p unit directions) and one VJP_p; the median of --reps repetitions each.  Prints the card name and power
 limit read in the same run.  Usage: python tools/sens_timing.py [--batch 4096] [--reps 20]
 """
 import argparse
@@ -58,11 +59,26 @@ def main():
     fac, st = h.ocp_sens_factor(par_t)
     t_jac = timed(lambda: h.ocp_jvp(fac, eye))
     t_vjp = timed(lambda: h.ocp_vjp(fac, gw))
+    npp = h.np_params
+    eye_p = torch.eye(npp, dtype=torch.float64, device=h.device).expand(B, -1, -1).contiguous()
+    eye_d = eye_p[:, :prob.nd].contiguous()
+    t_factor_p = timed(lambda: h.ocp_sens_factor_p(par_t))
+    fac_p, st_p = h.ocp_sens_factor_p(par_t)
+    h.ocp_jvp_p(fac_p, eye_p); h.ocp_vjp_p(fac_p, gw); torch.cuda.synchronize()
+    t_jac_d = timed(lambda: h.ocp_jvp_p(fac_p, eye_d))
+    t_jac_p = timed(lambda: h.ocp_jvp_p(fac_p, eye_p))
+    t_vjp_p = timed(lambda: h.ocp_vjp_p(fac_p, gw))
     res = dict(card=card, problem="nmpc_cstr (Ex_NMPC)", batch=B, ntheta=nth, reps=a.reps,
                sens_status_counts={int(k): int(v) for k, v in zip(*np.unique(st.cpu().numpy(), return_counts=True))},
                solve_ms=t_solve, factor_ms=t_factor, jacobian_ms=t_jac, vjp_ms=t_vjp,
                factor_plus_jacobian_over_solve=(t_factor + t_jac) / t_solve, vjp_over_solve=t_vjp / t_solve,
-               factor_plus_vjp_over_solve=(t_factor + t_vjp) / t_solve)
+               factor_plus_vjp_over_solve=(t_factor + t_vjp) / t_solve,
+               n_p=npp, capture_p_doubles_per_instance=int(h.L.mpcb_ocp_sens_size_p()),
+               sens_p_status_counts={int(k): int(v) for k, v in zip(*np.unique(st_p.cpu().numpy(), return_counts=True))},
+               factor_p_ms=t_factor_p, d_jacobian_ms=t_jac_d, p_jacobian_ms=t_jac_p, vjp_p_ms=t_vjp_p,
+               factor_p_plus_d_jacobian_over_solve=(t_factor_p + t_jac_d) / t_solve,
+               factor_p_plus_p_jacobian_over_solve=(t_factor_p + t_jac_p) / t_solve,
+               factor_p_plus_vjp_p_over_solve=(t_factor_p + t_vjp_p) / t_solve)
     print(json.dumps(res, indent=1))
 
 
