@@ -102,7 +102,6 @@ __global__ void __launch_bounds__(128) k_ocp_eval_first(OcpArgs a) {
 #define KKT_SCRATCH_BYTES ((int)sizeof(double) * KktScratch::total * (32 / MPCB_KKT_LANES))
 #define KKT_WARPS (4 * KKT_SCRATCH_BYTES <= 48 * 1024 ? 4 : (2 * KKT_SCRATCH_BYTES <= 48 * 1024 ? 2 : 1))
 #endif
-#if MPCB_KKT_LANES > 1
 // -DMPCB_FUSE_LS=1 (opt-in, one warp per instance only): the warp that computed the step also runs the instance's filter
 // line search - trial points over its lanes (stage k on lane k mod 32), decision, backtracking - so a tick is two
 // kernels (k_ocp_eval, k_ocp_kkt).  Same device functions and arithmetic as the four-kernel tick, GPU suite green, but
@@ -111,6 +110,16 @@ __global__ void __launch_bounds__(128) k_ocp_eval_first(OcpArgs a) {
 #ifndef MPCB_FUSE_LS
 #define MPCB_FUSE_LS 0
 #endif
+#if MPCB_FUSE_LS && MPCB_KKT_LANES != 32
+// the fused trial loop strides over the 32 lanes of a warp and ocp_accept reduces over the whole warp: with lane groups
+// it would mix instances, with one thread per instance there is no warp to run it
+#  error "MPCB_FUSE_LS=1 requires MPCB_KKT_LANES=32 (the fused line search runs on one whole warp per instance)"
+#endif
+#if MPCB_KKT_LANES > 1
+// the 32 * KKT_WARPS / MPCB_KKT_LANES instances of a block keep their KKT scratch in static shared memory
+static_assert(sizeof(double) * KktScratch::total * (32 * KKT_WARPS / MPCB_KKT_LANES) <= 48 * 1024,
+              "MPCB_KKT_LANES: the KKT scratch of the lane groups of one warp exceeds the 48 kB of static shared memory; "
+              "this problem needs more lanes per instance or the one-thread mapping -DMPCB_KKT_LANES=1");
 #ifdef MPCB_KKT_MINBLOCKS
 #define KKT_BOUNDS __launch_bounds__(32 * KKT_WARPS, MPCB_KKT_MINBLOCKS)
 #else
@@ -140,7 +149,6 @@ __global__ void KKT_BOUNDS k_ocp_kkt(OcpArgs a, int* n_active) {
 }
 #define KKT_GRID(B) nblk((long)(B) * MPCB_KKT_LANES, 32 * KKT_WARPS), 32 * KKT_WARPS
 #else
-#define MPCB_FUSE_LS 0
 __global__ void __launch_bounds__(32) k_ocp_kkt(OcpArgs a, int* n_active) {
     (void)n_active;
     const int inst = blockIdx.x * blockDim.x + threadIdx.x;

@@ -554,8 +554,15 @@ MPCB_UNROLL
 #ifndef MPCB_KKT_LANES
 #  define MPCB_KKT_LANES 32
 #endif
-// MPCB_KKT_LANES may be any power of two <= 32: with L < 32 a warp carries 32/L instances ("lane groups"); the stage
-// blocks of small systems (Ex_NMPC: 3 x 5) leave most of 32 lanes idle, and the kernel is bound by issue slots.
+// MPCB_KKT_LANES is one of 1, 2, 4, 8, 16, 32: with L < 32 a warp carries 32/L instances ("lane groups"); the stage
+// blocks of small systems (Ex_NMPC: 3 x 5) leave most of 32 lanes idle, and the kernel is bound by issue slots.  The
+// 32/L scratches of a warp share the 48 kB of static shared memory, so lane groups only build for problems whose
+// KktScratch is small enough (mpcb_api.cu refuses the others: syn_12_4_20 at 4 lanes, syn_20_6_20 at 16 lanes or fewer
+// - the latter builds with 32 lanes or with one thread per instance, whose scratch is thread-local).
+#if MPCB_KKT_LANES != 1 && MPCB_KKT_LANES != 2 && MPCB_KKT_LANES != 4 && MPCB_KKT_LANES != 8 && \
+    MPCB_KKT_LANES != 16 && MPCB_KKT_LANES != 32
+#  error "MPCB_KKT_LANES must be one of 1, 2, 4, 8, 16, 32 (the lane-group masks and reductions assume a power of two <= 32)"
+#endif
 #if defined(__CUDA_ARCH__) && (MPCB_KKT_LANES > 1)
 #  define LANE_ID    ((int)(threadIdx.x & (MPCB_KKT_LANES - 1)))
 #  define N_LANES    MPCB_KKT_LANES
