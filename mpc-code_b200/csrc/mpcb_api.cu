@@ -92,74 +92,43 @@ __global__ void __launch_bounds__(128) k_ocp_eval_first(OcpArgs a) {
 }
 #endif
 
-// KKT step: one thread per instance (small stage blocks, MPCB_KKT_LANES == 1) or one warp per instance with
-// per-warp scratch in shared memory (MPCB_KKT_LANES == 32)
 #ifndef MPCB_TGT_BLOCK
 #define MPCB_TGT_BLOCK 64       // threads per block of the one-thread-per-instance target solve
 #endif
 #ifndef KKT_WARPS
-// warps (instances) per block of the KKT kernel: as many as fit the 48 kB of static shared memory, at most 4
+// warps per block of the KKT kernel: as many as fit the 48 kB of static shared memory, at most 4
 #define KKT_SCRATCH_BYTES ((int)sizeof(double) * KktScratch::total * (32 / MPCB_KKT_LANES))
 #define KKT_WARPS (4 * KKT_SCRATCH_BYTES <= 48 * 1024 ? 4 : (2 * KKT_SCRATCH_BYTES <= 48 * 1024 ? 2 : 1))
 #endif
-// -DMPCB_FUSE_LS=1 (opt-in, one warp per instance only): the warp that computed the step also runs the instance's filter
-// line search - trial points over its lanes (stage k on lane k mod 32), decision, backtracking - so a tick is two
-// kernels (k_ocp_eval, k_ocp_kkt).  Same device functions and arithmetic as the four-kernel tick, GPU suite green, but
-// SLOWER on Ex_NMPC (612 k vs 687 k steps/s, profiles/r02_variants_fuse.txt): the RK4 roll-outs of the trial run at the
-// KKT kernel's 7 warps per scheduler and pay their full latency, the separate k_ocp_trial hides it with 4x the warps.
-#ifndef MPCB_FUSE_LS
-#define MPCB_FUSE_LS 0
-#endif
-#if MPCB_FUSE_LS && MPCB_KKT_LANES != 32
-// the fused trial loop strides over the 32 lanes of a warp and ocp_accept reduces over the whole warp: with lane groups
-// it would mix instances, with one thread per instance there is no warp to run it
-#  error "MPCB_FUSE_LS=1 requires MPCB_KKT_LANES=32 (the fused line search runs on one whole warp per instance)"
-#endif
+// Per-instance kernels of the KKT mapping (k_ocp_kkt, k_ocp_sens_factor): KktLanes::n lanes per instance.  Lane groups
+// run KKT_WARPS warps per block and keep their KktScratch in static shared memory, one row per group; one thread per
+// instance runs blocks of 32 threads and keeps it thread-local.  KKT_SCRATCH(sm) declares `double* sm`.
 #if MPCB_KKT_LANES > 1
-// the 32 * KKT_WARPS / MPCB_KKT_LANES instances of a block keep their KKT scratch in static shared memory
-static_assert(sizeof(double) * KktScratch::total * (32 * KKT_WARPS / MPCB_KKT_LANES) <= 48 * 1024,
+#define KKT_THREADS (32 * KKT_WARPS)
+static_assert(sizeof(double) * KktScratch::total * (KKT_THREADS / MPCB_KKT_LANES) <= 48 * 1024,
               "MPCB_KKT_LANES: the KKT scratch of the lane groups of one warp exceeds the 48 kB of static shared memory; "
               "this problem needs more lanes per instance or the one-thread mapping -DMPCB_KKT_LANES=1");
+#define KKT_SCRATCH(sm) __shared__ __align__(16) double sm##_rows[KKT_THREADS / KktLanes::n][KktScratch::total]; \
+                        double* sm = sm##_rows[threadIdx.x / KktLanes::n]
+#else
+#define KKT_THREADS 32
+#define KKT_SCRATCH(sm) double sm[KktScratch::total]
+#endif
 #ifdef MPCB_KKT_MINBLOCKS
-#define KKT_BOUNDS __launch_bounds__(32 * KKT_WARPS, MPCB_KKT_MINBLOCKS)
+#define KKT_BOUNDS __launch_bounds__(KKT_THREADS, MPCB_KKT_MINBLOCKS)
 #else
-#define KKT_BOUNDS __launch_bounds__(32 * KKT_WARPS)
+#define KKT_BOUNDS __launch_bounds__(KKT_THREADS)
 #endif
-__global__ void KKT_BOUNDS k_ocp_kkt(OcpArgs a, int* n_active) {
-    constexpr int GROUPS = 32 * KKT_WARPS / MPCB_KKT_LANES;        // instances per block
-    __shared__ __align__(16) double scratch[GROUPS][KktScratch::total];
-    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) / MPCB_KKT_LANES;
+#define KKT_GRID(B) nblk((long)(B) * MPCB_KKT_LANES, KKT_THREADS), KKT_THREADS
+
+__global__ void KKT_BOUNDS k_ocp_kkt(OcpArgs a) {
+    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) / KktLanes::n;
     if (inst >= a.B) return;
     if (a.st[inst].state != ST_EVAL) return;
+    KKT_SCRATCH(sm);
     OcpInst I = ocp_view(a, inst);
-    ocp_kkt(I, a.S, scratch[threadIdx.x / MPCB_KKT_LANES]);
-#if MPCB_FUSE_LS
-    const int lane = threadIdx.x & 31;
-    volatile int* state = &a.st[inst].state;
-    while (*state == ST_LS) {
-        if (lane == 0) atomicAdd(a.counters + 1, 1ULL);
-        for (int k = lane; k < NH; k += 32) ocp_trial_stage(I, a.S, k);
-        __syncwarp();
-        ocp_accept(I, a.S);
-    }
-    if (n_active && lane == 0 && *state != ST_DONE) atomicAdd(n_active, 1);
-#else
-    (void)n_active;
-#endif
+    ocp_kkt(I, a.S, sm);
 }
-#define KKT_GRID(B) nblk((long)(B) * MPCB_KKT_LANES, 32 * KKT_WARPS), 32 * KKT_WARPS
-#else
-__global__ void __launch_bounds__(32) k_ocp_kkt(OcpArgs a, int* n_active) {
-    (void)n_active;
-    const int inst = blockIdx.x * blockDim.x + threadIdx.x;
-    if (inst >= a.B) return;
-    if (a.st[inst].state != ST_EVAL) return;
-    double scratch[KktScratch::total];
-    OcpInst I = ocp_view(a, inst);
-    ocp_kkt(I, a.S, scratch);
-}
-#define KKT_GRID(B) nblk((long)(B), 32), 32
-#endif
 
 __global__ void __launch_bounds__(128) k_ocp_trial(OcpArgs a) {
     const int tid = blockIdx.x * blockDim.x + threadIdx.x;
@@ -173,13 +142,13 @@ __global__ void __launch_bounds__(128) k_ocp_trial(OcpArgs a) {
 
 // n_active != null: count the instances that are not done after this tick
 __global__ void __launch_bounds__(32 * KKT_WARPS) k_ocp_accept(OcpArgs a, int* n_active) {
-    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) / WarpLanes::n;
     if (inst >= a.B) return;
     if (a.st[inst].state == ST_LS) {
         OcpInst I = ocp_view(a, inst);
         ocp_accept(I, a.S);
     }
-    if (n_active && (threadIdx.x & 31) == 0 && a.st[inst].state != ST_DONE) atomicAdd(n_active, 1);
+    if (n_active && threadIdx.x % WarpLanes::n == 0 && a.st[inst].state != ST_DONE) atomicAdd(n_active, 1);
 }
 
 // Loop condition of the device-driven solve (body of the CUDA-graph WHILE node, after k_ocp_accept): another tick while
@@ -230,24 +199,14 @@ __device__ __forceinline__ void sens_factor_inst(const double* ws, const double*
                                                  int inst, double* sm) {
     OcpInst I = ocp_inst(const_cast<double*>(ws) + (size_t)inst * OcpLayout::total, nullptr, par + (size_t)inst * NPAR, st + inst);
     const int r = ocp_sens_factor(I, fac + (size_t)inst * SensLayout::total, sm);
-    if ((threadIdx.x & (MPCB_KKT_LANES - 1)) == 0) status[inst] = r;
+    if (KktLanes::id() == 0) status[inst] = r;
 }
-#if MPCB_KKT_LANES > 1
 __global__ void KKT_BOUNDS k_ocp_sens_factor(int B, const double* ws, const double* par, InstState* st, double* fac, int* status) {
-    constexpr int GROUPS = 32 * KKT_WARPS / MPCB_KKT_LANES;
-    __shared__ __align__(16) double scratch[GROUPS][KktScratch::total];
-    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) / MPCB_KKT_LANES;
+    const int inst = (blockIdx.x * blockDim.x + threadIdx.x) / KktLanes::n;
     if (inst >= B) return;
-    sens_factor_inst(ws, par, st, fac, status, inst, scratch[threadIdx.x / MPCB_KKT_LANES]);
+    KKT_SCRATCH(sm);
+    sens_factor_inst(ws, par, st, fac, status, inst, sm);
 }
-#else
-__global__ void __launch_bounds__(32) k_ocp_sens_factor(int B, const double* ws, const double* par, InstState* st, double* fac, int* status) {
-    const int inst = blockIdx.x * blockDim.x + threadIdx.x;
-    if (inst >= B) return;
-    double scratch[KktScratch::total];
-    sens_factor_inst(ws, par, st, fac, status, inst, scratch);
-}
-#endif
 // JVP: one thread per (instance, direction); the directions of an instance sit on consecutive lanes, so their reads of
 // the instance's capture are broadcasts.  VJP: one thread per instance.
 __global__ void __launch_bounds__(128) k_ocp_jvp(int B, int ndir, const double* fac, const double* dth, double* dw) {
@@ -720,14 +679,14 @@ static bool same_opts(const mpcb_opts_t& a, const mpcb_opts_t& b) {
 #if MPCB_HAS_OCP
 // Build the device-driven solve as a CUDA graph:
 //   memset counters -> k_ocp_init -> U unrolled ticks -> k_ocp_cond -> WHILE { tick -> k_ocp_cond } -> k_ocp_output
-// with tick = k_ocp_eval -> k_ocp_kkt (line search inside; four kernels with -DMPCB_FUSE_LS=0).  The loop condition is set on the device by k_ocp_cond
+// with tick = k_ocp_eval -> k_ocp_kkt -> k_ocp_trial -> k_ocp_accept.  The loop condition is set on the device by k_ocp_cond
 // (cudaGraphSetConditional), so a whole solve - however many ticks its slowest instance needs - is ONE graph launch and the
 // host never waits on it (round 1 polled a device counter every two ticks, with one spinning host thread per group).
 // The first U ticks are plain kernel nodes: a node inside a WHILE body costs ~5 us of device-side scheduling that
 // serialises across streams (measured: profiles/r02_groups_sweep_graph.txt), a plain node ~1.5 us, and a tick whose
 // instances are all done is four kernels that exit at once.  U = MPCB_GRAPH_UNROLL (environment), default 10: a warm
 // closed-loop step of Ex_NMPC needs 11-13 ticks.
-#define TICK_KERNELS (MPCB_FUSE_LS ? 2 : 4)
+#define TICK_KERNELS 4                   // launches per tick
 static int add_tick(mpcb_ctx* h, cudaGraph_t g, cudaGraphNode_t* dep, int ndep, OcpArgs& a, int* n_active, cudaGraphNode_t* last,
                     bool first = false) {
     const int bs = 128;
@@ -747,21 +706,14 @@ static int add_tick(mpcb_ctx* h, cudaGraph_t g, cudaGraphNode_t* dep, int ndep, 
     kp.sharedMemBytes = 0;
     { dim3 gk(1), bk(1); auto set = [&](int gx, int bx) { gk = dim3(gx); bk = dim3(bx); }; set(KKT_GRID(h->B));
       kp.func = (void*)k_ocp_kkt; kp.gridDim = gk; kp.blockDim = bk; }
-    void* args2[] = {&a, &n_active};
-    kp.kernelParams = args2;
-#if MPCB_FUSE_LS
-    (void)bs;
-    CK(cudaGraphAddKernelNode(last, g, &n_eval, 1, &kp));
-#else
     cudaGraphNode_t n_kkt, n_trial;
     CK(cudaGraphAddKernelNode(&n_kkt, g, &n_eval, 1, &kp));
-    kp.kernelParams = args1;
     kp.func = (void*)k_ocp_trial; kp.gridDim = dim3(nblk(nst, bs)); kp.blockDim = dim3(bs);
     CK(cudaGraphAddKernelNode(&n_trial, g, &n_kkt, 1, &kp));
+    void* args2[] = {&a, &n_active};
     kp.func = (void*)k_ocp_accept; kp.gridDim = dim3(nblk((long)h->B * 32, 32 * KKT_WARPS)); kp.blockDim = dim3(32 * KKT_WARPS);
     kp.kernelParams = args2;
     CK(cudaGraphAddKernelNode(last, g, &n_trial, 1, &kp));
-#endif
     return 0;
 }
 
@@ -844,15 +796,10 @@ static int ocp_host_loop(mpcb_ctx* h, OcpArgs& a, double* f, int* status, int* i
             else
 #endif
             { Prof p(h, s, KC_OCP_EVAL); k_ocp_eval<<<nblk(nst, MPCB_EVAL_BLOCK), MPCB_EVAL_BLOCK, EVAL_SMEM_BYTES, s>>>(a); }
-#if MPCB_FUSE_LS
-            if (c == check_every - 1) CK(cudaMemsetAsync(h->n_active, 0, sizeof(int), s));
-            { Prof p(h, s, KC_OCP_KKT); k_ocp_kkt<<<KKT_GRID(h->B), 0, s>>>(a, h->n_active); }
-#else
-            { Prof p(h, s, KC_OCP_KKT); k_ocp_kkt<<<KKT_GRID(h->B), 0, s>>>(a, nullptr); }
+            { Prof p(h, s, KC_OCP_KKT); k_ocp_kkt<<<KKT_GRID(h->B), 0, s>>>(a); }
             { Prof p(h, s, KC_OCP_TRIAL); k_ocp_trial<<<nblk(nst, bs), bs, 0, s>>>(a); }
             if (c == check_every - 1) CK(cudaMemsetAsync(h->n_active, 0, sizeof(int), s));
             { Prof p(h, s, KC_OCP_ACCEPT); k_ocp_accept<<<nblk((long)h->B * 32, 32 * KKT_WARPS), 32 * KKT_WARPS, 0, s>>>(a, h->n_active); }
-#endif
             launches += TICK_KERNELS; ticks++;
         }
         CK(cudaMemcpyAsync(h->h_active, h->n_active, sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -1389,7 +1336,7 @@ int mpcb_last_ticks(mpcb_handle_t h) {
     return (int)worst;
 }
 
-// kernel launches made through this handle since its creation (host launches + 5 per device-driven tick)
+// kernel launches made through this handle since its creation (host launches + TICK_KERNELS per device-driven tick)
 long mpcb_total_launches(mpcb_handle_t h) {
     unsigned long long last = 0, total = 0;
     read_ticks(h, &last, &total);

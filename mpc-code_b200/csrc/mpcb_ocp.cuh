@@ -542,11 +542,11 @@ MPCB_UNROLL
 }
 
 // =============================================================================================
-// Lane-generic helpers.  ocp_kkt / ocp_accept are written once and run either by MPCB_KKT_LANES = 32 lanes
-// of a warp (lanes strided over matrix entries, reductions by shuffle, per-warp scratch in shared memory:
-// the mapping for large stage blocks), by one device thread per instance (MPCB_KKT_LANES = 1: everything in
-// registers, records streamed with 128-bit loads - the mapping for small systems such as Ex_NMPC), or by a
-// single host "lane" (tests).
+// Lane-generic helpers.  ocp_kkt / ocp_accept are written once over a lane group (Lanes<L>, mpcb_device.cuh) and run
+// either by MPCB_KKT_LANES = 32 lanes of a warp (lanes strided over matrix entries, reductions by shuffle, per-warp
+// scratch in shared memory: the mapping for large stage blocks), by one device thread per instance (MPCB_KKT_LANES = 1:
+// everything in registers, records read in place - the mapping for small systems such as Ex_NMPC), or by a single host
+// "lane" (tests).
 // =============================================================================================
 // Measured on B200 at 4 096 instances (profiles/r01_variants.txt): one warp per instance is faster than one thread per
 // instance (the latter has 5x fewer instructions but only 128 warps to hide latency with); the thread mapping is the
@@ -563,24 +563,8 @@ MPCB_UNROLL
     MPCB_KKT_LANES != 16 && MPCB_KKT_LANES != 32
 #  error "MPCB_KKT_LANES must be one of 1, 2, 4, 8, 16, 32 (the lane-group masks and reductions assume a power of two <= 32)"
 #endif
-#if defined(__CUDA_ARCH__) && (MPCB_KKT_LANES > 1)
-#  define LANE_ID    ((int)(threadIdx.x & (MPCB_KKT_LANES - 1)))
-#  define N_LANES    MPCB_KKT_LANES
-#  define GROUP_MASK (MPCB_KKT_LANES == 32 ? 0xffffffffu : (((1u << (MPCB_KKT_LANES & 31)) - 1u) << ((threadIdx.x & 31) & ~(MPCB_KKT_LANES - 1))))
-#  define W_SYNC()   __syncwarp(GROUP_MASK)
-#  define W_SUM(v)   group_sum<MPCB_KKT_LANES>(v, GROUP_MASK)
-#  define W_MAX(v)   group_max<MPCB_KKT_LANES>(v, GROUP_MASK)
-#  define W_MIN(v)   group_min<MPCB_KKT_LANES>(v, GROUP_MASK)
-#  define KKT_ON_LANES 1
-#else
-#  define LANE_ID   0
-#  define N_LANES   1
-#  define W_SYNC()
-#  define W_SUM(v)  (v)
-#  define W_MAX(v)  (v)
-#  define W_MIN(v)  (v)
-#  define KKT_ON_LANES 0
-#endif
+typedef Lanes<MPCB_KKT_LANES> KktLanes;       // ocp_riccati, ocp_kkt, ocp_sens_factor
+typedef Lanes<32> WarpLanes;                  // ocp_accept: one whole warp per instance
 #define KKT_STAGED (MPCB_KKT_LANES > 1)        // records staged through the scratch (lane mappings) or read in place
 
 // scratch (doubles): shared memory per warp with 32 lanes, thread-local (registers) with one lane
@@ -588,9 +572,6 @@ MPCB_UNROLL
 // UBLKCP) from the workspace straight into a ring of KKT_NBUF shared-memory buffers, completion signalled on one mbarrier
 // per buffer, issued KKT_NBUF - 1 stages ahead of the stage being processed.  Round 1 staged the next record through
 // registers (one stage ahead): a third of the kernel's stall samples sat on that copy (profiles/r02_v2_sass_k_ocp_kkt.txt).
-#ifndef MPCB_KKT_TMA
-#define MPCB_KKT_TMA 1
-#endif
 #define KKT_RBUF ((R_BWD + 1) / 2 * 2)          // doubles per ring buffer: a 16-byte multiple
 #define KKT_NBUF (KKT_RBUF > 600 ? 2 : 3)       // large stage blocks: two buffers (the scratch must fit 48 kB of static shared memory)
 struct KktScratch {
@@ -620,7 +601,7 @@ struct KktScratch {
     static constexpr int total = (nuS + NXT + 1) / 2 * 2;           // even: every instance's scratch stays 16-byte aligned
 };
 
-#if defined(__CUDA_ARCH__) && KKT_STAGED && MPCB_KKT_TMA
+#if defined(__CUDA_ARCH__) && KKT_STAGED
 #define KKT_USE_TMA 1
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(void* bar, int count) {
@@ -665,39 +646,6 @@ struct RecRing {
 #define KKT_USE_TMA 0
 #endif
 
-// Streaming of the per-stage records by the sequential sweeps.  With 32 lanes the record of the NEXT stage to be
-// visited is loaded into registers (REC_PER_LANE doubles per lane) while the current stage is being processed, and
-// only copied to shared memory when its turn comes: the DRAM/L2 latency of the load overlaps the arithmetic
-// (ncu before this: 54 % of the kernel's stall samples sat on the record copy).  With one lane the record is read in
-// place.
-#define REC_PER_LANE ((R_BWD + MPCB_KKT_LANES - 1) / MPCB_KKT_LANES)
-struct RecStream {
-    double pre[REC_PER_LANE];
-};
-MPCB_HD void rec_prefetch(RecStream& rs, const double* rk) {
-#if KKT_ON_LANES
-MPCB_UNROLL
-    for (int q = 0; q < REC_PER_LANE; ++q) { const int e = LANE_ID + N_LANES * q; rs.pre[q] = (e < R_BWD) ? rk[e] : 0.0; }
-#else
-    (void)rs; (void)rk;
-#endif
-}
-// publish the prefetched record (must be the one of `rk`) and start fetching `rk_next` (may be null)
-MPCB_HD const double* stage_record(RecStream& rs, const double* rk, const double* rk_next, double* sm) {
-#if KKT_ON_LANES
-    double* R = sm + KktScratch::R;
-    W_SYNC();
-MPCB_UNROLL
-    for (int q = 0; q < REC_PER_LANE; ++q) { const int e = LANE_ID + N_LANES * q; if (e < R_BWD) R[e] = rs.pre[q]; }
-    if (rk_next) rec_prefetch(rs, rk_next);
-    W_SYNC();
-    return R;
-#else
-    (void)rs; (void)rk_next; (void)sm;
-    return rk;
-#endif
-}
-
 #if KKT_USE_TMA
 typedef RecRing KktIo;
 #else
@@ -707,20 +655,20 @@ struct KktIo { int unused; };
 // Riccati backward sweep with regularisation dw on every primal variable (and slack).  Returns false when
 // some R_k + B_k' P_{k+1} B_k is not positive definite (wrong inertia).
 MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo& io) {
-    const int lane = LANE_ID;
+    const int lane = KktLanes::id();
     double* P = sm + KktScratch::P; double* p = sm + KktScratch::p; double* M = sm + KktScratch::M;
     double* q = sm + KktScratch::q; double* T = sm + KktScratch::T; double* f = sm + KktScratch::f;
     double* Kk = sm + KktScratch::K; double* kk = sm + KktScratch::kk; double* cf = sm + KktScratch::cf;
     // ---- terminal stage
     {
         const double* t = I.trec;
-        for (int e = lane; e < NXA * NXA; e += N_LANES) {
+        for (int e = lane; e < NXA * NXA; e += KktLanes::n) {
             const int i = e % NXA, j = e / NXA;
             double v = t[T_H + e];
             if (i == j) v += dwreg + t[T_ZL + i] * t[T_IL + i] + t[T_ZU + i] * t[T_IU + i];
             P[e] = v;
         }
-        for (int i = lane; i < NXA; i += N_LANES) p[i] = t[T_GN + i] - mu * t[T_IL + i] + mu * t[T_IU + i];
+        for (int i = lane; i < NXA; i += KktLanes::n) p[i] = t[T_GN + i] - mu * t[T_IL + i] + mu * t[T_IU + i];
     }
 #if MPCB_TERMCONS
     // Terminal equality E dx_N = -r_T with multiplier nu (new value solved for directly).  By linearity of the sweep
@@ -731,11 +679,11 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
     double* Pi = sm + KktScratch::PiA; double* Pn = sm + KktScratch::PiB;
     double* BtPi = sm + KktScratch::BtPi; double* Ga = sm + KktScratch::Ga;
     double* Gm = sm + KktScratch::Gm; double* hT = sm + KktScratch::hT;
-    for (int e = lane; e < NXA * NXT; e += N_LANES) Pi[e] = (e % NXA == e / NXA) ? 1.0 : 0.0;
-    for (int e = lane; e < NXT * NXT; e += N_LANES) Gm[e] = 0.0;
-    for (int e = lane; e < NXT; e += N_LANES) hT[e] = 0.0;
+    for (int e = lane; e < NXA * NXT; e += KktLanes::n) Pi[e] = (e % NXA == e / NXA) ? 1.0 : 0.0;
+    for (int e = lane; e < NXT * NXT; e += KktLanes::n) Gm[e] = 0.0;
+    for (int e = lane; e < NXT; e += KktLanes::n) hT[e] = 0.0;
 #endif
-    W_SYNC();
+    KktLanes::sync();
 #if KKT_USE_TMA
     // the first KKT_NBUF - 1 records are requested up front, record k - (KKT_NBUF - 1) when stage k starts: the copies
     // stay that many stages ahead of the compute
@@ -745,23 +693,21 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
             io.issue((NH - 1 - d) % KKT_NBUF, I.rec + (NH - 1 - d) * REC_SZ, KKT_RBUF, nullptr, 0);
 #else
     (void)io;
-    RecStream rs;
-    rec_prefetch(rs, I.rec + (NH - 1) * REC_SZ);
 #endif
     for (int k = NH - 1; k >= 0; --k) {
 #if KKT_USE_TMA
         if (lane == 0 && k >= AHEAD) io.issue((k - AHEAD) % KKT_NBUF, I.rec + (k - AHEAD) * REC_SZ, KKT_RBUF, nullptr, 0);
         const double* R = io.wait(k % KKT_NBUF);
 #else
-        const double* R = stage_record(rs, I.rec + k * REC_SZ, (k > 0) ? I.rec + (k - 1) * REC_SZ : nullptr, sm);
+        const double* R = I.rec + k * REC_SZ;          // one lane: the record is read in place
 #endif
         double* fk = I.frec + k * FREC_SZ;
         // (a) P_{k+1}, p_{k+1} go to the forward record; slack coefficients
-        for (int e = lane; e < NXA * NXA; e += N_LANES) fk[FREC_P + e] = P[e];
-        for (int e = lane; e < NXA; e += N_LANES) fk[FREC_PV + e] = p[e];
+        for (int e = lane; e < NXA * NXA; e += KktLanes::n) fk[FREC_P + e] = P[e];
+        for (int e = lane; e < NXA; e += KktLanes::n) fk[FREC_PV + e] = p[e];
 #if MPCB_TERMCONS
-        for (int e = lane; e < NXA * NXT; e += N_LANES) fk[FREC_PI + e] = Pi[e];
-        for (int e = lane; e < NU * NXT; e += N_LANES) {
+        for (int e = lane; e < NXA * NXT; e += KktLanes::n) fk[FREC_PI + e] = Pi[e];
+        for (int e = lane; e < NU * NXT; e += KktLanes::n) {
             const int l = e % NU, j = e / NU;
             double a = 0.0;
             for (int i = 0; i < NXA; ++i) a += R[R_AB + NXA * NXA + i + NXA * l] * Pi[i + NXA * j];
@@ -769,24 +715,24 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
         }
 #endif
 #if NG > 0
-        for (int r = lane; r < NG; r += N_LANES)
+        for (int r = lane; r < NG; r += KktLanes::n)
             cf[r] = (R[R_SG + r] + dwreg) * R[R_RG + r] - mu * R[R_ISL + r] + mu * R[R_ISU + r];
 #endif
         // (b) f = P c + p ;  T = P [A B]
-        for (int i = lane; i < NXA; i += N_LANES) {
+        for (int i = lane; i < NXA; i += KktLanes::n) {
             double a = p[i];
             for (int j = 0; j < NXA; ++j) a += P[i + NXA * j] * R[R_C + j];
             f[i] = a;
         }
-        for (int e = lane; e < NXA * NZA; e += N_LANES) {
+        for (int e = lane; e < NXA * NZA; e += KktLanes::n) {
             const int i = e % NXA, j = e / NXA;
             double a = 0.0;
             for (int l = 0; l < NXA; ++l) a += P[i + NXA * l] * R[R_AB + l + NXA * j];
             T[e] = a;
         }
-        W_SYNC();
+        KktLanes::sync();
         // (c) M = M0 + dw (I + G'G) + [A B]' P [A B] ;  q = grad - mu/dL + mu/dU + G' cf + [A B]' f
-        for (int e = lane; e < NZA * NZA; e += N_LANES) {
+        for (int e = lane; e < NZA * NZA; e += KktLanes::n) {
             const int i = e % NZA, j = e / NZA;
             double m = R[R_M + e] + (i == j ? dwreg : 0.0);
 #if NG > 0
@@ -795,7 +741,7 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
             for (int l = 0; l < NXA; ++l) m += R[R_AB + l + NXA * i] * T[l + NXA * j];
             M[e] = m;
         }
-        for (int i = lane; i < NZA; i += N_LANES) {
+        for (int i = lane; i < NZA; i += KktLanes::n) {
             double a = R[R_GL + i] - mu * R[R_IL + i] + mu * R[R_IU + i];
 #if NG > 0
             for (int r = 0; r < NG; ++r) a += R[R_G + r + NG * i] * cf[r];
@@ -803,7 +749,7 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
             for (int l = 0; l < NXA; ++l) a += R[R_AB + l + NXA * i] * f[l];
             q[i] = a;
         }
-        W_SYNC();
+        KktLanes::sync();
         // (d) Cholesky of the input block M_uu = L L' (every lane, in registers); Li = 1 / diag(L)
         double L[NU * NU], Li[NU];
         bool pd = true;
@@ -828,12 +774,12 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
 #if KKT_USE_TMA
             for (int d = 1; d <= KKT_NBUF - 1; ++d)              // drain the copies in flight before the sweep is repeated
                 if (k >= d) io.wait((k - d) % KKT_NBUF);
-            W_SYNC();
+            KktLanes::sync();
 #endif
             return false;
         }
         // (e) K = -Muu^{-1} Mux (NU x NXA), kff = -Muu^{-1} q_u : one column per lane
-        for (int c = lane; c <= NXA + NXT; c += N_LANES) {
+        for (int c = lane; c <= NXA + NXT; c += KktLanes::n) {
             double y[NU];
             for (int i = 0; i < NU; ++i) {
 #if MPCB_TERMCONS
@@ -857,22 +803,22 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
 #endif
             }
         }
-        W_SYNC();
+        KktLanes::sync();
 #if MPCB_TERMCONS
-        for (int e = lane; e < NXA * NXT; e += N_LANES) {
+        for (int e = lane; e < NXA * NXT; e += KktLanes::n) {
             const int i = e % NXA, j = e / NXA;
             double a = 0.0;
             for (int l = 0; l < NXA; ++l) a += R[R_AB + l + NXA * i] * Pi[l + NXA * j];
             for (int m = 0; m < NU; ++m) a += Kk[m + NU * i] * BtPi[m + NU * j];
             Pn[e] = a;
         }
-        for (int e = lane; e < NXT * NXT; e += N_LANES) {
+        for (int e = lane; e < NXT * NXT; e += KktLanes::n) {
             const int j1 = e % NXT, j2 = e / NXT;
             double a = Gm[e];
             for (int m = 0; m < NU; ++m) a -= BtPi[m + NU * j1] * Ga[m + NU * j2];
             Gm[e] = a;
         }
-        for (int j = lane; j < NXT; j += N_LANES) {
+        for (int j = lane; j < NXT; j += KktLanes::n) {
             double a = hT[j];
             for (int i = 0; i < NXA; ++i) {
                 double bc = R[R_C + i];
@@ -884,28 +830,30 @@ MPCB_HD bool ocp_riccati(OcpInst& I, double mu, double dwreg, double* sm, KktIo&
         { double* tmp = Pi; Pi = Pn; Pn = tmp; }
 #endif
         // (f) P = Mxx + Mxu K (symmetrised), p = q_x + Mxu kff
-        for (int e = lane; e < NXA * NXA; e += N_LANES) {
+        for (int e = lane; e < NXA * NXA; e += KktLanes::n) {
             const int i = e % NXA, j = e / NXA;
             double a = M[i + NZA * j], b = M[j + NZA * i];
             for (int l = 0; l < NU; ++l) { a += M[i + NZA * (NXA + l)] * Kk[l + NU * j]; b += M[j + NZA * (NXA + l)] * Kk[l + NU * i]; }
             P[e] = (i == j) ? a : 0.5 * (a + b);
         }
-        for (int i = lane; i < NXA; i += N_LANES) {
+        for (int i = lane; i < NXA; i += KktLanes::n) {
             double a = q[i];
             for (int l = 0; l < NU; ++l) a += M[i + NZA * (NXA + l)] * kk[l];
             p[i] = a;
         }
-        W_SYNC();
+        KktLanes::sync();
     }
     return true;
 }
 
+// end the solve of the instance run by the lane group G (ocp_kkt: KktLanes, ocp_accept: WarpLanes)
+template <class G>
 MPCB_HD void ocp_finish(OcpInst& I, const OcpShared& S, int status, double fval) {
     InstState& st = *I.st;
     if (S.o.honor_original_bounds)
-        for (int i = NXA + LANE_ID; i < NWI; i += N_LANES) I.w[i] = fmin(fmax(I.w[i], S.lbx[i]), S.ubx[i]);
-    if (LANE_ID == 0) { st.status = status; st.state = ST_DONE; st.fval = fval; }
-    W_SYNC();
+        for (int i = NXA + G::id(); i < NWI; i += G::n) I.w[i] = fmin(fmax(I.w[i], S.lbx[i]), S.ubx[i]);
+    if (G::id() == 0) { st.status = status; st.state = ST_DONE; st.fval = fval; }
+    G::sync();
 }
 
 // Step-size bookkeeping for one bounded quantity with step dv, division free:
@@ -924,18 +872,18 @@ MPCB_HD void step_terms(double dv, double iL, double iU, double qL, double qU, d
 MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
     InstState& st = *I.st;
     const double rf = S.o.bound_relax;
-    const int lane = LANE_ID;
+    const int lane = KktLanes::id();
     const int iter = st.iter;
     // ---- reduce the per-stage partials written by the evaluation
     double fobj = 0.0, theta = 0.0, dual = 0.0, prim = 0.0, ysum = 0.0, zsum = 0.0, nbd = 0.0, pmin = 1e300, pmax = -1e300;
     double barr = 0.0;
-    for (int k = lane; k <= NH; k += N_LANES) {
+    for (int k = lane; k <= NH; k += KktLanes::n) {
         const double* pp = (k < NH) ? (I.rec + k * REC_SZ + R_PART) : (I.trec + T_PART);
         fobj += pp[0]; theta += pp[1]; dual = fmax(dual, pp[2]); prim = fmax(prim, pp[3]); ysum += pp[4];
         zsum += pp[5]; nbd += pp[6]; pmin = fmin(pmin, pp[7]); pmax = fmax(pmax, pp[8]); barr += pp[9];
     }
-    fobj = W_SUM(fobj); theta = W_SUM(theta); dual = W_MAX(dual); prim = W_MAX(prim); ysum = W_SUM(ysum);
-    zsum = W_SUM(zsum); nbd = W_SUM(nbd); pmin = W_MIN(pmin); pmax = W_MAX(pmax); barr = W_SUM(barr);
+    fobj = KktLanes::sum(fobj); theta = KktLanes::sum(theta); dual = KktLanes::max(dual); prim = KktLanes::max(prim); ysum = KktLanes::sum(ysum);
+    zsum = KktLanes::sum(zsum); nbd = KktLanes::sum(nbd); pmin = KktLanes::min(pmin); pmax = KktLanes::max(pmax); barr = KktLanes::sum(barr);
 #if NG > 0
     // A stage-0 range row that does not depend on u_0 is a constant (x_0 is fixed).  Outside its relaxed
     // bounds the OCP is infeasible: IPOPT would end in restoration with Infeasible_Problem_Detected, the
@@ -950,7 +898,7 @@ MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
             const double v = r0[R_GV + r], lo = S.lbg[r], hi = S.ubg[r];
             if ((fin(lo) && v < rlo(lo, rf) - S.o.tol) || (fin(hi) && v > rhi(hi, rf) + S.o.tol)) infeasible = true;
         }
-        if (infeasible) { ocp_finish(I, S, 2, fobj); return; }
+        if (infeasible) { ocp_finish<KktLanes>(I, S, 2, fobj); return; }
     }
 #endif
     // ---- optimality error and termination (IPOPT: tol, dual_inf_tol=1, constr_viol_tol=1e-4, compl_inf_tol=1e-4)
@@ -963,19 +911,19 @@ MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
     const double E0 = fmax(fmax(dual / sd, prim), c0 / sc);
     int acc_cnt = st.acc_cnt;
     const bool resto = st.resto != 0;     // restoration iteration: no termination test, no barrier update (see ocp_accept)
-    W_SYNC();
+    KktLanes::sync();
     if (lane == 0) st.E0 = E0;
-    if (!(E0 == E0) || !fin(E0)) { ocp_finish(I, S, -13, fobj); return; }
+    if (!(E0 == E0) || !fin(E0)) { ocp_finish<KktLanes>(I, S, -13, fobj); return; }
     if (!resto) {
-        if (E0 <= S.o.tol && dual <= 1.0 && prim <= 1e-4 && c0 <= 1e-4) { ocp_finish(I, S, 0, fobj); return; }
+        if (E0 <= S.o.tol && dual <= 1.0 && prim <= 1e-4 && c0 <= 1e-4) { ocp_finish<KktLanes>(I, S, 0, fobj); return; }
         if (E0 <= S.o.acceptable_tol && dual <= 1e10 && prim <= 1e-2 && c0 <= 1e-2) {
             acc_cnt += 1;
-            if (acc_cnt >= S.o.acceptable_iter) { ocp_finish(I, S, 1, fobj); return; }
+            if (acc_cnt >= S.o.acceptable_iter) { ocp_finish<KktLanes>(I, S, 1, fobj); return; }
         } else {
             acc_cnt = 0;
         }
     }
-    if (iter >= S.o.max_iter) { ocp_finish(I, S, -1, fobj); return; }
+    if (iter >= S.o.max_iter) { ocp_finish<KktLanes>(I, S, -1, fobj); return; }
     // ---- monotone barrier update (kappa_eps=10, kappa_mu=0.2, theta_mu=1.5)
     double mu = st.mu;
     const double mu_min = S.o.tol / 10.0;
@@ -990,23 +938,23 @@ MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
     const double tau = changed ? fmax(0.99, 1.0 - mu) : st.tau;
     const double dw_last = st.dw_last;
     const double theta0_old = st.theta0;
-    W_SYNC();
+    KktLanes::sync();
     // ---- Newton step by Riccati recursion, inertia-correcting ladder on delta_w
     double dwreg = 0.0;
     bool first = true, ok = false;
     KktIo io;
 #if KKT_USE_TMA
     io.init(sm, lane);
-    W_SYNC();
+    KktLanes::sync();
 #endif
     for (int attempt = 0; attempt < 60; ++attempt) {
         if (ocp_riccati(I, mu, dwreg, sm, io)) { ok = true; break; }
-        W_SYNC();
+        KktLanes::sync();
         if (first) { dwreg = (dw_last == 0.0) ? 1e-4 : fmax(1e-20, dw_last / 3.0); first = false; }
         else dwreg *= (dw_last == 0.0) ? 100.0 : 8.0;
         if (dwreg > 1e40) break;
     }
-    if (!ok) { ocp_finish(I, S, -3, fobj); return; }
+    if (!ok) { ocp_finish<KktLanes>(I, S, -3, fobj); return; }
 #if MPCB_TERMCONS
     // ---- multiplier of the terminal equality: G nu = h + r_T (G is the horizon's reachability Gramian weighted by
     //      Muu^{-1}: positive definite when x_s can be reached; otherwise IPOPT's jacobian_regularization delta_c)
@@ -1030,7 +978,7 @@ MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
                 }
             }
         }
-        if (!pd) { ocp_finish(I, S, -3, fobj); return; }
+        if (!pd) { ocp_finish<KktLanes>(I, S, -3, fobj); return; }
         for (int i = 0; i < NXT; ++i) {
             double a = hT[i] + I.trec[T_RT + i];
             for (int l = 0; l < i; ++l) a -= L[i + NXT * l] * y[l];
@@ -1041,16 +989,16 @@ MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
             for (int l = i + 1; l < NXT; ++l) a -= L[l + NXT * i] * y[l];
             y[i] = a / L[i + NXT * i];
         }
-        W_SYNC();
-        for (int i = lane; i < NXT; i += N_LANES) { nuS[i] = y[i]; I.nuTn[i] = y[i]; }
-        W_SYNC();
+        KktLanes::sync();
+        for (int i = lane; i < NXT; i += KktLanes::n) { nuS[i] = y[i]; I.nuTn[i] = y[i]; }
+        KktLanes::sync();
     }
 #endif
     // ---- forward sweep, sequential part: only  du_k = K_k dx_k + k_k  and  dx_{k+1} = A dx_k + B du_k + c  (two lane
-    //      phases per stage; the [A|B], c head of the record and the K, k head of the forward record are prefetched
-    //      one stage ahead, one double per lane)
+    //      phases per stage; the [A|B], c head of the record and the K, k head of the forward record come through the
+    //      ring with lane groups and are read in place with one lane)
     double* dxa = sm + KktScratch::dx; double* du = sm + KktScratch::du; double* dxb = sm + KktScratch::dxn;
-    for (int i = lane; i < NXA; i += N_LANES) { dxa[i] = 0.0; I.dw[i] = 0.0; }
+    for (int i = lane; i < NXA; i += KktLanes::n) { dxa[i] = 0.0; I.dw[i] = 0.0; }
 #if KKT_USE_TMA
     // [A|B], c head of the record and K, k head of the forward record of stage k: two bulk copies into one ring buffer,
     // requested two stages ahead.  The forward records were written by this warp's ordinary stores in the backward sweep:
@@ -1058,45 +1006,22 @@ MPCB_HD void ocp_kkt(OcpInst& I, const OcpShared& S, double* sm) {
     constexpr int NHEAD = (R_C + NXA + 1) / 2 * 2, NFH = (FREC_P + 1) / 2 * 2;
     static_assert(NHEAD + NFH <= KKT_RBUF, "forward heads must fit a ring buffer");
     asm volatile("fence.proxy.async;" ::: "memory");
-    W_SYNC();
+    KktLanes::sync();
     if (lane == 0)
         for (int d = 0; d < KKT_NBUF - 1 && d < NH; ++d)
             io.issue(d % KKT_NBUF, I.rec + d * REC_SZ, NHEAD, I.frec + d * FREC_SZ, NFH);
-#elif KKT_ON_LANES
-    constexpr int NHEAD = R_C + NXA, NFH = FREC_P;              // doubles needed per stage: record head, forward-record head
-    constexpr int HPL = (NHEAD + NFH + N_LANES - 1) / N_LANES;
-    double* Rs = sm + KktScratch::R;                            // staged: [record head | forward-record head]
-    double hpre[HPL];
-MPCB_UNROLL
-    for (int q = 0; q < HPL; ++q) {
-        const int e = lane + N_LANES * q;
-        hpre[q] = (e < NHEAD) ? I.rec[e] : ((e < NHEAD + NFH) ? I.frec[e - NHEAD] : 0.0);
-    }
 #endif
-    W_SYNC();
+    KktLanes::sync();
     for (int k = 0; k < NH; ++k) {
         double* dx = (k & 1) ? dxb : dxa; double* dxn = (k & 1) ? dxa : dxb;
 #if KKT_USE_TMA
         if (lane == 0 && k + KKT_NBUF - 1 < NH)
             io.issue((k + KKT_NBUF - 1) % KKT_NBUF, I.rec + (k + KKT_NBUF - 1) * REC_SZ, NHEAD, I.frec + (k + KKT_NBUF - 1) * FREC_SZ, NFH);
         const double* R = io.wait(k % KKT_NBUF); const double* F = R + NHEAD;
-#elif KKT_ON_LANES
-MPCB_UNROLL
-        for (int q = 0; q < HPL; ++q) { const int e = lane + N_LANES * q; if (e < NHEAD + NFH) Rs[e] = hpre[q]; }
-        if (k + 1 < NH) {
-            const double* rn = I.rec + (k + 1) * REC_SZ; const double* fn = I.frec + (k + 1) * FREC_SZ;
-MPCB_UNROLL
-            for (int q = 0; q < HPL; ++q) {
-                const int e = lane + N_LANES * q;
-                hpre[q] = (e < NHEAD) ? rn[e] : ((e < NHEAD + NFH) ? fn[e - NHEAD] : 0.0);
-            }
-        }
-        W_SYNC();
-        const double* R = Rs; const double* F = Rs + NHEAD;
 #else
         const double* R = I.rec + k * REC_SZ; const double* F = I.frec + k * FREC_SZ;
 #endif
-        for (int i = lane; i < NU; i += N_LANES) {
+        for (int i = lane; i < NU; i += KktLanes::n) {
             double a = F[FREC_KF + i];
             for (int j = 0; j < NXA; ++j) a += F[FREC_K + i + NU * j] * dx[j];
 #if MPCB_TERMCONS
@@ -1105,20 +1030,20 @@ MPCB_UNROLL
             du[i] = a;
             I.dw[k * NZA + NXA + i] = a;
         }
-        W_SYNC();
-        for (int i = lane; i < NXA; i += N_LANES) {
+        KktLanes::sync();
+        for (int i = lane; i < NXA; i += KktLanes::n) {
             double a = R[R_C + i];
             for (int j = 0; j < NXA; ++j) a += R[R_AB + i + NXA * j] * dx[j];
             for (int j = 0; j < NU; ++j) a += R[R_AB + NXA * NXA + i + NXA * j] * du[j];
             dxn[i] = a;
             I.dw[(k + 1) * NZA + i] = a;
         }
-        W_SYNC();
+        KktLanes::sync();
     }
     // ---- stage-parallel part (lanes over stages): new dynamics multipliers, slack / multiplier steps of the range
     //      rows, fraction to the boundary (primal and dual) and the directional derivative of the barrier function
     double rp = 0.0, rd = 0.0, gphid = 0.0;       // largest primal / dual boundary ratios, directional derivative
-    for (int k = lane; k <= NH; k += N_LANES) {
+    for (int k = lane; k <= NH; k += KktLanes::n) {
         if (k == NH) {
             const double* t = I.trec;
             for (int j = 0; j < NXA; ++j) {
@@ -1153,7 +1078,7 @@ MPCB_UNROLL
         }
 #endif
     }
-    rp = W_MAX(rp); rd = W_MAX(rd); gphid = W_SUM(gphid);
+    rp = KktLanes::max(rp); rd = KktLanes::max(rd); gphid = KktLanes::sum(gphid);
     const double amax = (rp > tau) ? tau / rp : 1.0;
     const double az = (rd > tau) ? tau / rd : 1.0;
     const double phi = fobj - mu * barr;
@@ -1179,7 +1104,7 @@ MPCB_UNROLL
         st.ls_iter = 0;
         st.state = ST_LS;
     }
-    W_SYNC();
+    KktLanes::sync();
 }
 
 // =============================================================================================
@@ -1263,42 +1188,13 @@ MPCB_UNROLL
 // accept: filter line-search decision for one instance.  Always one warp per instance on the device
 // (the updates are element-wise over w, lam, s, z), one lane on the host.
 // =============================================================================================
-#undef LANE_ID
-#undef N_LANES
-#undef W_SYNC
-#undef W_SUM
-#undef W_MAX
-#undef W_MIN
-#undef GROUP_MASK
-#ifdef __CUDA_ARCH__
-#  define LANE_ID   ((int)(threadIdx.x & 31))
-#  define N_LANES   32
-#  define W_SYNC()  __syncwarp()
-#  define W_SUM(v)  warp_sum(v)
-#  define W_MAX(v)  warp_max(v)
-#  define W_MIN(v)  warp_min(v)
-#else
-#  define LANE_ID   0
-#  define N_LANES   1
-#  define W_SYNC()
-#  define W_SUM(v)  (v)
-#  define W_MAX(v)  (v)
-#  define W_MIN(v)  (v)
-#endif
-MPCB_HD void ocp_finish_w(OcpInst& I, const OcpShared& S, int status, double fval) {
-    InstState& st = *I.st;
-    if (S.o.honor_original_bounds)
-        for (int i = NXA + LANE_ID; i < NWI; i += N_LANES) I.w[i] = fmin(fmax(I.w[i], S.lbx[i]), S.ubx[i]);
-    if (LANE_ID == 0) { st.status = status; st.state = ST_DONE; st.fval = fval; }
-    W_SYNC();
-}
 MPCB_HD void ocp_accept(OcpInst& I, const OcpShared& S) {
     InstState& st = *I.st;
-    const int lane = LANE_ID;
+    const int lane = WarpLanes::id();
     const double rf = S.o.bound_relax, mu = st.mu;
     double th_t = 0.0, f_t = 0.0, b_t = 0.0;
-    for (int k = lane; k <= NH; k += N_LANES) { f_t += I.partt[k * 4 + 0]; th_t += I.partt[k * 4 + 1]; b_t += I.partt[k * 4 + 2]; }
-    th_t = W_SUM(th_t); f_t = W_SUM(f_t); b_t = W_SUM(b_t);
+    for (int k = lane; k <= NH; k += WarpLanes::n) { f_t += I.partt[k * 4 + 0]; th_t += I.partt[k * 4 + 1]; b_t += I.partt[k * 4 + 2]; }
+    th_t = WarpLanes::sum(th_t); f_t = WarpLanes::sum(f_t); b_t = WarpLanes::sum(b_t);
     const double ph_t = f_t - mu * b_t;
     const double theta = st.theta, phi = st.phi, gphid = st.gphid, alpha = st.alpha, az = st.alpha_z;
     const double theta_min = 1e-4 * fmax(1.0, st.theta0), theta_max = 1e4 * fmax(1.0, st.theta0);
@@ -1320,7 +1216,7 @@ MPCB_HD void ocp_accept(OcpInst& I, const OcpShared& S) {
     const double amin = st.amin;
     const int resto = st.resto, resto_calls = st.resto_calls;
     const double theta_entry = st.theta_entry;
-    W_SYNC();
+    WarpLanes::sync();
     if (resto) {
         // ---- restoration iteration (proximal Gauss-Newton step on the constraint violation, see ocp_eval_stage):
         //      Armijo backtracking on the violation alone; multipliers restart from zero / mu over the slack; back to
@@ -1328,24 +1224,24 @@ MPCB_HD void ocp_accept(OcpInst& I, const OcpShared& S) {
         //      (which holds the entry point) accepts the new point
         // a step shorter than 1e-5 of the Gauss-Newton step (jammed against the bounds, or no descent): the violation
         // cannot be reduced - a stationary point of the infeasibility (IPOPT: Infeasible_Problem_Detected)
-        if (!(alpha > 1e-5)) { ocp_finish_w(I, S, theta > 1e-4 ? 2 : -2, st.fval); return; }
+        if (!(alpha > 1e-5)) { ocp_finish<WarpLanes>(I, S, theta > 1e-4 ? 2 : -2, st.fval); return; }
         const bool fine = (th_t == th_t) && fin(th_t) && th_t <= (1.0 - 1e-4 * alpha) * theta;
         if (!fine) {
             if (lane == 0) { st.alpha = 0.5 * alpha; st.ls_iter += 1; }
-            W_SYNC();
+            WarpLanes::sync();
             return;
         }
-        for (int i = NXA + lane; i < NWI; i += N_LANES) {
+        for (int i = NXA + lane; i < NWI; i += WarpLanes::n) {
             const double lo = S.lbx[i], hi = S.ubx[i];
             const double wn = I.w[i] + alpha * I.dw[i];
             if (fin(lo)) I.zL[i] = mu / (wn - rlo(lo, rf));
             if (fin(hi)) I.zU[i] = mu / (rhi(hi, rf) - wn);
             I.w[i] = wn;
         }
-        for (int i = lane; i < NH * NXA; i += N_LANES) I.lam[i] = 0.0;
-        for (int i = lane; i < NXT; i += N_LANES) I.nuT[i] = 0.0;
+        for (int i = lane; i < NH * NXA; i += WarpLanes::n) I.lam[i] = 0.0;
+        for (int i = lane; i < NXT; i += WarpLanes::n) I.nuT[i] = 0.0;
 #if NG > 0
-        for (int i = lane; i < NH * NG; i += N_LANES) {
+        for (int i = lane; i < NH * NG; i += WarpLanes::n) {
             const double lo = S.lbg[i], hi = S.ubg[i];
             const double sn = I.s[i] + alpha * I.ds[i];
             if (fin(lo)) I.vL[i] = mu / (sn - rlo(lo, rf));
@@ -1359,34 +1255,34 @@ MPCB_HD void ocp_accept(OcpInst& I, const OcpShared& S) {
             for (int i = 0; i < nfilt; ++i)
                 if (th_t >= st.filt[2 * i] && ph_t >= st.filt[2 * i + 1]) { leave = false; break; }
         if (lane == 0) { st.iter += 1; st.state = ST_EVAL; if (leave) st.resto = 0; }
-        W_SYNC();
+        WarpLanes::sync();
         return;
     }
     if (!accepted) {
         const double an = 0.5 * alpha;
         const bool give_up = !(an >= amin * (1.0 - 1e-12)) || an <= 1e-16;
         if (lane == 0) { st.alpha = an; st.ls_iter += 1; }
-        W_SYNC();
+        WarpLanes::sync();
         if (give_up) {
             // IPOPT enters its restoration phase here: it looks for a point whose violation is kappa_resto times the
             // current one and which the filter, augmented by the current point, accepts; it reports
             // Infeasible_Problem_Detected (the status the reference loop acts on, MPC_code.py:786) when it ends at a
             // stationary point of the violation, and Restoration_Failed when called at an (almost) feasible point.
             // Same entry, goal and exits here; the sub-solver is simpler (proximal Gauss-Newton instead of an l1 IPM).
-            if (theta < 1e-6 || resto_calls >= 3) { ocp_finish_w(I, S, theta > 1e-4 ? 2 : -2, st.fval); return; }
+            if (theta < 1e-6 || resto_calls >= 3) { ocp_finish<WarpLanes>(I, S, theta > 1e-4 ? 2 : -2, st.fval); return; }
             if (lane == 0) {
                 if (nfilt < MPCB_MAXFILT) {
                     st.filt[2 * nfilt] = (1.0 - 1e-5) * theta; st.filt[2 * nfilt + 1] = phi - 1e-8 * theta; st.nfilt = nfilt + 1;
                 }
                 st.resto = 1; st.resto_calls = resto_calls + 1; st.theta_entry = theta; st.state = ST_EVAL;
             }
-            W_SYNC();
+            WarpLanes::sync();
         }
         return;
     }
     // ---- take the step; bound multipliers with their own step size, then the kappa_sigma safeguard
     const double ks = 1e10;
-    for (int i = NXA + lane; i < NWI; i += N_LANES) {
+    for (int i = NXA + lane; i < NWI; i += WarpLanes::n) {
         const double lo = S.lbx[i], hi = S.ubx[i], dv = I.dw[i];
         const double wn = I.w[i] + alpha * dv;
         if (fin(lo)) {
@@ -1401,10 +1297,10 @@ MPCB_HD void ocp_accept(OcpInst& I, const OcpShared& S) {
         }
         I.w[i] = wn;
     }
-    for (int i = lane; i < NH * NXA; i += N_LANES) I.lam[i] += alpha * (I.lamn[i] - I.lam[i]);
-    for (int i = lane; i < NXT; i += N_LANES) I.nuT[i] += alpha * (I.nuTn[i] - I.nuT[i]);
+    for (int i = lane; i < NH * NXA; i += WarpLanes::n) I.lam[i] += alpha * (I.lamn[i] - I.lam[i]);
+    for (int i = lane; i < NXT; i += WarpLanes::n) I.nuT[i] += alpha * (I.nuTn[i] - I.nuT[i]);
 #if NG > 0
-    for (int i = lane; i < NH * NG; i += N_LANES) {
+    for (int i = lane; i < NH * NG; i += WarpLanes::n) {
         const double lo = S.lbg[i], hi = S.ubg[i], dv = I.ds[i];
         const double sn = I.s[i] + alpha * dv;
         if (fin(lo)) {
@@ -1430,5 +1326,5 @@ MPCB_HD void ocp_accept(OcpInst& I, const OcpShared& S) {
         st.iter += 1;
         st.state = ST_EVAL;
     }
-    W_SYNC();
+    WarpLanes::sync();
 }

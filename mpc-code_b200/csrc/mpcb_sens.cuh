@@ -79,18 +79,6 @@ MPCB_HD void sens_mixed_term(const OcpInst& I, double* QT, double* RT) {
 }
 
 // ---- factor: one instance, lanes as in ocp_kkt (ocp_riccati runs on them) ----------------------------------------
-#if defined(__CUDA_ARCH__) && (MPCB_KKT_LANES > 1)
-#  define S_LANE ((int)(threadIdx.x & (MPCB_KKT_LANES - 1)))
-#  define S_NL   MPCB_KKT_LANES
-#  define S_MASK (MPCB_KKT_LANES == 32 ? 0xffffffffu : \
-                  (((1u << (MPCB_KKT_LANES & 31)) - 1u) << ((threadIdx.x & 31) & ~(MPCB_KKT_LANES - 1))))
-#  define S_SYNC() __syncwarp(S_MASK)
-#else
-#  define S_LANE 0
-#  define S_NL   1
-#  define S_SYNC()
-#endif
-
 // Cholesky L L' = A of an n x n SPD matrix (column-major, lower part read); Li = 1 / diag(L).  False if not SPD.
 template <int n>
 MPCB_HD bool sens_chol(const double* A, double* L, double* Li) {
@@ -117,33 +105,33 @@ MPCB_HD void sens_chol_solve(const double* L, const double* Li, double* b) {    
 
 // Status: 0 computed, 1 the solve did not end with status 0 / 1, 2 wrong inertia at delta_w = 0.
 MPCB_HD int ocp_sens_factor(const OcpInst& I, double* fac, double* sm) {
-    const int lane = S_LANE;
+    const int lane = KktLanes::id();
     const int solve_status = I.st->status;
     if (solve_status != 0 && solve_status != 1) {
         if (lane == 0) fac[SensLayout::head] = 1.0;
-        S_SYNC();
+        KktLanes::sync();
         return 1;
     }
     // mixed blocks (stage-parallel over the lanes) and the [A|B] blocks
-    for (int k = lane; k <= NH; k += S_NL) {
+    for (int k = lane; k <= NH; k += KktLanes::n) {
         if (k == NH) { sens_mixed_term(I, fac + SensLayout::qt, fac + SensLayout::rt); continue; }
         sens_mixed_stage(I, k, fac + SensLayout::q + k * NZA * NTH);
         for (int e = 0; e < NXA * NZA; ++e) fac[SensLayout::ab + k * NXA * NZA + e] = I.rec[k * REC_SZ + R_AB + e];
     }
-    S_SYNC();
+    KktLanes::sync();
     // backward Riccati sweep with delta_w = 0; its forward records (K, P_{k+1}, Gamma, Pi_{k+1}) go to fac
     OcpInst Ic = I;
     Ic.frec = fac + SensLayout::frec;
     KktIo io;
 #if KKT_USE_TMA
     io.init(sm, lane);
-    S_SYNC();
+    KktLanes::sync();
 #endif
     bool ok = ocp_riccati(Ic, I.st->mu, 0.0, sm, io);
-    S_SYNC();
+    KktLanes::sync();
     // Cholesky factors of R~_k = M_uu + B' P_{k+1} B (stage-parallel; the sweep keeps them only in registers)
     bool pd = ok;
-    for (int k = lane; ok && k < NH; k += S_NL) {
+    for (int k = lane; ok && k < NH; k += KktLanes::n) {
         const double* R = I.rec + k * REC_SZ; const double* F = fac + SensLayout::frec + k * FREC_SZ;
         double Muu[NU * NU];
         for (int j = 0; j < NU; ++j)
@@ -159,9 +147,7 @@ MPCB_HD int ocp_sens_factor(const OcpInst& I, double* fac, double* sm) {
         double* C = fac + SensLayout::chol + k * (NU * NU + NU);
         if (!sens_chol<NU>(Muu, C, C + NU * NU)) pd = false;
     }
-#if defined(__CUDA_ARCH__) && (MPCB_KKT_LANES > 1)
-    pd = __all_sync(S_MASK, pd) != 0;          // over the lanes of this instance only
-#endif
+    pd = KktLanes::all(pd);                    // over the lanes of this instance only
 #if MPCB_TERMCONS
     // Gramian of the terminal equality (no delta_c): Cholesky factor; Pi_0 (the sweep swaps its two Pi buffers per stage)
     if (ok) {
@@ -170,7 +156,7 @@ MPCB_HD int ocp_sens_factor(const OcpInst& I, double* fac, double* sm) {
         double Gs[NXT * NXT], Lg[NXT * NXT], Lgi[NXT];
         for (int j = 0; j < NXT; ++j) for (int i = 0; i < NXT; ++i) Gs[i + NXT * j] = 0.5 * (Gm[i + NXT * j] + Gm[j + NXT * i]);
         if (!sens_chol<NXT>(Gs, Lg, Lgi)) pd = false;
-        S_SYNC();
+        KktLanes::sync();
         if (lane == 0) {
             for (int e = 0; e < NXT * NXT; ++e) fac[SensLayout::gl + e] = Lg[e];
             for (int e = 0; e < NXA * NXT; ++e) fac[SensLayout::pi0 + e] = Pi[e];
@@ -178,9 +164,9 @@ MPCB_HD int ocp_sens_factor(const OcpInst& I, double* fac, double* sm) {
     }
 #endif
     const int status = (ok && pd) ? 0 : 2;
-    S_SYNC();
+    KktLanes::sync();
     if (lane == 0) fac[SensLayout::head] = (double)status;
-    S_SYNC();
+    KktLanes::sync();
     return status;
 }
 

@@ -1,11 +1,10 @@
 """The OCP solve under every build-time kernel mapping the sources keep, and the mappings they refuse.
 
 The KKT kernel (and the sensitivity factor, which shares its mapping) runs on MPCB_KKT_LANES = 32 lanes per instance by
-default; -DMPCB_KKT_LANES=1/16/8/4 are one thread per instance and lane groups, -DMPCB_KKT_TMA=0 stages the records
-through registers instead of the bulk-copy ring, -DMPCB_FUSE_LS=1 runs the line search inside the KKT kernel.  The
-evaluation kernel has its own switches (MPCB_EVAL_FIRST, MPCB_STAGE_CACHE, MPCB_EVAL_SMEM, MPCB_VEC_REC).  Each of these
-is a different device code path; the `-m gpu` tests below build every one listed in PLAN and compare it with the default
-build of the same problem on the same inputs.  Without a GPU: the refusals, and the CPU harness without the stage cache.
+default; -DMPCB_KKT_LANES=1/16/8/4 are one thread per instance and lane groups.  The evaluation kernel has its own
+switches (MPCB_EVAL_FIRST, MPCB_STAGE_CACHE, MPCB_EVAL_SMEM, MPCB_VEC_REC).  Each of these is a different device code
+path; the `-m gpu` tests below build every one listed in PLAN and compare it with the default build of the same problem
+on the same inputs.  Without a GPU: the refusals, and the CPU harness without the stage cache.
 """
 import ctypes
 import os
@@ -29,19 +28,16 @@ def _build(name, flags):
 
 
 # ==== refusals: stop in the compiler's front end, with a message that names the switch ================================
-FUSE_MSG = "MPCB_FUSE_LS=1 requires MPCB_KKT_LANES=32"
 LANES_MSG = "MPCB_KKT_LANES must be one of 1, 2, 4, 8, 16, 32"
 SMEM_MSG = "exceeds the 48 kB of static shared memory"
 
 
 @pytest.mark.parametrize("name, flags, message", [
-    ("nmpc_cstr", ("-DMPCB_FUSE_LS=1", "-DMPCB_KKT_LANES=8"), FUSE_MSG),     # trial loop and ocp_accept would mix instances
-    ("nmpc_cstr", ("-DMPCB_FUSE_LS=1", "-DMPCB_KKT_LANES=1"), FUSE_MSG),     # no warp to run the fused line search on
     ("nmpc_cstr", ("-DMPCB_KKT_LANES=12",), LANES_MSG),
     ("nmpc_cstr", ("-DMPCB_KKT_LANES=64",), LANES_MSG),
     ("syn_12_4_20", ("-DMPCB_KKT_LANES=4",), SMEM_MSG),                     # 8 scratches of 2 510 doubles per warp
     ("syn_20_6_20", ("-DMPCB_KKT_LANES=16",), SMEM_MSG),
-], ids=["fusels-lanes8", "fusels-lanes1", "lanes12", "lanes64", "syn_12_4_20-lanes4", "syn_20_6_20-lanes16"])
+], ids=["lanes12", "lanes64", "syn_12_4_20-lanes4", "syn_20_6_20-lanes16"])
 def test_unsupported_mapping_is_refused_at_compile_time(name, flags, message):
     with pytest.raises(RuntimeError, match="nvcc failed") as err:
         _build(name, flags)
@@ -118,21 +114,19 @@ MAPPINGS = {   # label: (nvcc flags, comparison class with the default build, rt
     "lanes16": (("-DMPCB_KKT_LANES=16",), TOLERANCE, 1e-9),
     "lanes8": (("-DMPCB_KKT_LANES=8",), TOLERANCE, 1e-9),
     "lanes4": (("-DMPCB_KKT_LANES=4",), TOLERANCE, 1e-9),
-    "tma0": (("-DMPCB_KKT_TMA=0",), BITWISE, 0.0),           # staging only
-    "fusels": (("-DMPCB_FUSE_LS=1",), BITWISE, 0.0),         # same device functions, two kernels per tick
     "evalfirst0": (("-DMPCB_EVAL_FIRST=0",), TOLERANCE, 1e-9),
     "stagecache0": (("-DMPCB_STAGE_CACHE=0",), TOLERANCE, 1e-7),
     "evalsmem0": (("-DMPCB_EVAL_SMEM=0",), BITWISE, 0.0),    # sub-step records in local memory
     "vecrec0": (("-DMPCB_VEC_REC=0",), BITWISE, 0.0),        # scalar record stores
 }
-KKT = ("lanes1", "lanes16", "lanes8", "lanes4", "tma0", "fusels")
+KKT = ("lanes1", "lanes16", "lanes8", "lanes4")
 PLAN = {   # problem: the mappings it is checked under (those that change its code and build)
     "nmpc_cstr": KKT + ("evalfirst0", "stagecache0", "evalsmem0", "vecrec0"),   # RK4, output rows, first-tick kernel
     "nmpc_cstr_termcons": KKT,                   # terminal equality: Pi / Gramian scratch, FREC_GA terms
     "lmpc_wb": KKT,                              # Delta-u form: NXA > NX
     "enmpc_reactor": KKT + ("evalsmem0", "vecrec0"),   # ContForm, indefinite Hessian: early sweep exit, restoration
     "syn_4_2_70": KKT,                           # N = 70: several rounds of every stage loop at every lane count
-    "syn_20_6_20": ("lanes1", "tma0"),           # KKT_NBUF = 2, dense derivative path; lane groups do not fit
+    "syn_20_6_20": ("lanes1",),                  # KKT_NBUF = 2, dense derivative path; lane groups do not fit
 }
 ROWS = [(name, label) for name, labels in PLAN.items() for label in labels]
 ROW_IDS = ["%s-%s" % row for row in ROWS]

@@ -15,7 +15,6 @@ VARIANTS = {
     "full_first_eval": "-DMPCB_EVAL_FIRST=0",
 }
 # KKT kernel occupancy (profiles/r02_variants_kktocc.txt): "-DMPCB_KKT_MINBLOCKS=1" (118 regs) | "=5" (96) | "=6" (80)
-# line search fused into the KKT warp: "-DMPCB_FUSE_LS=1" (profiles/r02_variants_fuse.txt)
 # round-2 register/occupancy sweep of k_ocp_eval (profiles/r02_variants_*.txt):
 #   "" (128x3, 168 regs) | -DMPCB_EVAL_MINBLOCKS=2 (254 regs, the default since) |
 #   -DMPCB_EVAL_BLOCK=64 -DMPCB_EVAL_MINBLOCKS=5 -DMPCB_EVAL_MAXNREG=200 | -DMPCB_EVAL_BLOCK=32 -DMPCB_EVAL_MINBLOCKS=9 -DMPCB_EVAL_MAXNREG=224
