@@ -142,6 +142,29 @@ int  mpcb_ocp_sens_factor_p(mpcb_handle_t h, const double* par, double* fac, int
 int  mpcb_ocp_jvp_p(mpcb_handle_t h, const double* fac, int ndir, const double* dp, double* dw, void* stream);
 int  mpcb_ocp_vjp_p(mpcb_handle_t h, const double* fac, const double* gw, double* gp, void* stream);
 
+/* Sensitivities of the steady-state target solution with respect to
+ *   theta_ss = [usp (nu) | ysp (ny) | xsp (nx) | d (nd) | Us_prev (nu) | px (npx) | py (npy)]
+ * (par_ss without vec(lambda) and t, which are held constant; ntheta_ss = 2nu+ny+nx+nd+npx+npy).  The derivative of
+ * the OCP's kind applied to the target's barrier KKT system at the returned iterate: K of the Newton step (Hessian of
+ * the Lagrangian + Sigma = Z/D, with the slacks of User_g_ineq_SS condensed like any bounded variable) without
+ * regularisation, dwss/dtheta_ss = -[K^-1 dF/dtheta_ss]_{0:nwss}.  With honor_original_bounds it is taken at the
+ * iterate before the final clipping.  mpcb_target keeps no workspace, so the factor call solves the problem again,
+ * from the same guess and with the same code, and captures at its end.
+ *   mpcb_target_sens_size:   doubles per instance of the capture `fac`: [0] its status, [1] the solve's status,
+ *                            [2 : 2+nwss] the solution, then the Bunch-Kaufman factor of K, its pivots, dF/dtheta_ss.
+ *   mpcb_target_sens_factor: par_ss and wss0 as given to mpcb_target (wss0 is not modified; the stored wss equals that
+ *                            call's output); writes only fac [B, size] and status [B]: 0 computed; 1 the solve's status
+ *                            was not 0 or 1; 2 wrong inertia of K.  Any status other than 0 makes that instance's
+ *                            outputs of jvp / vjp NaN.
+ *   mpcb_target_jvp:         dwss [B, ndir, nwss] = T dth for dth [B, ndir, ntheta_ss], T = d(wss opt)/d(theta_ss).
+ *   mpcb_target_vjp:         gth [B, ntheta_ss] = T' gwss for gwss [B, nwss].
+ * Without the target problem, or for a large model on the dense derivative path (decided at code generation), all
+ * four return < 0. */
+long mpcb_target_sens_size(void);
+int  mpcb_target_sens_factor(mpcb_handle_t h, const double* par_ss, const double* wss0, double* fac, int* status, void* stream);
+int  mpcb_target_jvp(mpcb_handle_t h, const double* fac, int ndir, const double* dth, double* dwss, void* stream);
+int  mpcb_target_vjp(mpcb_handle_t h, const double* fac, const double* gwss, double* gth, void* stream);
+
 /* Plant measurement  y = Fy_p(x,u,pyp,t,pymp) + noise   (MPC_code.py:531-541); noise may be NULL. */
 int  mpcb_plant_meas(mpcb_handle_t h, const double* x, const double* u, const double* t, const double* pyp,
                      const double* pymp, const double* noise, double* y, void* stream);

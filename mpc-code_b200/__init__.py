@@ -9,6 +9,7 @@ __version__ = "0.1.0"
 from .loader import load_example  # noqa: F401
 from .problem import build_problem, make_specs  # noqa: F401
 from .sensitivity import OcpLayer, OcpSensitivity, params_of, theta_of, with_params, with_theta  # noqa: F401
+from .sensitivity import TargetLayer, TargetSensitivity, theta_ss_of, with_theta_ss  # noqa: F401
 
 
 def compile_problem(*args, **kwargs):

@@ -261,6 +261,35 @@ __global__ void __launch_bounds__(64) k_target_resto(int B, const double* par, d
     if (inst >= B) return;
     tgt_solve_resto(par + (size_t)inst * MPCB_NPARSS, w + (size_t)inst * NWS, f + inst, status + inst, iters + inst, S);
 }
+#if MPCB_SENS_TGT
+// sensitivities of the target solution (mpcb_target_sens_factor): the mapping and the two variants of k_target
+__global__ void __launch_bounds__(64) k_target_sens(int B, const double* par, const double* w0, double* fac, int* status,
+                                                    TgtShared S) {
+    const int inst = blockIdx.x * blockDim.x + threadIdx.x;
+    if (inst >= B) return;
+    tgt_sens_regular(par + (size_t)inst * MPCB_NPARSS, w0 + (size_t)inst * NWS, fac + (size_t)inst * TgtSensLayout::total,
+                     status + inst, S);
+}
+__global__ void __launch_bounds__(64) k_target_sens_resto(int B, const double* par, const double* w0, double* fac, int* status,
+                                                          TgtShared S) {
+    const int inst = blockIdx.x * blockDim.x + threadIdx.x;
+    if (inst >= B) return;
+    tgt_sens_resto(par + (size_t)inst * MPCB_NPARSS, w0 + (size_t)inst * NWS, fac + (size_t)inst * TgtSensLayout::total,
+                   status + inst, S);
+}
+// JVP: one thread per (instance, direction), as k_ocp_jvp; VJP: one thread per instance
+__global__ void __launch_bounds__(128) k_target_jvp(int B, int ndir, const double* fac, const double* dth, double* dw) {
+    const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tid >= (long)B * ndir) return;
+    const long inst = tid / ndir;
+    tgt_jvp_dir(fac + inst * TgtSensLayout::total, dth + tid * NTS, dw + tid * NWS);
+}
+__global__ void __launch_bounds__(128) k_target_vjp(int B, const double* fac, const double* gw, double* gth) {
+    const long inst = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (inst >= B) return;
+    tgt_vjp_inst(fac + inst * TgtSensLayout::total, gw + inst * NWS, gth + inst * NTS);
+}
+#endif
 #endif
 
 __global__ void __launch_bounds__(64) k_estimate(int B, int est_type, const double* y, const double* u, const double* t,
@@ -1024,6 +1053,60 @@ int mpcb_target(mpcb_handle_t h, const double* par_ss, double* wss, double* fss,
 #else
     h->err = "library built without the target problem"; return -3;
 #endif
+}
+
+long mpcb_target_sens_size(void) {
+#if MPCB_SENS_TGT
+    return TgtSensLayout::total;
+#else
+    return -1;
+#endif
+}
+
+static int tgt_sens_refuse(mpcb_ctx* h) {
+    if (!MPCB_HAS_TARGET) { h->err = "library built without the target problem"; return -3; }
+    if (MPCB_SENS_TGT) return 0;
+    h->err = "target sensitivities are not generated for this problem (a large model on the dense derivative path, or a "
+             "map after the RK4 integration that is not affine in d / px)";
+    return -4;
+}
+
+// Solves the target problem again from wss0 (not modified) and writes only `fac` and `status`.
+int mpcb_target_sens_factor(mpcb_handle_t h, const double* par_ss, const double* wss0, double* fac, int* status, void* stream) {
+    if (int rc = tgt_sens_refuse(h)) return rc;
+#if MPCB_SENS_TGT
+    cudaStream_t s = (cudaStream_t)stream;
+    TgtShared S; S.lbx = h->ss_lbx; S.ubx = h->ss_ubx; S.o = to_ipm(h->opts_ss);
+    { Prof p(h, s, KC_OTHER); k_target_sens<<<nblk(h->B, MPCB_TGT_BLOCK), MPCB_TGT_BLOCK, 0, s>>>(h->B, par_ss, wss0, fac, status, S); }
+    { Prof p(h, s, KC_OTHER); k_target_sens_resto<<<nblk(h->B, MPCB_TGT_BLOCK), MPCB_TGT_BLOCK, 0, s>>>(h->B, par_ss, wss0, fac, status, S); }
+    h->host_launches += 2;
+    CK(cudaGetLastError());
+#endif
+    return 0;
+}
+
+int mpcb_target_jvp(mpcb_handle_t h, const double* fac, int ndir, const double* dth, double* dwss, void* stream) {
+    if (int rc = tgt_sens_refuse(h)) return rc;
+    if (ndir < 0) { h->err = "mpcb_target_jvp: ndir must be >= 0"; return -2; }
+    if (ndir == 0) return 0;
+#if MPCB_SENS_TGT
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_target_jvp<<<nblk((long)h->B * ndir, 128), 128, 0, s>>>(h->B, ndir, fac, dth, dwss); }
+    CK(cudaGetLastError());
+#endif
+    return 0;
+}
+
+int mpcb_target_vjp(mpcb_handle_t h, const double* fac, const double* gwss, double* gth, void* stream) {
+    if (int rc = tgt_sens_refuse(h)) return rc;
+#if MPCB_SENS_TGT
+    cudaStream_t s = (cudaStream_t)stream;
+    h->host_launches += 1;
+    { Prof p(h, s, KC_OTHER); k_target_vjp<<<nblk(h->B, 128), 128, 0, s>>>(h->B, fac, gwss, gth); }
+    CK(cudaGetLastError());
+#endif
+    return 0;
 }
 
 int mpcb_estimate(mpcb_handle_t h, int est_type, const double* y, const double* u, const double* t, const double* px,

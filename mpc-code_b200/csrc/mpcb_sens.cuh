@@ -380,7 +380,8 @@ MPCB_HD int sens_p_index(int k, int c) {
     return c < ND ? c : (c < NPM ? ND + k * NPX + (c - ND) : ND + NPX * NH + k * NPY + (c - NPM));
 }
 
-#if MPCB_SENS_P
+// sens_dyn_dp also gives the d / px columns of the target problem's model equalities (mpcb_target.cuh, MPCB_SENS_TGT)
+#if MPCB_SENS_P || MPCB_SENS_TGT
 #if MPCB_DYN_RK4 && MPCB_SENS_NQ > 0
 // The model ODE on the augmented state [x; q], q' = 0: q holds the components MPCB_SENS_QIDX of [d; px] that the
 // right-hand side reads (the generated mdlp_* take them from the state, the rest from the context).  Run with the
@@ -445,6 +446,9 @@ MPCB_HD void sens_dyn_dp(const double* x, const double* u, const double* d, cons
     mdl_F_dp(x, u, d, &t0, px, lam, Fm, Hm);
 #endif
 }
+#endif  // MPCB_SENS_P || MPCB_SENS_TGT
+
+#if MPCB_SENS_P
 
 // stage k: Fp (NXA x NPK) and Qp (NZA x NPK) at w*, with the multipliers the stage record was built with
 MPCB_HD void sens_p_stage(const OcpInst& I, int k, double* Fp, double* Qp) {

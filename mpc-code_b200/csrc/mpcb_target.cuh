@@ -7,6 +7,12 @@
 // Estimator: Estimator.py:231-386.  Plant: Utilities.py:21-100 as called at MPC_code.py:531-534,813-816.
 #pragma once
 #include "mpcb_ocp.cuh"
+#ifndef MPCB_SENS_TGT
+#define MPCB_SENS_TGT 0                   // 1: the generator wrote the target problem's mixed derivatives (tgt_*_dth)
+#endif
+#if MPCB_SENS_TGT
+#include "mpcb_sens.cuh"                  // sens_dyn_dp: the d / px columns of the model equalities
+#endif
 
 #define NWS  MPCB_NWSS
 // user rows of the target problem (Target_Calc.py:87-109): NGT inequalities g_SS <= 0, each with a slack variable
@@ -179,13 +185,84 @@ MPCB_HD void tgt_eval(const double* w, const double* par, const double* lam, boo
         for (int i = 0; i < MCS; ++i) J[i + MCS * (NWS + j)] = (i == NX + NY + j) ? -1.0 : 0.0;
 }
 
+#if MPCB_SENS_TGT
+// ---------------------------------------------------------------------------------------------
+// Sensitivities of the target solution with respect to theta_ss = [usp | ysp | xsp | d | Us_prev | px | py] (par_ss
+// without vec(lam) and t, which are held constant).  At the returned iterate the barrier KKT system F(v; theta_ss) = 0
+// of v = [xs, us, ys, slacks] is differentiated: dv/dtheta_ss = -K^{-1} dF/dtheta_ss, with K the matrix of the Newton
+// step (Hessian of the Lagrangian + Sigma = Z / D on the bounded variables, J and J') without regularisation, and
+// dF/dtheta_ss = [d(grad_v L)/dtheta_ss ; dc/dtheta_ss] with the final equality multipliers.  The bounds are shared
+// constants and add no theta terms.  With honor_original_bounds the solve clips w after its loop: the derivative is
+// taken at the iterate before that clipping (the stored wss is the clipped one, which mpcb_target returns).
+// The solve keeps its multipliers in registers, so the capture solves the problem again from the same guess, with the
+// same code (tgt_solve_t<., true>), and builds the capture in the solver's tail.
+// ---------------------------------------------------------------------------------------------
+#define NTS MPCB_NTHSS
+struct TgtSensLayout {                                               // doubles per instance
+    static constexpr int head = 0;                                   // [0] status (0 / 1 / 2), [1] status of the solve
+    static constexpr int w = 2;                                      // NWS  the solution (mpcb_target's output)
+    static constexpr int K = w + NWS;                                // NKS*NKS  Bunch-Kaufman factor of K
+    static constexpr int piv = K + NKS * NKS;                        // NKS  its pivots
+    static constexpr int fth = piv + NKS;                            // NKS*NTS  dF/dtheta_ss, column-major
+    static constexpr int total = (fth + NKS * NTS + 1) / 2 * 2;
+};
+
+// dF/dtheta_ss at (w, y), rows [grad_v L (NVT) | c (MCS)]; the slack rows and columns have no theta terms
+MPCB_HD void tgt_eval_dth(const double* w, const double* par, const double* y, double* Fth) {
+    double Lt[NWS * NTS], Yt[NOUT * NTS], HYt[NWS * NTS];
+    tgt_cost_dth(w, par, Lt);
+    tgt_out_dth(w, par, y + NX, Yt, HYt);
+    for (int e = 0; e < NKS * NTS; ++e) Fth[e] = 0.0;
+    for (int t = 0; t < NTS; ++t) {
+        for (int j = 0; j < NWS; ++j) Fth[j + NKS * t] = Lt[j + NWS * t] + HYt[j + NWS * t];
+        for (int i = 0; i < NOUT; ++i) Fth[NVT + NX + i + NKS * t] = Yt[i + NOUT * t];
+    }
+    // d and px enter the model equalities Fx(xs, us) - xs = 0 (theta_ss columns OFFSS_D + c and OFFSS_LAM + c - ND)
+    double dl[ND + 1], pxl[NPX + 1], Fm[NX * NPM + 1], Hm[NZ * NPM + 1];
+    for (int i = 0; i < ND; ++i) dl[i] = par[MPCB_OFFSS_D + i];
+    for (int i = 0; i < NPX; ++i) pxl[i] = par[MPCB_OFFSS_PX + i];
+    sens_dyn_dp(w, w + NX, dl, pxl, par[MPCB_OFFSS_T], y, Fm, Hm);
+    for (int c = 0; c < NPM; ++c) {
+        const int t = c < ND ? MPCB_OFFSS_D + c : MPCB_OFFSS_LAM + (c - ND);
+        for (int r = 0; r < NZ; ++r) Fth[r + NKS * t] += Hm[r + NZ * c];
+        for (int i = 0; i < NX; ++i) Fth[NVT + i + NKS * t] += Fm[i + NX * c];
+    }
+}
+
+// Capture at the final iterate of a solve that ended with `status`: K without regularisation, its factor and inertia
+// check (NVT, MCS, 0), dF/dtheta_ss.  cap[0]: 0 computed, 1 the solve ended with a status other than 0 / 1, 2 wrong inertia.
+MPCB_HD void tgt_capture(const double* par, const double* w, const double* y, const double* zL, const double* zU,
+                         const double* lo, const double* hi, const bool* hl, const bool* hu, const double* J,
+                         const double* Hp, int status, double* cap) {
+    cap[1] = (double)status;
+    if (status != 0 && status != 1) { cap[TgtSensLayout::head] = 1.0; return; }
+    double K[NKS * NKS]; int ipiv[NKS], np_, nn_, nz_;
+    for (int i = 0; i < NKS * NKS; ++i) K[i] = 0.0;
+    for (int j = 0; j < NVT; ++j) {
+        if (j < NWS) for (int i = j; i < NWS; ++i) K[i + NKS * j] = Hp[tri(i, j)];
+        double sig = 0.0;
+        if (hl[j]) sig += zL[j] / (w[j] - lo[j]);
+        if (hu[j]) sig += zU[j] / (hi[j] - w[j]);
+        K[j + NKS * j] += sig;
+        for (int i = 0; i < MCS; ++i) K[NVT + i + NKS * j] = J[i + MCS * j];
+    }
+    bk_factor<NKS>(K, ipiv, &np_, &nn_, &nz_);
+    for (int i = 0; i < NKS * NKS; ++i) cap[TgtSensLayout::K + i] = K[i];
+    for (int i = 0; i < NKS; ++i) cap[TgtSensLayout::piv + i] = (double)ipiv[i];
+    tgt_eval_dth(w, par, y, cap + TgtSensLayout::fth);
+    cap[TgtSensLayout::head] = (np_ == NVT && nn_ == MCS && nz_ == 0) ? 0.0 : 2.0;
+}
+#endif  // MPCB_SENS_TGT
+
 // Whole interior-point solve of one target problem (same algorithm as oracle/ipm.py and mpcb_ocp.cuh).
 // MPCB_TGT_RESTO = false: the regular iterations only; a failed line search returns TGT_NEEDS_RESTO and `tgt_solve`
 // repeats the (cold-started, deterministic) solve with the variant that carries the feasibility restoration.  Keeping
 // the restoration out of the common variant halves its register spills (ptxas: 520 / 1288 B vs 1132 / 1930 B).
+// CAPTURE = true (mpcb_target_sens_factor): the tail also writes the sensitivity capture `cap` of the final iterate.
 #define TGT_NEEDS_RESTO 1000
-template <bool MPCB_TGT_RESTO>
-MPCB_HD void tgt_solve_t(const double* par, double* w_io, double* fout, int* status_out, int* iters_out, const TgtShared& S) {
+template <bool MPCB_TGT_RESTO, bool CAPTURE = false>
+MPCB_HD void tgt_solve_t(const double* par, double* w_io, double* fout, int* status_out, int* iters_out, const TgtShared& S,
+                         double* cap = nullptr) {
     const IpmOpts& o = S.o;
     const double rf = o.bound_relax;
     double w[NVT], lo[NVT], hi[NVT]; bool hl[NVT], hu[NVT];
@@ -394,6 +471,12 @@ MPCB_HD void tgt_solve_t(const double* par, double* w_io, double* fout, int* sta
         it += 1;
         evaluate = true;
     }
+#if MPCB_SENS_TGT
+    if constexpr (CAPTURE)
+        if (status != TGT_NEEDS_RESTO) tgt_capture(par, w, y, zL, zU, lo, hi, hl, hu, J, Hp, status, cap);
+#else
+    (void)cap;
+#endif
     if (o.honor_original_bounds) {
         for (int j = 0; j < NWS; ++j) w[j] = fmin(fmax(w[j], S.lbx[j]), S.ubx[j]);
         double ct[MCS];
@@ -426,6 +509,53 @@ MPCB_HD void tgt_solve(const double* par, double* w, double* fout, int* status_o
     tgt_solve_regular(par, w, fout, status_out, iters_out, S);
     tgt_solve_resto(par, w, fout, status_out, iters_out, S);
 }
+
+#if MPCB_SENS_TGT
+// The capture of one instance (mpcb_target_sens_factor): the solve of mpcb_target from the same guess wss0 (not modified),
+// in the same two variants; *st is TGT_NEEDS_RESTO between them, then the capture's status.
+MPCB_HD void tgt_sens_regular(const double* par, const double* wss0, double* cap, int* st, const TgtShared& S) {
+    double w[NWS], f; int status, iters;
+    for (int i = 0; i < NWS; ++i) w[i] = wss0[i];
+    tgt_solve_t<false, true>(par, w, &f, &status, &iters, S, cap);
+    if (status == TGT_NEEDS_RESTO) { *st = status; return; }
+    for (int i = 0; i < NWS; ++i) cap[TgtSensLayout::w + i] = w[i];
+    *st = (int)cap[TgtSensLayout::head];
+}
+MPCB_HD void tgt_sens_resto(const double* par, const double* wss0, double* cap, int* st, const TgtShared& S) {
+    if (*st != TGT_NEEDS_RESTO) return;
+    double w[NWS], f; int status, iters;
+    for (int i = 0; i < NWS; ++i) w[i] = wss0[i];
+    tgt_solve_t<true, true>(par, w, &f, &status, &iters, S, cap);
+    for (int i = 0; i < NWS; ++i) cap[TgtSensLayout::w + i] = w[i];
+    *st = (int)cap[TgtSensLayout::head];
+}
+
+// JVP: dw = -[K^{-1} dF/dtheta_ss dth]_{0:NWS};  VJP: K v = [gw; 0], g = -dF/dtheta_ss' v (K is symmetric)
+MPCB_HD void tgt_jvp_dir(const double* cap, const double* th, double* dw) {
+    if (cap[TgtSensLayout::head] != 0.0) { for (int i = 0; i < NWS; ++i) dw[i] = NAN; return; }
+    const double* F = cap + TgtSensLayout::fth;
+    double r[NKS]; int ipiv[NKS];
+    for (int i = 0; i < NKS; ++i) {
+        double a = 0.0;
+        for (int t = 0; t < NTS; ++t) a -= F[i + NKS * t] * th[t];
+        r[i] = a; ipiv[i] = (int)cap[TgtSensLayout::piv + i];
+    }
+    bk_solve<NKS>(cap + TgtSensLayout::K, ipiv, r);
+    for (int i = 0; i < NWS; ++i) dw[i] = r[i];
+}
+MPCB_HD void tgt_vjp_inst(const double* cap, const double* gw, double* g) {
+    if (cap[TgtSensLayout::head] != 0.0) { for (int t = 0; t < NTS; ++t) g[t] = NAN; return; }
+    const double* F = cap + TgtSensLayout::fth;
+    double r[NKS]; int ipiv[NKS];
+    for (int i = 0; i < NKS; ++i) { r[i] = i < NWS ? gw[i] : 0.0; ipiv[i] = (int)cap[TgtSensLayout::piv + i]; }
+    bk_solve<NKS>(cap + TgtSensLayout::K, ipiv, r);
+    for (int t = 0; t < NTS; ++t) {
+        double a = 0.0;
+        for (int i = 0; i < NKS; ++i) a -= F[i + NKS * t] * r[i];
+        g[t] = a;
+    }
+}
+#endif  // MPCB_SENS_TGT
 #endif  // MPCB_HAS_TARGET
 
 // ---------------------------------------------------------------------------------------------

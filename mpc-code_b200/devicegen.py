@@ -178,14 +178,10 @@ def _sens_p_functions(prob, o, D, ins_c, zz, stage_cost, rows) -> List[CFunction
     """Mixed derivatives for the OCP sensitivities with respect to the parameters that enter the dynamics
     (csrc/mpcb_sens.cuh, mpcb_ocp_sens_factor_p): stage k depends on p_k = [d; px_k; py_k] only, the terminal maps on d.
 
-    * dynamics, RK4: the right-hand side is integrated on the augmented state [x; q] with q' = 0, where q holds the
-      components of (d, px) that the right-hand side reads (MPCB_SENS_QIDX, indices into [d; px]).  The RK4 sweeps of the
-      solve then give dx_N/dq in the q columns of the sensitivity block and the mixed Hessian of lam' x_N in the packed
-      Hessian.  The map applied after the integration (Bd d + px) must be affine; its Jacobian is added.
-    * dynamics, discrete / linear: dF/d[d; px] and d(grad_{x,u} lam' F)/d[d; px] directly.
+    * dynamics: `_sens_model_functions`.
     * stage cost, range rows and terminal maps: as ``_sens_functions`` with respect to p_k (terminal: d).
     MPCB_SENS_P = 0 (the p entry points refuse) when `_sens_p_refusal` names a reason."""
-    nx, nu, nd, npx = prob.nx, prob.nu, prob.nd, prob.npx
+    nd = prob.nd
     par, off = o.par, o.off
     exprs = [stage_cost, o.term_cost] + ([o.term_eq] if o.term_eq is not None else []) + ([rows[0]] if rows else [])
     why = _sens_p_refusal(prob, o, exprs)
@@ -203,6 +199,23 @@ def _sens_p_functions(prob, o, D, ins_c, zz, stage_cost, rows) -> List[CFunction
         R, mult = rows
         fns.append(CFunction("ocp_out_dp", ins_c + [("mult", mult)],
                              [("Yp", jacobian(R, pk)), ("HYp", jacobian(gradient(mtimes(mult.T, R), zz), pk))]))
+    model = _sens_model_functions(prob, D)
+    if model is None:
+        raise NotImplementedError("the map applied after the RK4 integration must be affine in (d, px)")
+    return fns + model
+
+
+def _sens_model_functions(prob, D) -> Optional[List[CFunction]]:
+    """The model part of the sensitivities with respect to [d; px] (csrc/mpcb_sens.cuh, sens_dyn_dp), shared by the OCP
+    p-blocks and the target problem's capture: dF/d[d; px] and d(grad_{x,u} lam' F)/d[d; px] of the stage map.
+
+    * RK4: the right-hand side is integrated on the augmented state [x; q] with q' = 0, where q holds the components of
+      (d, px) that the right-hand side reads (MPCB_SENS_QIDX, indices into [d; px]).  The RK4 sweeps then give dx_N/dq in
+      the q columns of the sensitivity block and the mixed Hessian of lam' x_N in the packed Hessian.  The map applied
+      after the integration (Bd d + px) must be affine; its Jacobian is added.  None when it is not.
+    * discrete / linear: dF/d[d; px] and d(grad_{x,u} lam' F)/d[d; px] directly."""
+    nx, nu, nd, npx = prob.nx, prob.nu, prob.nd, prob.npx
+    fns: List[CFunction] = []
     x, u, d, t, px = [SX.sym(n, k) for n, k in (("x", nx), ("u", nu), ("d", nd), ("t", 1), ("px", npx))]
     dpx = vertcat(d, px)
     base = [("x", x), ("u", u), ("d", d), ("t", t), ("px", px)]
@@ -215,7 +228,7 @@ def _sens_p_functions(prob, o, D, ins_c, zz, stage_cost, rows) -> List[CFunction
         post = SX(prob.Fx_model.meta["post"](d, px))
         Jpost = jacobian(post, dpx)
         if _depends_on(Jpost, dpx):
-            raise NotImplementedError("the map applied after the RK4 integration must be affine in (d, px)")
+            return None
         fns.append(CFunction("mdl_post_dp", [("d", d), ("px", px)], [("Jp", Jpost)]))
         if qidx:
             nq = len(qidx)
@@ -237,6 +250,28 @@ def _sens_p_functions(prob, o, D, ins_c, zz, stage_cost, rows) -> List[CFunction
         fns.append(CFunction("mdl_F_dp", base + [("lam", lam)],
                              [("Fp", jacobian(F, dpx)), ("Hp", jacobian(gradient(mtimes(lam.T, F), vertcat(x, u)), dpx))]))
     return fns
+
+
+
+
+def _sens_tgt_functions(prob, t_, D, yres, mult, model: bool) -> List[CFunction]:
+    """Mixed derivatives for the sensitivities of the target problem (csrc/mpcb_target.cuh, mpcb_target_sens_factor)
+    with respect to theta_ss = [usp | ysp | xsp | d | Us_prev | px | py] (par_ss without vec(lam) and t): the cost
+    gradient, and the rows after the model equalities (outputs, g_SS, h_SS) with their multiplier-weighted gradient.  The
+    d / px columns of the model equalities come from `sens_dyn_dp`, whose generated functions are added here when the OCP
+    p-blocks did not add them (``model``).  MPCB_SENS_TGT = 0 (the target entry points refuse) for large models on the
+    dense derivative path and for a post-integration map that is not affine."""
+    refused = (prob.Fx_model.meta.get("kind") == "rk4" and _use_dense(prob.nx, prob.nu)) or not D.get("MPCB_HAS_OCP")
+    fns = [] if refused or not model else _sens_model_functions(prob, D)
+    D["MPCB_SENS_TGT"] = int(not refused and fns is not None)
+    if not D["MPCB_SENS_TGT"]:
+        return []
+    w, par, off = t_.wss, t_.par, t_.off
+    th = par[0:off["lam"]] if off["end"] == off["px"] else vertcat(par[0:off["lam"]], par[off["px"]:off["end"]])
+    D["MPCB_NTHSS"] = th.numel()
+    return fns + [CFunction("tgt_cost_dth", [("w", w), ("par", par)], [("Lt", jacobian(gradient(t_.cost, w), th))]),
+                  CFunction("tgt_out_dth", [("w", w), ("par", par), ("mult", mult)],
+                            [("Yt", jacobian(yres, th)), ("HYt", jacobian(gradient(mtimes(mult.T, yres), w), th))])]
 
 
 def generate_header(prob, ss_spec, ocp_spec, opts: Optional[Dict] = None) -> Dict[str, object]:
@@ -402,6 +437,7 @@ def generate_header(prob, ss_spec, ocp_spec, opts: Optional[Dict] = None) -> Dic
         fns.append(CFunction("tgt_out", [("w", w), ("par", par)], [("r", yres)]))
         fns.append(CFunction("tgt_out_d", [("w", w), ("par", par), ("mult", mult)],
                              [("r", yres), ("J", jacobian(yres, w)), ("H", tril_pack(Hy))]))
+        fns += _sens_tgt_functions(prob, t_, D, yres, mult, model=not D.get("MPCB_SENS_P"))
     else:
         D["MPCB_HAS_TARGET"] = 0
 

@@ -271,6 +271,40 @@ class BatchedMpc:
                                "use step()")
         return self.solver.sensitivity().feedback_gain()
 
+    def controller_gains(self):
+        """The controller's linearisation at the last `step()`, through the target problem and the OCP: a dict of
+        [B, nu, n] tensors
+
+        * ``x_hat``: dU_0/dx_hat (the target does not read x_hat: `feedback_gain`);
+        * ``u_prev``: dU_0/du_{k-1} with Delta-u terms, else None;
+        * ``usp``, ``ysp``, ``xsp``: the set-point gains J_theta[:, x_s|u_s] T[(x_s,u_s), .] with T = dwss/dtheta_ss;
+        * ``d_hat``: the total dU_0/dd_hat = J_p[:, d] + J_theta[:, x_s|u_s] T[(x_s,u_s), d]; None when nd = 0 or when the
+          OCP has no sensitivities with respect to p (decided at code generation).
+
+        An instance whose target solve was rejected as infeasible keeps its previous targets, so its T-terms are zero;
+        an instance whose OCP or target capture failed gives NaN.  Not available after `step_fused`."""
+        if self._fused:
+            raise RuntimeError("controller_gains() after step_fused(): the fused step keeps its target and OCP problems on "
+                               "the device; use step()")
+        t, p = self.torch, self.prob
+        nx, nu, ny, nd = p.nx, p.nu, p.ny, p.nd
+        with_p = bool(nd) and bool(self.cp.build["gen"]["defines"].get("MPCB_SENS_P"))
+        ocp = self.solver.sensitivity(params=with_p)
+        K = ocp.feedback_gain()
+        out = dict(x_hat=K[0], u_prev=K[1]) if self.cp.ocp_spec.uses_uprev else dict(x_hat=K, u_prev=None)
+        # dU_0/d[x_s; u_s]: theta columns nx .. 2nx+nu
+        E = t.zeros(nx + nu, self.h.ntheta, dtype=t.float64, device=self.h.device)
+        E[t.arange(nx + nu), t.arange(nx, 2 * nx + nu)] = 1.0
+        G = ocp.jvp(E.expand(self.B, -1, -1))[:, :, nx:nx + nu].transpose(1, 2)              # [B, nu, nx+nu]
+        T = self.solver_ss.sensitivity().jacobian()[:, :nx + nu]                               # [B, nx+nu, ntheta_ss]
+        T = T.masked_fill((self.solver_ss.stats()["status"] == INFEASIBLE).view(-1, 1, 1), 0.0)
+        GT = t.bmm(G, T)                                                                      # [B, nu, ntheta_ss]
+        for name, a, n in (("usp", 0, nu), ("ysp", nu, ny), ("xsp", nu + ny, nx)):
+            out[name] = GT[:, :, a:a + n].contiguous()
+        o_d = nu + ny + nx
+        out["d_hat"] = ocp.disturbance_gain() + GT[:, :, o_d:o_d + nd] if with_p else None
+        return out
+
     # -- the same step through the fused C entry point (mpcb_step): no host glue between the solves ----------
     def fused_reset(self):
         """Hand the current loop state to the device-resident loop of `mpcb_step`.  Only at the start of a run: the

@@ -12,6 +12,13 @@ disturbance estimate d_hat and the per-stage model offsets, whose derivatives ar
 * `OcpSensitivity` (from ``BatchedNlpSolver.sensitivity()``): JVP, VJP, the feedback gain dU_0/dx_hat and, with
   ``params=True``, the JVP / VJP in p and the disturbance gain dU_0/dd_hat.
 * `OcpLayer`: the solve as a differentiable function of theta (and of p with ``params=True``) for ``torch.autograd``.
+
+The steady-state target problem has sensitivities with respect to theta_ss = [usp | ysp | xsp | d | Us_prev | px | py],
+the part of ``par_ss`` the loop feeds in (``par_ss`` without vec(lambda) and t; ``ntheta_ss = 2nu+ny+nx+nd+npx+npy``):
+
+* `TargetSensitivity` (from ``solver_ss.sensitivity()``): JVP, VJP and the Jacobian dwss/dtheta_ss.
+* `TargetLayer`: the target solve as a differentiable function of theta_ss.
+* ``BatchedMpc.controller_gains()`` composes them with the OCP's into the controller's total gains.
 """
 from __future__ import annotations
 
@@ -104,8 +111,8 @@ class OcpSensitivity:
 
     def disturbance_gain(self):
         """dU_0/dd_hat [B, nu, nd] with the targets x_s, u_s held fixed: the OCP's response to the disturbance estimate.
-        In the closed loop d_hat also moves x_s and u_s through the target problem; that part of the total derivative is
-        not included (the target problem's sensitivities are not available)."""
+        In the closed loop d_hat also moves x_s and u_s through the target problem; that part is not included here.
+        ``BatchedMpc.controller_gains()["d_hat"]`` is the total derivative through the target problem."""
         self._require_params()
         torch = _torch()
         nx, nu, nd, B = self.nx, self.nu, self.nd, self.handle.batch
@@ -113,6 +120,74 @@ class OcpSensitivity:
         E[torch.arange(nd), torch.arange(nd)] = 1.0
         dw = self.handle.ocp_jvp_p(self.fac, E.expand(B, -1, -1))
         return dw[:, :, nx:nx + nu].transpose(1, 2).contiguous()
+
+
+def theta_ss_slices(nx: int, nu: int, ny: int, nd: int):
+    """The two slices of ``par_ss`` that make up theta_ss: [usp | ysp | xsp | d | Us_prev], and [px | py]."""
+    off_lam = 2 * nu + ny + nx + nd
+    return slice(0, off_lam), slice(off_lam + ny * nu + 1, None)
+
+
+def theta_ss_of(par_ss, nx: int, nu: int, ny: int, nd: int):
+    """theta_ss [B, ntheta_ss] of target parameter vectors ``par_ss`` [B, nparss]."""
+    a, b = theta_ss_slices(nx, nu, ny, nd)
+    return _torch().cat([par_ss[:, a], par_ss[:, b]], dim=1)
+
+
+def with_theta_ss(par_ss, theta_ss, nx: int, nu: int, ny: int, nd: int):
+    """``par_ss`` with its theta_ss part replaced by ``theta_ss`` (differentiable in both)."""
+    a, b = theta_ss_slices(nx, nu, ny, nd)
+    return _torch().cat([theta_ss[:, :a.stop], par_ss[:, a.stop:b.start], theta_ss[:, a.stop:]], dim=1)
+
+
+class TargetSensitivity:
+    """Captured sensitivities of one batched target solve with respect to theta_ss.  ``status`` [B] (int32, device): 0
+    computed, 1 the solve ended with a status other than 0 / 1, 2 wrong inertia of the KKT matrix; every output of an
+    instance with status != 0 is NaN.  The capture ``fac`` belongs to this object."""
+
+    def __init__(self, handle, fac, status):
+        self.handle, self.fac, self.status = handle, fac, status
+        self.ntheta_ss = handle.ntheta_ss
+
+    @property
+    def wss(self):
+        """[B, nwss] the solution the capture was taken at (bit for bit the output of the target solve it repeats)."""
+        return self.fac[:, 2:2 + self.handle.lib.dims.nwss]
+
+    def jvp(self, dth):
+        """dwss [B, ndir, nwss] for dth [B, ndir, ntheta_ss]; a [B, ntheta_ss] input gives [B, nwss]."""
+        dw = self.handle.target_jvp(self.fac, dth)
+        return dw[:, 0] if getattr(dth, "ndim", 3) == 2 else dw
+
+    def vjp(self, gw):
+        """gth [B, ntheta_ss] = (dwss/dtheta_ss)' gw for gw [B, nwss]."""
+        return self.handle.target_vjp(self.fac, gw)
+
+    def jacobian(self):
+        """dwss/dtheta_ss [B, nwss, ntheta_ss]."""
+        torch = _torch()
+        E = torch.eye(self.ntheta_ss, dtype=torch.float64, device=self.handle.device)
+        return self.handle.target_jvp(self.fac, E.expand(self.handle.batch, -1, -1)).transpose(1, 2).contiguous()
+
+
+class TargetLayer:
+    """``wss = TargetLayer(solver_ss)(theta_ss, par_ss, wss0)``: the batched target solve as a function of theta_ss,
+    differentiable through ``torch.autograd`` (backward = one VJP on the captured factorisation).  ``par_ss`` supplies
+    vec(lambda) and t (its theta_ss part is replaced) and ``wss0`` is the initial guess; neither may require grad.
+    Once differentiable."""
+
+    def __init__(self, solver_ss, lbx=None, ubx=None):
+        if solver_ss.kind != "target":
+            raise NotImplementedError("TargetLayer wraps the target solver")
+        self.solver, self.bounds = solver_ss, dict(lbx=lbx, ubx=ubx)
+        self.last = None                # TargetSensitivity of the last forward pass
+
+    def __call__(self, theta_ss, par_ss, wss0):
+        for name, t in (("par_ss", par_ss), ("wss0", wss0)):
+            if getattr(t, "requires_grad", False):
+                raise ValueError("TargetLayer differentiates with respect to theta_ss only: %s must not require grad "
+                                 "(sensitivities with respect to t and lambda are not available)" % name)
+        return _target_function().apply(theta_ss, par_ss, wss0, self)
 
 
 class OcpLayer:
@@ -201,8 +276,42 @@ def _make_function_p():
     return OcpFunctionP
 
 
+def _make_target_function():
+    torch = _torch()
+    from torch.autograd.function import once_differentiable
+
+    class TargetFunction(torch.autograd.Function):
+        @staticmethod
+        def forward(ctx, theta_ss, par_ss, wss0, layer):
+            h = layer.solver.handle
+            d = h.lib.dims
+            p = with_theta_ss(h.tensor(par_ss, d.nparss), theta_ss.detach().to(h.device, torch.float64), d.nx, d.nu, d.ny, d.nd)
+            sol = layer.solver(x0=wss0, p=p, **layer.bounds)
+            sens = layer.solver.sensitivity()
+            layer.last = sens
+            ctx.sens = sens
+            ctx.dtype, ctx.device = theta_ss.dtype, theta_ss.device
+            return sol["x"]
+
+        @staticmethod
+        @once_differentiable
+        def backward(ctx, gw):
+            g = ctx.sens.vjp(gw.contiguous())
+            return g.to(device=ctx.device, dtype=ctx.dtype), None, None, None
+
+    return TargetFunction
+
+
 _FUNCTION = None
 _FUNCTION_P = None
+_FUNCTION_TGT = None
+
+
+def _target_function():
+    global _FUNCTION_TGT
+    if _FUNCTION_TGT is None:
+        _FUNCTION_TGT = _make_target_function()
+    return _FUNCTION_TGT
 
 
 def _ocp_function():

@@ -37,7 +37,8 @@ C_SYMBOLS = ("mpcb_abi_version", "mpcb_default_opts", "mpcb_get_dims", "mpcb_mod
              "mpcb_last_launches", "mpcb_last_ticks", "mpcb_total_launches", "mpcb_set_groups", "mpcb_set_policy", "mpcb_set_profiling", "mpcb_get_profile", "mpcb_dfma_peak",
              "mpcb_loop_reset", "mpcb_step", "mpcb_loop_get",
              "mpcb_ocp_sens_size", "mpcb_ocp_sens_factor", "mpcb_ocp_jvp", "mpcb_ocp_vjp",
-             "mpcb_ocp_sens_size_p", "mpcb_ocp_sens_factor_p", "mpcb_ocp_jvp_p", "mpcb_ocp_vjp_p")
+             "mpcb_ocp_sens_size_p", "mpcb_ocp_sens_factor_p", "mpcb_ocp_jvp_p", "mpcb_ocp_vjp_p",
+             "mpcb_target_sens_size", "mpcb_target_sens_factor", "mpcb_target_jvp", "mpcb_target_vjp")
 
 
 class MpcbLibrary:
@@ -85,6 +86,10 @@ class MpcbLibrary:
         L.mpcb_ocp_sens_factor_p.argtypes = [vp] * 5
         L.mpcb_ocp_jvp_p.argtypes = [vp, vp, ci, vp, vp, vp]
         L.mpcb_ocp_vjp_p.argtypes = [vp] * 5
+        L.mpcb_target_sens_size.restype = ctypes.c_long
+        L.mpcb_target_sens_factor.argtypes = [vp] * 6
+        L.mpcb_target_jvp.argtypes = [vp, vp, ci, vp, vp, vp]
+        L.mpcb_target_vjp.argtypes = [vp] * 5
         self.dims = MpcbDims()
         L.mpcb_get_dims(ctypes.byref(self.dims))
 
@@ -262,6 +267,46 @@ class MpcbHandle:
         self._check(self.L.mpcb_target(self._h, par_ss.data_ptr(), wss.data_ptr(), f.data_ptr(), st.data_ptr(), it.data_ptr(), self._stream()))
         return wss, f, st, it
 
+    # -- sensitivities of the target solution (include/mpcb.h, mpcb_target_sens_factor) ----------------------------
+    @property
+    def ntheta_ss(self) -> int:
+        """Size of theta_ss = [usp | ysp | xsp | d | Us_prev | px | py]."""
+        d = self.lib.dims
+        return 2 * d.nu + d.ny + d.nx + d.nd + d.npx + d.npy
+
+    def target_sens_factor(self, par_ss, wss0):
+        """Capture of the sensitivities of the target solve from ``par_ss`` and the initial guess ``wss0`` (those of the
+        `target` call; the problem is solved again): ``(fac [B, size], status [B])``."""
+        torch = _torch()
+        d = self.lib.dims
+        par_ss = self.tensor(par_ss, d.nparss); wss0 = self.tensor(wss0, d.nwss)
+        size = int(self.L.mpcb_target_sens_size())
+        fac = self.empty(self.batch, max(size, 1))
+        st = self.empty(self.batch, dtype=torch.int32)
+        self._check(self.L.mpcb_target_sens_factor(self._h, par_ss.data_ptr(), wss0.data_ptr(), fac.data_ptr(), st.data_ptr(),
+                                                   self._stream()))
+        return fac, st
+
+    def target_jvp(self, fac, dth):
+        """dwss [B, ndir, nwss] = T dth for dth [B, ndir, ntheta_ss] (or [B, ntheta_ss]: one direction)."""
+        d = self.lib.dims
+        dt = self.tensor(dth)
+        if dt.ndim == 2:
+            dt = dt.unsqueeze(1)
+        if dt.ndim != 3 or dt.shape[0] != self.batch or dt.shape[2] != self.ntheta_ss:
+            raise ValueError("dth must be [B, ndir, %d], got %s" % (self.ntheta_ss, tuple(dt.shape)))
+        dt = dt.contiguous()
+        dw = self.empty(self.batch, dt.shape[1], d.nwss)
+        self._check(self.L.mpcb_target_jvp(self._h, fac.data_ptr(), int(dt.shape[1]), dt.data_ptr(), dw.data_ptr(), self._stream()))
+        return dw
+
+    def target_vjp(self, fac, gw):
+        """gth [B, ntheta_ss] = T' gw for gw [B, nwss]."""
+        gw = self.tensor(gw, self.lib.dims.nwss)
+        g = self.empty(self.batch, self.ntheta_ss)
+        self._check(self.L.mpcb_target_vjp(self._h, fac.data_ptr(), gw.data_ptr(), g.data_ptr(), self._stream()))
+        return g
+
     def estimate(self, est_type, y, u_prev, t, px, py, xi, P):
         d = self.lib.dims
         y = self.tensor(y, d.ny); u_prev = self.tensor(u_prev, d.nu); t = self.tensor(t, 1)
@@ -401,6 +446,7 @@ class BatchedNlpSolver:
         self.handle: Optional[MpcbHandle] = None
         self._last = None
         self._last_ocp = None           # (par, handle solve count) of the last OCP call, for sensitivity()
+        self._last_target = None        # copies of (p, x0) of the last target call, for sensitivity()
         self._bounds_key = None
 
     def attach(self, handle: MpcbHandle):
@@ -461,7 +507,9 @@ class BatchedNlpSolver:
             x, f, st, it = self.handle.ocp(par, x0)
             self._last_ocp = (par, self.handle.ocp_solves)
         else:
-            x, f, st, it = self.handle.target(p, x0)
+            d = self.handle.lib.dims
+            self._last_target = (self.handle.tensor(p, d.nparss).clone(), self.handle.tensor(x0, d.nwss).clone())
+            x, f, st, it = self.handle.target(*self._last_target)
         self._last = (st, it)
         return {"x": x, "f": f}
 
@@ -469,9 +517,12 @@ class BatchedNlpSolver:
         """Sensitivities of the last solve with respect to theta = [x_hat | x_s | u_s | u_{k-1}] (see
         `mpc_code_b200.sensitivity`): an `OcpSensitivity` that owns its capture and stays valid after later solves.
         ``params=True`` also captures the sensitivities with respect to p = [d | px | py] (`OcpSensitivity.jvp_p`).
-        Must be called before the handle solves another OCP, with the solve's ``p`` not modified in place since."""
-        if self.kind != "ocp":
-            raise NotImplementedError("sensitivities are available for the dynamic OCP only, not the target problem")
+        Must be called before the handle solves another OCP, with the solve's ``p`` not modified in place since.
+
+        On the target solver: a `TargetSensitivity` of the last solve through this solver, with respect to theta_ss =
+        [usp | ysp | xsp | d | Us_prev | px | py] (the problem is solved again from that call's ``p`` and ``x0``)."""
+        if self.kind == "target":
+            return self._target_sensitivity(params)
         self._require()
         if self._last_ocp is None:
             raise RuntimeError("sensitivity() before the first solve")
@@ -481,6 +532,17 @@ class BatchedNlpSolver:
         from .sensitivity import OcpSensitivity
         fac, st = (self.handle.ocp_sens_factor_p if params else self.handle.ocp_sens_factor)(par)
         return OcpSensitivity(self.handle, fac, st, uses_uprev=bool(self.spec.uses_uprev), params=params)
+
+    def _target_sensitivity(self, params):
+        if params:
+            raise ValueError("params=True is for the OCP: theta_ss of the target problem already contains d, px and py")
+        self._require()
+        if self._last_target is None:
+            raise NotImplementedError("sensitivity() of the target problem before a solve through this solver: the fused "
+                                      "step (mpcb_step) keeps its target problem on the device and has no sensitivities")
+        from .sensitivity import TargetSensitivity
+        fac, st = self.handle.target_sens_factor(*self._last_target)
+        return TargetSensitivity(self.handle, fac, st)
 
     def stats(self):
         if self._last is None:

@@ -2,8 +2,9 @@
 
 CUDA events around, after warm-up: the batched mpcb_ocp solve, mpcb_ocp_sens_factor, the full theta-Jacobian (one JVP
 of all ntheta unit directions) and one VJP; for p = [d | px | py] mpcb_ocp_sens_factor_p, the d-Jacobian (nd unit
-directions), the full p-Jacobian (all n_p unit directions) and one VJP_p; the median of --reps repetitions each.  Prints the card name and power
-limit read in the same run.  Usage: python tools/sens_timing.py [--batch 4096] [--reps 20]
+directions), the full p-Jacobian (all n_p unit directions) and one VJP_p; for the target problem the batched mpcb_target
+solve, mpcb_target_sens_factor (which solves again), the full theta_ss-Jacobian and one VJP; the median of --reps
+repetitions each.  Prints the card name and power limit read in the same run.  Usage: python tools/sens_timing.py [--batch 4096] [--reps 20]
 """
 import argparse
 import json
@@ -68,6 +69,23 @@ def main():
     t_jac_d = timed(lambda: h.ocp_jvp_p(fac_p, eye_d))
     t_jac_p = timed(lambda: h.ocp_jvp_p(fac_p, eye_p))
     t_vjp_p = timed(lambda: h.ocp_vjp_p(fac_p, gw))
+    # target problem: the golden instances with perturbed disturbance estimates and output set-points
+    par_ss = G["ss_par"][np.arange(B) % G["ss_par"].shape[0]].copy()
+    o = ss.off
+    par_ss[:, o["ysp"]:o["xsp"]] *= 1 + 0.01 * rng.uniform(-1, 1, (B, prob.ny))
+    par_ss[:, o["d"]:o["usprev"]] *= 1 + 0.01 * rng.uniform(-1, 1, (B, prob.nd))
+    par_ss = h.tensor(par_ss, ss.npar)
+    wss0 = h.tensor(G["ss_w0"][np.arange(B) % G["ss_w0"].shape[0]], ss.nw)
+    solver_ss = BatchedNlpSolver("target", ss).attach(h)
+    eye_ss = torch.eye(h.ntheta_ss, dtype=torch.float64, device=h.device).expand(B, -1, -1).contiguous()
+    gws = torch.as_tensor(rng.standard_normal((B, ss.nw)), device=h.device)
+    solver_ss(x0=wss0, p=par_ss)
+    fac_t, st_t = h.target_sens_factor(par_ss, wss0)
+    h.target_jvp(fac_t, eye_ss); h.target_vjp(fac_t, gws); torch.cuda.synchronize()
+    t_tsolve = timed(lambda: h.target(par_ss, wss0))
+    t_tfactor = timed(lambda: h.target_sens_factor(par_ss, wss0))
+    t_tjac = timed(lambda: h.target_jvp(fac_t, eye_ss))
+    t_tvjp = timed(lambda: h.target_vjp(fac_t, gws))
     res = dict(card=card, problem="nmpc_cstr (Ex_NMPC)", batch=B, ntheta=nth, reps=a.reps,
                sens_status_counts={int(k): int(v) for k, v in zip(*np.unique(st.cpu().numpy(), return_counts=True))},
                solve_ms=t_solve, factor_ms=t_factor, jacobian_ms=t_jac, vjp_ms=t_vjp,
@@ -78,7 +96,12 @@ def main():
                factor_p_ms=t_factor_p, d_jacobian_ms=t_jac_d, p_jacobian_ms=t_jac_p, vjp_p_ms=t_vjp_p,
                factor_p_plus_d_jacobian_over_solve=(t_factor_p + t_jac_d) / t_solve,
                factor_p_plus_p_jacobian_over_solve=(t_factor_p + t_jac_p) / t_solve,
-               factor_p_plus_vjp_p_over_solve=(t_factor_p + t_vjp_p) / t_solve)
+               factor_p_plus_vjp_p_over_solve=(t_factor_p + t_vjp_p) / t_solve,
+               ntheta_ss=h.ntheta_ss, capture_target_doubles_per_instance=int(h.L.mpcb_target_sens_size()),
+               target_sens_status_counts={int(k): int(v) for k, v in zip(*np.unique(st_t.cpu().numpy(), return_counts=True))},
+               target_solve_ms=t_tsolve, target_factor_ms=t_tfactor, target_jacobian_ms=t_tjac, target_vjp_ms=t_tvjp,
+               target_factor_over_target_solve=t_tfactor / t_tsolve,
+               target_factor_plus_jacobian_over_ocp_solve=(t_tfactor + t_tjac) / t_solve)
     print(json.dumps(res, indent=1))
 
 
